@@ -26,13 +26,14 @@ EXPORTS = ["fc_rqs_apply", "fc_rqs_backward", "fc_rqs_bins", "fc_linspline_apply
            "fc_sos_backward", "fc_stdnormal_log_prob", "fc_linear_pack", "fc_linear_apply", "fc_linear_rqs_apply",
            "fc_linear_affine_apply", "fc_linear_splitk_apply", "fc_linear_splitk_t_apply", "fc_linear_transpose",
            "fc_linear_pack_transposed", "fc_linear_debug_profile",
-           "fc_elementwise_last_path", "fc_conditioner_layer_bytes", "fc_conditioner_pack_layer", "fc_conditioner_rqs_apply", "fc_conditioner_sos_apply", "fc_conditioner_affine_apply", "fc_conditioner_store_apply", "fc_conditioner_error", "fc_conditioner_profile",
+           "fc_elementwise_last_path", "fc_conditioner_layer_bytes", "fc_conditioner_pack_layer", "fc_conditioner_rqs_apply", "fc_conditioner_sos_apply", "fc_conditioner_affine_apply", "fc_conditioner_store_apply", "fc_context_terms", "fc_conditioner_error", "fc_conditioner_profile",
            "fc_actnorm_apply", "fc_actnorm_workspace_floats", "fc_actnorm_backward",
            "fc_made_inverse_smem_bytes", "fc_made_inverse_profile", "fc_made_inverse_rqs", "fc_made_inverse_affine",
            "fc_made_inverse_sos", "fc_made_inverse_linspline", "fc_made_inverse_quadspline", "fc_made_inverse_cubicspline",
            "fc_version", "fc_built_for_sm"]
 COND_MAX_LAYERS = 10
 COND_INITIAL, COND_BLOCK_FIRST, COND_BLOCK_SECOND, COND_FINAL = 0, 1, 2, 3
+COND_TERM_NONE, COND_TERM_ADD, COND_TERM_ADD_RELU, COND_TERM_GATE = 0, 1, 2, 3
 
 
 class RqsConfig(ctypes.Structure):
@@ -64,8 +65,8 @@ class LinearWeights(ctypes.Structure):
 class ConditionerLayer(ctypes.Structure):
     """struct fc_conditioner_layer"""
     _fields_ = [("kind", ctypes.c_int32), ("n_tiles", ctypes.c_int32), ("relu_next", ctypes.c_int32),
-                ("reserved", ctypes.c_int32), ("w_offset", ctypes.c_int64), ("bias", ctypes.c_void_p),
-                ("winv", ctypes.c_void_p)]
+                ("term_mode", ctypes.c_int32), ("w_offset", ctypes.c_int64), ("bias", ctypes.c_void_p),
+                ("winv", ctypes.c_void_p), ("terms", ctypes.c_void_p), ("term_width", ctypes.c_int64)]
 
 
 class Conditioner(ctypes.Structure):
@@ -139,6 +140,7 @@ def lib():
         L.fc_conditioner_affine_apply.argtypes = [ctypes.POINTER(Conditioner), vp, i64, i64, vp, i64, vp, i64, vp, i32,
                                                   i32, Cols, Cols, i32, i32, vp]
         L.fc_conditioner_store_apply.argtypes = [ctypes.POINTER(Conditioner), vp, i64, i64, vp, i64, i32, vp]
+        L.fc_context_terms.argtypes = [vp, i64, i64, i32, vp, vp, i32, vp, vp]
         L.fc_conditioner_error.argtypes = [ctypes.POINTER(ctypes.c_int32)]
         L.fc_conditioner_profile.argtypes = [ctypes.POINTER(ctypes.c_uint64)]
         L.fc_actnorm_apply.argtypes = [vp, i64, vp, vp, vp, i64, vp, i32, i64, i32, i32, vp]

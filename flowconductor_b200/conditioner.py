@@ -5,6 +5,12 @@
 kernel's weight ring, in one buffer, plus the per-layer bias / inverse-scale vectors and the layer table
 (`struct fc_conditioner`).  `rqs_apply` launches conditioner + rational-quadratic spline as ONE kernel on torch's current
 stream.  No fallback: CPU tensors or a missing library raise.
+
+Conditional nets (`context_features`): every `context_layer` of the net is stacked into one [T, C] matrix
+(`ContextPlan`, T = hidden width padded to the kernel's x the number of context layers), `context_terms` evaluates
+Wc ctx + bc for the whole batch in one launch as a T128 matrix, and the `*_apply` calls hand it to the kernel, whose
+hidden layers consume their columns (FC_COND_TERM_* of include/flowcon_b200.h).  The terms do not depend on the
+conditioner's inputs: a D-pass autoregressive inverse computes them once.
 """
 import ctypes
 
@@ -31,10 +37,104 @@ def _ceil_to(v, m):
 class PackedConditioner:
     """Packed weights of a whole conditioner.  Keeps the device buffers alive; `struct` is what the C ABI takes."""
 
-    def __init__(self, weights, vectors, struct, hidden, k_in, n_final_tiles, num_bins):
+    def __init__(self, weights, vectors, struct, hidden, k_in, n_final_tiles, num_bins, context=None):
         self.weights, self.vectors, self.struct = weights, vectors, struct
         # hidden: the width the kernel runs (128 / 256); num_bins: bins of the spline, or None for other bijections
         self.hidden, self.k_in, self.n_final_tiles, self.num_bins = hidden, k_in, n_final_tiles, num_bins
+        self.context = context  # ContextPlan of a conditional net, else None
+
+
+MIN_K_TC = 64  # context widths from here on take the tensor-core GEMM for their terms (nn/tc_autograd.py MIN_K)
+
+
+class ContextPlan:
+    """The context layers of a conditional net stacked into one affine map ctx -> [B, width] (T128).  `layers`: the
+    (conditioner layer index, FC_COND_TERM_* mode, first column) of every layer that consumes terms; the columns of
+    padding units (a net narrower than the kernel's width) have zero weights and bias."""
+
+    def __init__(self, weight, bias, layers, width, linear):
+        self.weight, self.bias, self.layers, self.width = weight, bias, layers, width
+        self.features = weight.shape[1]
+        self.linear = linear  # linear.PackedLinear for the tensor-core GEMM (C >= MIN_K_TC), else None
+
+
+def pack_context(net):
+    """ContextPlan of a conditional ResidualNet (a gate per block, resnet.py:45-52) or residual MADE (initial layer
+    made.py:274-279, the first layer of every block made.py:170-181); None for a net without context layers."""
+    from . import linear as fl
+
+    blocks = list(net.blocks)
+    if hasattr(net, "context_layer"):  # MADE
+        src = [(0, _cabi.COND_TERM_ADD_RELU, net.context_layer)]
+        src += [(1 + 2 * i, _cabi.COND_TERM_ADD, b.context_layer) for i, b in enumerate(blocks)]
+    elif getattr(net, "context_features", None) is not None:  # ResidualNet
+        src = [(2 + 2 * i, _cabi.COND_TERM_GATE, b.context_layer) for i, b in enumerate(blocks)]
+    else:
+        return None
+    hp = padded_hidden(net.initial_layer.weight.shape[0])
+    ref = src[0][2].weight
+    C = ref.shape[1]
+    weight = torch.zeros((hp * len(src), C), dtype=torch.float32, device=ref.device)
+    bias = torch.zeros((hp * len(src),), dtype=torch.float32, device=ref.device)
+    layers = []
+    for i, (layer, mode, lin) in enumerate(src):
+        n = lin.weight.shape[0]
+        weight[i * hp:i * hp + n] = lin.weight.detach()
+        if lin.bias is not None:
+            bias[i * hp:i * hp + n] = lin.bias.detach()
+        layers.append((layer, mode, i * hp))
+    linear = None
+    if C >= MIN_K_TC:
+        c4 = _ceil_to(C, 4)
+        cm = None if c4 == C else torch.arange(C, dtype=torch.int32, device=ref.device)
+        linear = fl.pack(weight, bias, col_map=cm, k_in=c4)
+    return ContextPlan(weight, bias, layers, weight.shape[0], linear)
+
+
+def context_terms(packed, ctx):
+    """Wc ctx + bc of every context layer, [B, width] as a linear.T128: ONE launch (fc_context_terms below the tensor-core
+    GEMM's minimum reduction, else fc_linear_apply).  `packed`: a PackedConditioner of a conditional net or its ContextPlan."""
+    from . import linear as fl
+
+    plan = packed.context if isinstance(packed, PackedConditioner) else packed
+    if plan is None:
+        raise ValueError("the conditioner has no context layers")
+    _cabi.require_cuda_f32(ctx, "context")
+    if ctx.dim() != 2 or ctx.shape[1] != plan.features:
+        raise ValueError("context has shape {}, the net expects {} features".format(tuple(ctx.shape), plan.features))
+    if plan.linear is not None:
+        a = ctx
+        k = plan.linear.k_in
+        if not (k == ctx.shape[1] and ctx.stride(1) == 1 and ctx.stride(0) % 4 == 0 and ctx.data_ptr() % 16 == 0):
+            a = ctx.new_zeros((ctx.shape[0], k))  # 16-byte row pitch for the GEMM's TMA loads
+            a[:, :ctx.shape[1]] = ctx
+        return fl.linear(a, plan.linear, out_t128=True)
+    L = _cabi.lib()
+    ctx, cp, ldc = _cabi.rows(ctx)
+    out = fl.T128(ctx.shape[0], plan.width, ctx.device)
+    with torch.cuda.device(ctx.device), _cabi.launch("fc_context_terms", ctx.device):
+        rc = L.fc_context_terms(cp, ldc, ctx.shape[0], plan.features, plan.weight.data_ptr(), plan.bias.data_ptr(),
+                                plan.width, out.buf.data_ptr(), _cabi.stream_ptr(ctx.device))
+    _cabi.check(rc, "fc_context_terms")
+    return out
+
+
+def _bind_terms(packed, terms, B):
+    """Point the layer table at this call's context terms (a conditional net needs them, any other net takes none)."""
+    if packed.context is None:
+        if terms is not None:
+            raise ValueError("context terms given for a conditioner without context layers")
+        return
+    if terms is None:
+        raise ValueError("a conditioner with context layers needs its context terms (conditioner.context_terms)")
+    if terms.rows != B or terms.width != packed.context.width:
+        raise ValueError("context terms are [{}, {}], expected [{}, {}]".format(terms.rows, terms.width, B,
+                                                                                  packed.context.width))
+    base = terms.buf.data_ptr()
+    for layer, _, col in packed.context.layers:
+        e = packed.struct.layers[layer]
+        e.terms = base + 4 * terms.TILE * col  # T128: a column group is the slow index inside a 128-row tile
+        e.term_width = terms.width
 
 
 def _pack_layer(L, dev, blob, offset, layer, mask, n_pad, k_pad, bn, row_map=None, col_map=None):
@@ -118,12 +218,13 @@ def supported_store_shape(hidden, k_in, num_blocks, n_out):
             and 1 <= num_blocks <= MAX_BLOCKS and _vectors_fit(hidden, num_blocks, STORE_PPAD, (n_out + 47) // 48))
 
 
-def pack(net, P, ppad, d_t, col_map=None, k_in=None, num_bins=None, final_row_map=None, group=1):
+def pack(net, P, ppad, d_t, col_map=None, k_in=None, num_bins=None, final_row_map=None, group=1, context=None):
     """Pack `net` (initial_layer, blocks[*].linear_layers[0..1], final_layer; optional `.mask` per layer, made.py:72)
     for the `fc_conditioner_*_apply` kernels: P parameters per feature in `ppad` accumulator columns (final_row_map /
     group: explicit placement of the final layer's rows, `group` features per `ppad`-column slot).  col_map / k_in:
     scatter of the first layer's input columns (a coupling layer's conditioner reads the full-width inputs:
-    coupling.py:82-86 folded into the weights)."""
+    coupling.py:82-86 folded into the weights; a conditional ResidualNet's initial layer reads [inputs | context]).
+    context: the net's ContextPlan (conditional nets)."""
     L = _cabi.lib()
     init, fin = net.initial_layer, net.final_layer
     dev = init.weight.device
@@ -174,36 +275,41 @@ def pack(net, P, ppad, d_t, col_map=None, k_in=None, num_bins=None, final_row_ma
             e.w_offset = offset
             e.bias, e.winv = vec[0].data_ptr(), vec[1].data_ptr()
             offset += size
-    return PackedConditioner(blob, vectors, st, hidden, k_in, n_final_tiles, num_bins)
+    if context is not None:
+        for layer, mode, _ in context.layers:
+            st.layers[layer].term_mode = mode
+    return PackedConditioner(blob, vectors, st, hidden, k_in, n_final_tiles, num_bins, context)
 
 
-def pack_rqs(net, num_bins, d_t, col_map=None, k_in=None, tails="linear"):
+def pack_rqs(net, num_bins, d_t, col_map=None, k_in=None, tails="linear", context=None):
     """`pack` for `fc_conditioner_rqs_apply` (3 K - 1 parameters per feature with linear tails, 3 K + 1 without)."""
     ppad = rqs_ppad(num_bins, tails)
     if ppad is None:
         raise ValueError("conditioner shape not supported by the fused kernel")
     P = 3 * num_bins - 1 if tails == "linear" else 3 * num_bins + 1
-    return pack(net, P, ppad, d_t, col_map=col_map, k_in=k_in, num_bins=num_bins)
+    return pack(net, P, ppad, d_t, col_map=col_map, k_in=k_in, num_bins=num_bins, context=context)
 
 
-def pack_sos(net, n_sigmoids, d_t, col_map=None, k_in=None):
+def pack_sos(net, n_sigmoids, d_t, col_map=None, k_in=None, context=None):
     """`pack` for `fc_conditioner_sos_apply` (3 n + 1 parameters per feature)."""
     if n_sigmoids not in SOS_SIGMOIDS:
         raise ValueError("conditioner shape not supported by the fused kernel")
-    return pack(net, 3 * n_sigmoids + 1, SOS_PPAD, d_t, col_map=col_map, k_in=k_in)
+    return pack(net, 3 * n_sigmoids + 1, SOS_PPAD, d_t, col_map=col_map, k_in=k_in, context=context)
 
 
-def pack_affine(net, d_t, layout, col_map=None, k_in=None):
+def pack_affine(net, d_t, layout, col_map=None, k_in=None, context=None):
     """`pack` for `fc_conditioner_affine_apply`: feature j's (raw scale, shift) in final-layer rows (2 j, 2 j + 1)."""
     from . import linear as fl
 
     rm = fl.affine_row_map(d_t, layout, net.final_layer.weight.device)
-    return pack(net, 2, AFFINE_PPAD, d_t, col_map=col_map, k_in=k_in, final_row_map=rm, group=AFFINE_GROUP)
+    return pack(net, 2, AFFINE_PPAD, d_t, col_map=col_map, k_in=k_in, final_row_map=rm, group=AFFINE_GROUP,
+                context=context)
 
 
-def rqs_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, cfg, status=None):
+def rqs_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, cfg, status=None, terms=None):
     """Whole conditioner + rational-quadratic spline in one kernel (fc_conditioner_rqs_apply).  a: [B, k_in] matrix the
-    initial layer multiplies; writes y[:, tcols] (and y[:, ccols] = x[:, ccols] unless y is x) and logabsdet."""
+    initial layer multiplies; writes y[:, tcols] (and y[:, ccols] = x[:, ccols] unless y is x) and logabsdet.
+    terms: `context_terms` of this call's context (conditional nets only)."""
     _cabi.require_cuda_f32(a, "conditioner inputs")
     _cabi.require_cuda_f32(x, "inputs")
     L = _cabi.lib()
@@ -212,6 +318,7 @@ def rqs_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, cfg, st
         raise ValueError("conditioner inputs have {} columns, the packed net expects {}".format(a.shape[1], packed.k_in))
     assert x.stride(1) == 1 and y.stride(1) == 1 and logabsdet.is_contiguous()
     B = a.shape[0]
+    _bind_terms(packed, terms, B)
     with torch.cuda.device(x.device), _cabi.launch("fc_conditioner_rqs_apply", x.device):
         rc = L.fc_conditioner_rqs_apply(ctypes.byref(packed.struct), ap, lda, B, x.data_ptr(), x.stride(0), y.data_ptr(),
                                         y.stride(0), logabsdet.data_ptr(), int(accumulate), d_t, _cabi.cols(tcols),
@@ -221,9 +328,9 @@ def rqs_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, cfg, st
     return y, logabsdet
 
 
-def sos_apply(packed, a, x, y, logabsdet, accumulate, d_t, n_sigmoids, offset):
+def sos_apply(packed, a, x, y, logabsdet, accumulate, d_t, n_sigmoids, offset, terms=None):
     """Whole conditioner + sum-of-sigmoids transform (forward) in one kernel (fc_conditioner_sos_apply).  a: [B, k_in]
-    matrix the initial layer multiplies (the context of a conditional layer, the inputs of a MADE)."""
+    matrix the initial layer multiplies (the context of a conditional layer, the inputs of a MADE); terms as `rqs_apply`."""
     _cabi.require_cuda_f32(a, "conditioner inputs")
     _cabi.require_cuda_f32(x, "inputs")
     L = _cabi.lib()
@@ -233,6 +340,7 @@ def sos_apply(packed, a, x, y, logabsdet, accumulate, d_t, n_sigmoids, offset):
     if a.shape[0] != x.shape[0]:
         raise ValueError("conditioner inputs and inputs differ in rows")
     assert x.stride(1) == 1 and y.stride(1) == 1 and logabsdet.is_contiguous()
+    _bind_terms(packed, terms, a.shape[0])
     with torch.cuda.device(x.device), _cabi.launch("fc_conditioner_sos_apply", x.device):
         rc = L.fc_conditioner_sos_apply(ctypes.byref(packed.struct), ap, lda, a.shape[0], x.data_ptr(), x.stride(0),
                                         y.data_ptr(), y.stride(0), logabsdet.data_ptr(), int(accumulate), d_t,
@@ -242,7 +350,7 @@ def sos_apply(packed, a, x, y, logabsdet, accumulate, d_t, n_sigmoids, offset):
     return y, logabsdet
 
 
-def affine_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, activation, inverse):
+def affine_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, activation, inverse, terms=None):
     """Whole conditioner + affine transform in one kernel (fc_conditioner_affine_apply); arguments as `rqs_apply`."""
     _cabi.require_cuda_f32(a, "conditioner inputs")
     _cabi.require_cuda_f32(x, "inputs")
@@ -253,6 +361,7 @@ def affine_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, acti
     if a.shape[0] != x.shape[0]:
         raise ValueError("conditioner inputs and inputs differ in rows")
     assert x.stride(1) == 1 and y.stride(1) == 1 and logabsdet.is_contiguous()
+    _bind_terms(packed, terms, a.shape[0])
     with torch.cuda.device(x.device), _cabi.launch("fc_conditioner_affine_apply", x.device):
         rc = L.fc_conditioner_affine_apply(ctypes.byref(packed.struct), ap, lda, a.shape[0], x.data_ptr(), x.stride(0),
                                            y.data_ptr(), y.stride(0), logabsdet.data_ptr(), int(accumulate), d_t,
@@ -262,23 +371,26 @@ def affine_apply(packed, a, x, y, logabsdet, accumulate, d_t, tcols, ccols, acti
     return y, logabsdet
 
 
-def pack_store(net, col_map=None, k_in=None):
+def pack_store(net, col_map=None, k_in=None, context=None):
     """`pack` for `fc_conditioner_store_apply` (the conditioner's outputs, no bijection): final-layer rows in their own order."""
     n_out = net.final_layer.weight.shape[0]
     rm = torch.arange(n_out, dtype=torch.int32, device=net.final_layer.weight.device)
-    packed = pack(net, STORE_PPAD, STORE_PPAD, (n_out + 47) // 48, col_map=col_map, k_in=k_in, final_row_map=rm)
+    packed = pack(net, STORE_PPAD, STORE_PPAD, (n_out + 47) // 48, col_map=col_map, k_in=k_in, final_row_map=rm,
+                  context=context)
     packed.n_out = n_out
     return packed
 
 
-def store_apply(packed, a, out):
-    """The whole conditioner in one kernel, outputs to `out` [B, out_features] (fc_conditioner_store_apply)."""
+def store_apply(packed, a, out, terms=None):
+    """The whole conditioner in one kernel, outputs to `out` [B, out_features] (fc_conditioner_store_apply); terms as
+    `rqs_apply`."""
     _cabi.require_cuda_f32(a, "conditioner inputs")
     L = _cabi.lib()
     a, ap, lda = _cabi.rows(a)
     if a.shape[1] != packed.k_in:
         raise ValueError("conditioner inputs have {} columns, the packed net expects {}".format(a.shape[1], packed.k_in))
     assert out.shape == (a.shape[0], packed.n_out) and out.stride(1) == 1 and out.is_cuda and out.dtype == torch.float32
+    _bind_terms(packed, terms, a.shape[0])
     with torch.cuda.device(a.device), _cabi.launch("fc_conditioner_store_apply", a.device):
         rc = L.fc_conditioner_store_apply(ctypes.byref(packed.struct), ap, lda, a.shape[0], out.data_ptr(), out.stride(0),
                                           packed.n_out, _cabi.stream_ptr(a.device))

@@ -73,6 +73,9 @@ struct CondLayerDev {
   int col0;            // first column of the layer in the shared-memory bias / exponent vectors
   const float* bias;   // [n_tiles * bn]
   const float* winv;   // [1] exact power of two: 1 / the layer's weight scale
+  int term_mode;       // FC_COND_TERM_*: context terms consumed by this layer
+  const float* terms;  // T128 context terms from the layer's first column on
+  long long term_tile; // floats per 128-row tile of the term matrix (128 x its width)
 };
 
 struct CondArgs {
@@ -83,6 +86,7 @@ struct CondArgs {
   long long M;
   int num_tiles;  // 256-row tiles (one per CTA pair and step)
   int n_layers;
+  int has_terms;  // some layer consumes context terms
   int slots_per_tile;
   int total_cols;  // output columns of all layers (a multiple of 4): size of the bias / scale-exponent vectors in shared memory
   CondLayerDev L[kMaxCondLayers];
@@ -324,7 +328,9 @@ struct CondStore {
 
 // Bij the bijection, PPAD accumulator columns per feature, NT = hidden width / 128
 // HAND: every hand_period-th final tile is handed to the bijection warps entirely (instantiated where it pays)
-template <class Bij, int PPAD, int NT, bool HAND>
+// CTX: the hidden layers consume context terms (FC_COND_TERM_*; a separate instantiation, so that the code of nets without
+// context stays exactly as it is)
+template <class Bij, int PPAD, int NT, bool HAND, bool CTX>
 __global__ void __launch_bounds__(kCondThreads, 1) conditioner_f16x3_kernel(const CondArgs a) {
   constexpr int KCH = 2 * NT;         // 64-value chunks of a hidden-width reduction
   constexpr int FEATS = 96 / PPAD;    // features per final N tile
@@ -422,7 +428,21 @@ __global__ void __launch_bounds__(kCondThreads, 1) conditioner_f16x3_kernel(cons
       if (lane == 0) {
         int s = 0;
         uint32_t ph = 0;
+        // the context terms of a row tile -> L2 ahead of the row threads (in T128 a layer's columns of one 128-row tile
+        // are one contiguous block)
+        auto prefetch_terms = [&](int t) {
+          if ((long long)t * 256 + rank * kCM >= a.M) return;
+          for (int l = 0; l < a.n_layers - 1; ++l) {
+            const CondLayerDev& L = a.L[l];
+            if (L.term_mode != FC_COND_TERM_NONE)
+              bulk_prefetch_l2(L.terms + (long long)(2 * t + rank) * L.term_tile, (uint32_t)(L.n_tiles * L.bn * kCM * 4));
+          }
+        };
+        if constexpr (CTX) prefetch_terms(cl0);
         for (int tile = cl0; tile < a.num_tiles; tile += cl_step) {
+          if constexpr (CTX) {
+            if (tile + cl_step < a.num_tiles) prefetch_terms(tile + cl_step);
+          }
           for (int l = 0; l < a.n_layers; ++l) {
             const CondLayerDev& L = a.L[l];
             const unsigned char* src = a.weights + ((size_t)L.w_off16 << 4) + (size_t)rank * L.cta_bytes;
@@ -681,12 +701,16 @@ __global__ void __launch_bounds__(kCondThreads, 1) conditioner_f16x3_kernel(cons
         for (int nt = 0; nt < NT; ++nt) {
           const int n0 = nt * 128 + half * 64;
           float* hcol = hs + n0 * kCM + rl;
+          // this row's context terms of the 64 columns (T128: the warp's 32 rows read 512 contiguous bytes per float4)
+          const float4* g4 = nullptr;
+          if (CTX && L.term_mode != FC_COND_TERM_NONE && valid)
+            g4 = reinterpret_cast<const float4*>(L.terms + (long long)(2 * tile + rank) * L.term_tile) + (n0 >> 2) * kCM + rl;
           {
             // the register accumulators start from the bias (all lanes read the same words: broadcast) plus, in the second
             // layer of a block, the skip connection (resnet.py:56 / made.py:181: inputs + temps) — fetched while the
-            // first partial sums are still being computed
+            // first partial sums are still being computed; with context terms (MADE) + g or + relu(g), fetched the same way
             const float4* b4 = reinterpret_cast<const float4*>(vbias + L.col0 + n0);
-            const bool add_h = L.kind == FC_COND_BLOCK_SECOND;
+            const bool add_h = L.kind == FC_COND_BLOCK_SECOND && !(CTX && L.term_mode == FC_COND_TERM_GATE);
 #pragma unroll
             for (int j4 = 0; j4 < 16; ++j4) {
               const float4 b = b4[j4];
@@ -702,6 +726,23 @@ __global__ void __launch_bounds__(kCondThreads, 1) conditioner_f16x3_kernel(cons
                                             make_float2(hcol[j * kCM], hcol[(j + 1) * kCM]));
                 av[nt * 64 + j] = r.x;
                 av[nt * 64 + j + 1] = r.y;
+              }
+            }
+            if (CTX && g4 != nullptr && L.term_mode != FC_COND_TERM_GATE) {
+              const bool rl_g = L.term_mode == FC_COND_TERM_ADD_RELU;
+#pragma unroll
+              for (int j4 = 0; j4 < 16; ++j4) {
+                float4 g = __ldg(g4 + j4 * kCM);
+                if (rl_g) {
+                  g.x = fmaxf(g.x, 0.f);
+                  g.y = fmaxf(g.y, 0.f);
+                  g.z = fmaxf(g.z, 0.f);
+                  g.w = fmaxf(g.w, 0.f);
+                }
+                av[nt * 64 + 4 * j4 + 0] += g.x;
+                av[nt * 64 + 4 * j4 + 1] += g.y;
+                av[nt * 64 + 4 * j4 + 2] += g.z;
+                av[nt * 64 + 4 * j4 + 3] += g.w;
               }
             }
           }
@@ -731,6 +772,19 @@ __global__ void __launch_bounds__(kCondThreads, 1) conditioner_f16x3_kernel(cons
             CPROF_ADD(r_drain_h, t_d);
           }
           CPROF_T0(t_f);
+          if (CTX && L.term_mode == FC_COND_TERM_GATE) {
+            // ResidualNet block with context (resnet.py:45-52): h + t * sigmoid(g), F.glu of [t | g]
+#pragma unroll
+            for (int j4 = 0; j4 < 16; ++j4) {
+              const float4 g = g4 != nullptr ? __ldg(g4 + j4 * kCM) : make_float4(0.f, 0.f, 0.f, 0.f);
+              const float gv[4] = {g.x, g.y, g.z, g.w};
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                const int j = 4 * j4 + i;
+                av[nt * 64 + j] = fmaf(av[nt * 64 + j], fc_sigmoid(gv[i]), hcol[j * kCM]);
+              }
+            }
+          }
           // residual stream, ReLU
           if (L.kind == FC_COND_INITIAL || (L.kind == FC_COND_BLOCK_SECOND && L.relu_next)) {
             // (after the last block nothing reads the residual stream again)
@@ -1108,9 +1162,9 @@ __global__ void __launch_bounds__(128) cond_pack_kernel(const float* __restrict_
   }
 }
 
-template <class Bij, int PPAD, int NT, bool HAND = false>
-static int launch_conditioner(const CondArgs& args, cudaStream_t stream) {
-  auto kern = conditioner_f16x3_kernel<Bij, PPAD, NT, HAND>;
+template <class Bij, int PPAD, int NT, bool HAND, bool CTX>
+static int launch_conditioner_t(const CondArgs& args, cudaStream_t stream) {
+  auto kern = conditioner_f16x3_kernel<Bij, PPAD, NT, HAND, CTX>;
   static_assert(CondSmem::TOTAL <= 232448, "shared memory per CTA");
   static std::atomic<uint64_t> configured{0};
   int dev_id = 0;
@@ -1138,6 +1192,11 @@ static int launch_conditioner(const CondArgs& args, cudaStream_t stream) {
   if (cudaLaunchKernelEx(&cfg, kern, args) != cudaSuccess) return FC_ERR_CUDA;
   FC_CHECK_LAUNCH();
   return FC_OK;
+}
+template <class Bij, int PPAD, int NT, bool HAND = false>
+static int launch_conditioner(const CondArgs& args, cudaStream_t stream) {
+  return args.has_terms ? launch_conditioner_t<Bij, PPAD, NT, HAND, true>(args, stream)
+                        : launch_conditioner_t<Bij, PPAD, NT, HAND, false>(args, stream);
 }
 
 }  // namespace fc
@@ -1231,6 +1290,20 @@ static int cond_build_args(const fc_conditioner* net, const float* a, int64_t ld
     d.cta_bytes = (unsigned)(2 * (d.bn / 2) * 128);
     d.bias = s.bias;
     d.winv = s.winv;
+    // context terms: each mode belongs to one layer kind (header: FC_COND_TERM_*)
+    if (s.term_mode < FC_COND_TERM_NONE || s.term_mode > FC_COND_TERM_GATE) return FC_ERR_INVALID_ARGUMENT;
+    static const int kTermKind[4] = {-1, FC_COND_BLOCK_FIRST, FC_COND_INITIAL, FC_COND_BLOCK_SECOND};
+    d.term_mode = s.term_mode;
+    d.terms = nullptr;
+    d.term_tile = 0;
+    if (s.term_mode != FC_COND_TERM_NONE) {
+      if (s.kind != kTermKind[s.term_mode] || (B > 0 && !s.terms)) return FC_ERR_INVALID_ARGUMENT;
+      if ((reinterpret_cast<uintptr_t>(s.terms) & 15) || s.term_width < (int64_t)s.n_tiles * 128 || (s.term_width & 15))
+        return FC_ERR_UNSUPPORTED;
+      d.terms = s.terms;
+      d.term_tile = 128 * s.term_width;
+      args.has_terms = 1;
+    }
     d.col0 = args.total_cols;
     args.total_cols += d.n_tiles * d.bn;
     args.slots_per_tile += d.n_tiles * d.k_chunks;

@@ -880,6 +880,13 @@ FC_HD void fc_sigmoid_parts(float z, float& sig, float& dsig) {
   dsig = Er * r;
 }
 
+// sigma(z) alone, same arithmetic (the context gate of a conditional ResidualNet block, F.glu)
+FC_HD float fc_sigmoid(float z) {
+  const float E = fc_exp2(-fabsf(z) * FC_LOG2E);
+  const float r = fc_rcp(1.f + E);
+  return z >= 0.f ? r : E * r;
+}
+
 FC_HD float fc_tanh(float t) {
   const float at = fabsf(t);
   const float E = fc_exp2(at * (-2.f * FC_LOG2E));

@@ -7,6 +7,10 @@ runs as `fc_linear_rqs_apply` (spline in the GEMM epilogue) where the bijection 
 rational-quadratic spline with 8 or 16 bins; otherwise the final layer's parameters are materialised by
 `fc_linear_apply` and handed to the stand-alone element-wise kernel.
 
+Conditional nets (a ResidualNet with `context_features`, a MADE with a `context_layer`) run only on the fused
+conditioner kernel: their context layers become one launch of precomputed terms (`context_terms`) that the kernel's
+hidden layers consume; a conditional net of a shape the fused kernel does not cover stays on the torch modules.
+
 The packed weights are cached on the module and rebuilt when any parameter changes (data pointer or
 in-place version counter).  Training (autograd) keeps using the torch.nn modules and the custom ops of
 `flowconductor_b200.ops`: this path has no backward.
@@ -86,18 +90,20 @@ def wants_grad(net, *tensors):
 
 
 def supported_net(net, context):
-    """True if `net` is a ResidualNet / MADE configuration the kernels cover."""
+    """True if `net` is a ResidualNet / MADE configuration the kernels cover, called with a context exactly when it has
+    context layers."""
     from ..transforms import made as made_module
     from .nets.resnet import ResidualNet
 
-    if not ENABLED or context is not None:
+    if not ENABLED:
         return False
     if isinstance(net, ResidualNet):
-        if net.context_features is not None:
+        if (net.context_features is not None) != (context is not None):
             return False
         blocks = net.blocks
     elif isinstance(net, made_module.MADE):
-        if not net.use_residual_blocks or hasattr(net, "context_layer") or not _is_relu(net.activation):
+        if (not net.use_residual_blocks or hasattr(net, "context_layer") != (context is not None)
+                or not _is_relu(net.activation)):
             return False
         blocks = net.blocks
     else:
@@ -115,10 +121,80 @@ def supported_net(net, context):
 
 def usable(net, a, context, *other_inputs):
     """Should this conditioner call take the tensor-core path?  `a` is the matrix the first layer multiplies."""
-    if not supported_net(net, context) or wants_grad(net, a, *other_inputs):
+    if not supported_net(net, context) or wants_grad(net, a, context, *other_inputs):
         return False
     # (the TMA operand constraints — 16-byte aligned base and row pitch — are met by `aligned_inputs` below)
-    return a.is_cuda and a.dtype == torch.float32 and a.dim() == 2 and a.shape[0] > 0
+    if not (a.is_cuda and a.dtype == torch.float32 and a.dim() == 2 and a.shape[0] > 0):
+        return False
+    if context is None:
+        return True
+    # only the fused conditioner takes a context (the per-layer kernels do not): its store variant, which every layer
+    # can fall back to, must cover the net
+    return (context.is_cuda and context.dtype == torch.float32 and context.dim() == 2 and context.shape[0] == a.shape[0]
+            and FUSED_CONDITIONER and fcond.supported_store_shape(
+                net.initial_layer.weight.shape[0], _pad4(context_k_in(net, a.shape[1], context)), len(net.blocks),
+                net.final_layer.weight.shape[0]))
+
+
+def context_k_in(net, k_in, context):
+    """Input width of the initial layer: a conditional ResidualNet multiplies [inputs | context] (resnet.py:93-95), a
+    MADE only the inputs (its context enters through the terms)."""
+    from .nets.resnet import ResidualNet
+
+    return k_in + context.shape[1] if context is not None and isinstance(net, ResidualNet) else k_in
+
+
+def _with_context(net, a, col_map, k_in, context):
+    """(a, col_map, k_in) for the initial layer of `net` called with `context`: for a ResidualNet one zero-padded
+    [B, k_in + C] copy of [inputs | context] (16-byte row pitch) whose context columns the packed weights read through
+    col_map; unchanged otherwise."""
+    from .nets.resnet import ResidualNet
+
+    if context is None or not isinstance(net, ResidualNet):
+        return a, col_map, k_in
+    k = a.shape[1] if k_in is None else k_in
+    C = context.shape[1]
+    width = (k + C + 3) // 4 * 4
+    cat = a.new_empty((a.shape[0], width))
+    cat[:, :a.shape[1]] = a
+    cat[:, k:k + C] = context
+    if width > k + C:
+        cat[:, k + C:] = 0
+    n_in = net.initial_layer.weight.shape[1] - C  # the input columns of the initial layer come first (resnet.py:93-95)
+    # cached on the net (the col_map of a coupling layer is a buffer of the layer that owns the net)
+    key = (None,) if col_map is None else (id(col_map), col_map.data_ptr(), col_map._version)
+    key += (n_in, k, C, str(a.device))
+    cached = getattr(net, "_fc_ctx_cols", None)
+    if cached is None or cached[0] != key:
+        base = col_map if col_map is not None else torch.arange(n_in, dtype=torch.int32, device=a.device)
+        cm = torch.cat((base.to(torch.int32), torch.arange(k, k + C, dtype=torch.int32, device=a.device)))
+        cached = (key, cm)
+        object.__setattr__(net, "_fc_ctx_cols", cached)
+    return cat, cached[1], width
+
+
+def context_plan_for(net):
+    """ContextPlan (stacked context layers) of a conditional net, cached on the module like the packed weights."""
+    key = _param_key(net)
+    plan = getattr(net, "_fc_ctx_plan", None)
+    if plan is not None and plan[0] == key:
+        return plan[1]
+    packed = fcond.pack_context(net)
+    object.__setattr__(net, "_fc_ctx_plan", (key, packed))
+    _generation[0] += 1
+    return packed
+
+
+def context_terms(net, context):
+    """The context terms of one call (conditioner.context_terms): computed once, shared by every pass of a D-pass
+    autoregressive inverse."""
+    return fcond.context_terms(context_plan_for(net), context)
+
+
+def _terms(net, context, terms):
+    if context is None:
+        return None
+    return terms if terms is not None else context_terms(net, context)
 
 
 def aligned_inputs(a, col_map, k_in):
@@ -175,6 +251,8 @@ def invalidate(module):
             object.__setattr__(m, "_fc_cond_plan", None)
         if getattr(m, "_fc_made_plan", None) is not None:
             object.__setattr__(m, "_fc_made_plan", None)
+        if getattr(m, "_fc_ctx_plan", None) is not None:
+            object.__setattr__(m, "_fc_ctx_plan", None)
     _generation[0] += 1
 
 
@@ -242,19 +320,22 @@ def hidden(net, plan, a):
     return h
 
 
-def params(net, a, col_map=None, k_in=None):
-    """Full conditioner output [B, out_features] (final layer materialised)."""
+def params(net, a, col_map=None, k_in=None, context=None, terms=None):
+    """Full conditioner output [B, out_features] (final layer materialised).  context: the call's context (conditional
+    nets; `terms`: its context_terms when the caller already has them)."""
+    a, col_map, k_in = _with_context(net, a, col_map, k_in, context)
     a, col_map, k_in = aligned_inputs(a, col_map, k_in)
     k = k_in if k_in is not None else a.shape[1]
-    if store_fusable(net, k):  # the whole conditioner as one launch
+    if context is not None or store_fusable(net, k):  # the whole conditioner as one launch
         key = (_param_key(net), "store", k)
         plan = getattr(net, "_fc_cond_plan", None)
         if plan is None or plan[0] != key:
-            plan = (key, fcond.pack_store(net, col_map=col_map, k_in=k))
+            ctx = context_plan_for(net) if context is not None else None
+            plan = (key, fcond.pack_store(net, col_map=col_map, k_in=k, context=ctx))
             object.__setattr__(net, "_fc_cond_plan", plan)
             _generation[0] += 1
         out = torch.empty((a.shape[0], net.final_layer.weight.shape[0]), dtype=a.dtype, device=a.device)
-        return fcond.store_apply(plan[1], a, out)
+        return fcond.store_apply(plan[1], a, out, terms=_terms(net, context, terms))
     plan = plan_for(net, col_map, k_in if k_in is not None else a.shape[1], ("store",))
     n = plan.final.n_out
     n4 = (n + 3) // 4 * 4  # the store epilogue writes 16-byte vectors: round up into the zero-weight padding
@@ -273,17 +354,21 @@ def _output_buffer(inputs, allow_inplace=True):
 
 
 def affine_layer(net, a, inputs, tcols, ccols, layout, activation, inverse, col_map=None, k_in=None,
-                 allow_inplace=True):
-    """Conditioner + affine transform for one layer (final layer fused: fc_linear_affine_apply)."""
+                 allow_inplace=True, context=None, terms=None):
+    """Conditioner + affine transform for one layer (final layer fused: fc_linear_affine_apply).  A conditional net
+    (context given) must pass `affine_fusable` with its context_k_in."""
     d_t = tcols.numel() if tcols is not None else inputs.shape[1]
+    a, col_map, k_in = _with_context(net, a, col_map, k_in, context)
     a, col_map, k_in = aligned_inputs(a, col_map, k_in)
     k_in = k_in if k_in is not None else a.shape[1]
     if affine_fusable(net, k_in, d_t):
-        packed = affine_cond_plan_for(net, col_map, k_in, d_t, layout)
+        packed = affine_cond_plan_for(net, col_map, k_in, d_t, layout, context is not None)
         x, y = _output_buffer(inputs, allow_inplace)
         lad = torch.empty((x.shape[0],), dtype=x.dtype, device=x.device)
-        fcond.affine_apply(packed, a, x, y, lad, False, d_t, tcols, ccols, activation, inverse)
+        fcond.affine_apply(packed, a, x, y, lad, False, d_t, tcols, ccols, activation, inverse,
+                           terms=_terms(net, context, terms))
         return y, lad
+    assert context is None, "conditional nets run on the fused conditioner only"
     plan = plan_for(net, col_map, k_in, ("affine", layout))
     h = hidden(net, plan, a)
     x, y = _output_buffer(inputs, allow_inplace)
@@ -292,11 +377,14 @@ def affine_layer(net, a, inputs, tcols, ccols, layout, activation, inverse, col_
     return y, lad
 
 
-def rqs_fusable(spline, final_out_features, d_t, net=None, k_in=None):
+def rqs_fusable(spline, final_out_features, d_t, net=None, k_in=None, context=None):
     """Can the bijection run inside a tensor-core kernel?  Either in the final layer's epilogue (fc_linear_rqs_apply: linear
-    tails, 8 or 16 bins) or — `net` / `k_in` given — inside the fused conditioner (more bin counts, also without tails)."""
+    tails, 8 or 16 bins) or — `net` / `k_in` given — inside the fused conditioner (more bin counts, also without tails).
+    With a context only the fused conditioner qualifies."""
     if not ENABLED or final_out_features != d_t * spline.params_per_feature():
         return False
+    if context is not None:
+        return net is not None and conditioner_fusable(net, context_k_in(net, k_in, context), spline, d_t)
     if spline.tails == "linear" and spline.num_bins in fl.RQS_PPAD:
         return True
     return net is not None and conditioner_fusable(net, k_in, spline, d_t)
@@ -306,25 +394,28 @@ FUSED_AFFINE = os.environ.get("FC_FUSED_AFFINE", "1") != "0"  # A/B switch of th
 FUSED_CONDITIONER = True  # whole conditioner + spline as ONE persistent kernel (csrc/fc_conditioner.cu) where it applies
 
 
-def cond_plan_for(net, col_map, k_in, num_bins, d_t, tails="linear"):
-    """PackedConditioner of `net`, cached on the module like the per-layer plans (same key rules)."""
-    key = (_param_key(net), num_bins, tails, k_in, d_t)
+def cond_plan_for(net, col_map, k_in, num_bins, d_t, tails="linear", context=False):
+    """PackedConditioner of `net`, cached on the module like the per-layer plans (same key rules).  context: pack the
+    net's context layers as well (a conditional net called with its context)."""
+    key = (_param_key(net), num_bins, tails, k_in, d_t, context)
     plan = getattr(net, "_fc_cond_plan", None)
     if plan is not None and plan[0] == key:
         return plan[1]
-    packed = fcond.pack_rqs(net, num_bins, d_t, col_map=col_map, k_in=k_in, tails=tails)
+    packed = fcond.pack_rqs(net, num_bins, d_t, col_map=col_map, k_in=k_in, tails=tails,
+                            context=context_plan_for(net) if context else None)
     object.__setattr__(net, "_fc_cond_plan", (key, packed))
     _generation[0] += 1
     return packed
 
 
-def affine_cond_plan_for(net, col_map, k_in, d_t, layout):
+def affine_cond_plan_for(net, col_map, k_in, d_t, layout, context=False):
     """PackedConditioner of `net` for the fused affine kernel, cached like the spline plans."""
-    key = (_param_key(net), "affine", layout, k_in, d_t)
+    key = (_param_key(net), "affine", layout, k_in, d_t, context)
     plan = getattr(net, "_fc_cond_plan", None)
     if plan is not None and plan[0] == key:
         return plan[1]
-    packed = fcond.pack_affine(net, d_t, layout, col_map=col_map, k_in=k_in)
+    packed = fcond.pack_affine(net, d_t, layout, col_map=col_map, k_in=k_in,
+                               context=context_plan_for(net) if context else None)
     object.__setattr__(net, "_fc_cond_plan", (key, packed))
     _generation[0] += 1
     return packed
@@ -349,13 +440,14 @@ def affine_fusable(net, k_in, d_t=None):
         net.initial_layer.weight.shape[0], _pad4(k_in), len(net.blocks), d_t)
 
 
-def sos_cond_plan_for(net, k_in, n_sigmoids, d_t, col_map=None):
+def sos_cond_plan_for(net, k_in, n_sigmoids, d_t, col_map=None, context=False):
     """PackedConditioner of `net` for the fused sum-of-sigmoids kernel, cached like the spline plans."""
-    key = (_param_key(net), "sos", n_sigmoids, k_in, d_t)
+    key = (_param_key(net), "sos", n_sigmoids, k_in, d_t, context)
     plan = getattr(net, "_fc_cond_plan", None)
     if plan is not None and plan[0] == key:
         return plan[1]
-    packed = fcond.pack_sos(net, n_sigmoids, d_t, col_map=col_map, k_in=k_in)
+    packed = fcond.pack_sos(net, n_sigmoids, d_t, col_map=col_map, k_in=k_in,
+                            context=context_plan_for(net) if context else None)
     object.__setattr__(net, "_fc_cond_plan", (key, packed))
     _generation[0] += 1
     return packed
@@ -366,17 +458,18 @@ def sos_fusable(net, k_in, n_sigmoids, d_t=None):
                                                            n_sigmoids, d_t)
 
 
-def sos_layer(net, a, inputs, n_sigmoids, offset):
+def sos_layer(net, a, inputs, n_sigmoids, offset, context=None, terms=None):
     """Conditioner + sum-of-sigmoids transform (forward) as one kernel; returns (outputs, logabsdet).  `a` feeds the
-    conditioner (context / MADE inputs), `inputs` the bijection."""
-    a, col_map, k_in = aligned_inputs(a, None, None)
-    packed = sos_cond_plan_for(net, a.shape[1], int(n_sigmoids), inputs.shape[1], col_map)
+    conditioner (context / MADE inputs), `inputs` the bijection; `context`: the context of a conditional net."""
+    a, col_map, k_in = _with_context(net, a, None, None, context)
+    a, col_map, k_in = aligned_inputs(a, col_map, k_in)
+    packed = sos_cond_plan_for(net, a.shape[1], int(n_sigmoids), inputs.shape[1], col_map, context is not None)
     x = inputs if inputs.stride(1) == 1 else inputs.contiguous()
     y = torch.empty_like(x)
     consume_consent()
     mark_fresh(y)
     lad = torch.empty((x.shape[0],), dtype=x.dtype, device=x.device)
-    fcond.sos_apply(packed, a, x, y, lad, False, inputs.shape[1], n_sigmoids, offset)
+    fcond.sos_apply(packed, a, x, y, lad, False, inputs.shape[1], n_sigmoids, offset, terms=_terms(net, context, terms))
     return y, lad
 
 
@@ -389,26 +482,29 @@ def conditioner_fusable(net, k_in, spline, d_t=None):
 
 
 def rqs_layer(net, a, inputs, spline, tcols, ccols, inverse, hidden_for_scaling, col_map=None, k_in=None,
-              allow_inplace=True):
-    """Conditioner + spline for one layer; returns (outputs, logabsdet)."""
+              allow_inplace=True, context=None, terms=None):
+    """Conditioner + spline for one layer; returns (outputs, logabsdet).  A conditional net (context given) must pass
+    `rqs_fusable` with the context."""
     d_t = tcols.numel() if tcols is not None else inputs.shape[1]
+    a, col_map, k_in = _with_context(net, a, col_map, k_in, context)
     a, col_map, k_in = aligned_inputs(a, col_map, k_in)
     k_in = k_in if k_in is not None else a.shape[1]
     cfg, tails = spline.config(inverse, hidden_for_scaling)
     if conditioner_fusable(net, k_in, spline, d_t):
         from ..transforms import splines as fsplines
 
-        packed = cond_plan_for(net, col_map, k_in, int(spline.num_bins), d_t, spline.tails)
+        packed = cond_plan_for(net, col_map, k_in, int(spline.num_bins), d_t, spline.tails, context is not None)
         x, y = _output_buffer(inputs, allow_inplace)
         lad = torch.empty((x.shape[0],), dtype=x.dtype, device=x.device)
         # without tails the reference raises InputOutsideDomain after a host-side check (rational_quadratic.py:81-82): the
         # kernel reports through the status word instead
         status = torch.zeros((1,), dtype=torch.int32, device=x.device) if (tails == _cabi.TAILS_NONE or fsplines.STRICT) \
             else None
-        fcond.rqs_apply(packed, a, x, y, lad, False, d_t, tcols, ccols, cfg, status)
+        fcond.rqs_apply(packed, a, x, y, lad, False, d_t, tcols, ccols, cfg, status, terms=_terms(net, context, terms))
         if status is not None:
             fsplines.check_status(status, tails)
         return y, lad
+    assert context is None, "conditional nets run on the fused conditioner only"
     plan = plan_for(net, col_map, k_in, ("rqs", spline.num_bins))
     h = hidden(net, plan, a)
     x, y = _output_buffer(inputs, allow_inplace)

@@ -26,7 +26,7 @@ class AutoregressiveTransform(Transform):
 
     def forward(self, inputs, context=None):
         if tensorcore.usable(self.autoregressive_net, inputs, context):
-            return self._tensorcore_layer(inputs, inputs, inverse=False)
+            return self._tensorcore_layer(inputs, inputs, False, context)
         params = self.autoregressive_net(inputs, context)
         return self._elementwise_forward(inputs, params)
 
@@ -38,17 +38,20 @@ class AutoregressiveTransform(Transform):
         outputs = torch.zeros_like(inputs)
         logabsdet = None
         fast = tensorcore.usable(self.autoregressive_net, outputs, context, inputs)
+        # the context terms do not depend on the partially inverted outputs: one launch for all D passes
+        terms = tensorcore.context_terms(self.autoregressive_net, context) if fast and context is not None else None
         for _ in range(int(np.prod(inputs.shape[1:]))):
             if fast:
-                outputs, logabsdet = self._tensorcore_layer(outputs, inputs, inverse=True)
+                outputs, logabsdet = self._tensorcore_layer(outputs, inputs, True, context, terms)
             else:
                 params = self.autoregressive_net(outputs, context)
                 outputs, logabsdet = self._elementwise_inverse(inputs, params)
         return outputs, logabsdet
 
-    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse):
-        """MADE on the tensor cores (inference); `conditioner_inputs` feeds the MADE, `inputs` the bijection."""
-        params = tensorcore.params(self.autoregressive_net, conditioner_inputs)
+    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse, context=None, terms=None):
+        """MADE on the tensor cores (inference); `conditioner_inputs` feeds the MADE, `inputs` the bijection; `terms`:
+        the context terms of `context` when the caller has them already."""
+        params = tensorcore.params(self.autoregressive_net, conditioner_inputs, context=context, terms=terms)
         if inverse:
             return self._elementwise_inverse(inputs, params)
         return self._elementwise_forward(inputs, params)
@@ -102,10 +105,14 @@ class MaskedAffineAutoregressiveTransform(AutoregressiveTransform):
             return None
         return made_inverse.apply_affine(prog, inputs, _cabi.SCALE_SOFTPLUS_EPS)
 
-    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse):
-        return tensorcore.affine_layer(self.autoregressive_net, conditioner_inputs, inputs, None, None,
-                                       _cabi.AFFINE_INTERLEAVED, _cabi.SCALE_SOFTPLUS_EPS, inverse,
-                                       allow_inplace=not inverse)  # the inverse re-reads `inputs` D times
+    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse, context=None, terms=None):
+        net = self.autoregressive_net
+        if context is not None and not tensorcore.affine_fusable(net, inputs.shape[1], inputs.shape[1]):
+            return super()._tensorcore_layer(conditioner_inputs, inputs, inverse, context, terms)
+        return tensorcore.affine_layer(net, conditioner_inputs, inputs, None, None, _cabi.AFFINE_INTERLEAVED,
+                                       _cabi.SCALE_SOFTPLUS_EPS, inverse,
+                                       allow_inplace=not inverse,  # the inverse re-reads `inputs` D times
+                                       context=context, terms=terms)
 
 
 class MaskedSumOfSigmoidsTransform(AutoregressiveTransform):
@@ -134,12 +141,12 @@ class MaskedSumOfSigmoidsTransform(AutoregressiveTransform):
             return None
         return made_inverse.apply_sos(prog, inputs, self.n_sigmoids, -0.5, 50, 120.0)
 
-    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse):
+    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse, context=None, terms=None):
         net = self.autoregressive_net
         if (not inverse and conditioner_inputs is inputs
                 and tensorcore.sos_fusable(net, inputs.shape[1], self.n_sigmoids, inputs.shape[1])):
-            return tensorcore.sos_layer(net, inputs, inputs, self.n_sigmoids, -0.5)
-        return super()._tensorcore_layer(conditioner_inputs, inputs, inverse)
+            return tensorcore.sos_layer(net, inputs, inputs, self.n_sigmoids, -0.5, context, terms)
+        return super()._tensorcore_layer(conditioner_inputs, inputs, inverse, context, terms)
 
 
 class MaskedPiecewiseRationalQuadraticAutoregressiveTransform(AutoregressiveTransform):
@@ -189,13 +196,15 @@ class MaskedPiecewiseRationalQuadraticAutoregressiveTransform(AutoregressiveTran
             splines.check_status(status, tails)
         return outputs, logabsdet
 
-    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse):
+    def _tensorcore_layer(self, conditioner_inputs, inputs, inverse, context=None, terms=None):
         net = self.autoregressive_net
-        if not tensorcore.rqs_fusable(self._spline, net.final_layer.weight.shape[0], inputs.shape[1], net, inputs.shape[1]):
-            return super()._tensorcore_layer(conditioner_inputs, inputs, inverse)
+        if not tensorcore.rqs_fusable(self._spline, net.final_layer.weight.shape[0], inputs.shape[1], net, inputs.shape[1],
+                                      context):
+            return super()._tensorcore_layer(conditioner_inputs, inputs, inverse, context, terms)
         return tensorcore.rqs_layer(net, conditioner_inputs, inputs, self._spline, None, None, inverse,
                                     getattr(net, "hidden_features", None),
-                                    allow_inplace=not inverse)  # the inverse re-reads `inputs` D times
+                                    allow_inplace=not inverse,  # the inverse re-reads `inputs` D times
+                                    context=context, terms=terms)
 
 
 def _status_for(inputs, tails):

@@ -95,12 +95,12 @@ class CouplingTransform(Transform):
         if tensorcore.usable(self.transform_net, inputs, context):
             # inference: conditioner on the tensor cores; its first layer reads the full-width inputs through a
             # column-scattered weight, so the identity-column gather (coupling.py:82-86) disappears as well
-            return self._tensorcore_layer(inputs, inverse)
+            return self._tensorcore_layer(inputs, inverse, context)
         params = self.transform_net(inputs[:, self.identity_features], context)
         return self._coupling_layer(inputs, params, inverse)
 
-    def _tensorcore_layer(self, inputs, inverse):
-        params = tensorcore.params(self.transform_net, inputs, col_map=self._ccols, k_in=self.features)
+    def _tensorcore_layer(self, inputs, inverse, context=None):
+        params = tensorcore.params(self.transform_net, inputs, col_map=self._ccols, k_in=self.features, context=context)
         return self._coupling_layer(inputs, params, inverse)
 
     def _transform_dim_multiplier(self):
@@ -137,13 +137,15 @@ class AffineCouplingTransform(CouplingTransform):
         return ops.affine_layer(inputs, transform_params, self._tcols, self._ccols, _cabi.AFFINE_BLOCKED,
                                 self._activation_code, bool(inverse))
 
-    def _tensorcore_layer(self, inputs, inverse):
-        if self._transform_dim_multiplier() != 2:
-            return super()._tensorcore_layer(inputs, inverse)
+    def _tensorcore_layer(self, inputs, inverse, context=None):
+        net = self.transform_net
+        if self._transform_dim_multiplier() != 2 or (context is not None and not tensorcore.affine_fusable(
+                net, tensorcore.context_k_in(net, self.features, context), self.num_transform_features)):
+            return super()._tensorcore_layer(inputs, inverse, context)
         # final layer + scale-and-shift in one kernel
-        return tensorcore.affine_layer(self.transform_net, inputs, inputs, self._tcols, self._ccols,
-                                       _cabi.AFFINE_BLOCKED, self._activation_code, inverse, col_map=self._ccols,
-                                       k_in=self.features)
+        return tensorcore.affine_layer(net, inputs, inputs, self._tcols, self._ccols, _cabi.AFFINE_BLOCKED,
+                                       self._activation_code, inverse, col_map=self._ccols, k_in=self.features,
+                                       context=context)
 
 
 class AdditiveCouplingTransform(AffineCouplingTransform):
@@ -196,14 +198,14 @@ class PiecewiseRationalQuadraticCouplingTransform(CouplingTransform):
     def _coupling_layer(self, inputs, transform_params, inverse):
         return self._spline.apply(inputs, transform_params, self._tcols, self._ccols, inverse, self._scaling_width())
 
-    def _tensorcore_layer(self, inputs, inverse):
+    def _tensorcore_layer(self, inputs, inverse, context=None):
         net = self.transform_net
         if not tensorcore.rqs_fusable(self._spline, net.final_layer.weight.shape[0], self.num_transform_features, net,
-                                      self.features):
-            return super()._tensorcore_layer(inputs, inverse)
+                                      self.features, context):
+            return super()._tensorcore_layer(inputs, inverse, context)
         # final layer + spline in one kernel: the [B, D_t*P] parameter tensor never reaches HBM
         return tensorcore.rqs_layer(net, inputs, inputs, self._spline, self._tcols, self._ccols, inverse,
-                                    self._scaling_width(), col_map=self._ccols, k_in=self.features)
+                                    self._scaling_width(), col_map=self._ccols, k_in=self.features, context=context)
 
 
 class PiecewiseLinearCouplingTransform(CouplingTransform):

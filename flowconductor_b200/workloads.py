@@ -236,7 +236,7 @@ def build_flow(workload, seed=0):
             layers.append(transforms.PiecewiseRationalQuadraticCouplingTransform(
                 mask=make_mask(features, layer["mask"]),
                 transform_net_create_fn=lambda i, o, h=hidden, b=blocks: nets.ResidualNet(
-                    i, o, hidden_features=h, num_blocks=b),
+                    i, o, hidden_features=h, context_features=ctx, num_blocks=b),
                 num_bins=layer["num_bins"], tails=layer["tails"], tail_bound=layer["tail_bound"],
                 apply_unconditional_transform=layer.get("unconditional", False)))
         elif kind == "plin_coupling":
@@ -244,7 +244,7 @@ def build_flow(workload, seed=0):
             layers.append(transforms.PiecewiseLinearCouplingTransform(
                 mask=make_mask(features, layer["mask"]),
                 transform_net_create_fn=lambda i, o, h=hidden, b=blocks: nets.ResidualNet(
-                    i, o, hidden_features=h, num_blocks=b),
+                    i, o, hidden_features=h, context_features=ctx, num_blocks=b),
                 num_bins=layer["num_bins"], tails=layer["tails"], tail_bound=layer["tail_bound"],
                 apply_unconditional_transform=layer.get("unconditional", False)))
         elif kind == "pquad_coupling":
@@ -252,7 +252,7 @@ def build_flow(workload, seed=0):
             layers.append(transforms.PiecewiseQuadraticCouplingTransform(
                 mask=make_mask(features, layer["mask"]),
                 transform_net_create_fn=lambda i, o, h=hidden, b=blocks: nets.ResidualNet(
-                    i, o, hidden_features=h, num_blocks=b),
+                    i, o, hidden_features=h, context_features=ctx, num_blocks=b),
                 num_bins=layer["num_bins"], tails=layer["tails"], tail_bound=layer["tail_bound"],
                 apply_unconditional_transform=layer.get("unconditional", False)))
         elif kind == "pcubic_coupling":
@@ -260,7 +260,7 @@ def build_flow(workload, seed=0):
             layers.append(transforms.PiecewiseCubicCouplingTransform(
                 mask=make_mask(features, layer["mask"]),
                 transform_net_create_fn=lambda i, o, h=hidden, b=blocks: nets.ResidualNet(
-                    i, o, hidden_features=h, num_blocks=b),
+                    i, o, hidden_features=h, context_features=ctx, num_blocks=b),
                 num_bins=layer["num_bins"], tails=layer["tails"], tail_bound=layer["tail_bound"],
                 apply_unconditional_transform=layer.get("unconditional", False)))
         elif kind == "maf_pquad":
@@ -284,7 +284,7 @@ def build_flow(workload, seed=0):
             layers.append(transforms.AffineCouplingTransform(
                 mask=make_mask(features, layer["mask"]),
                 transform_net_create_fn=lambda i, o, h=hidden, b=blocks: nets.ResidualNet(
-                    i, o, hidden_features=h, num_blocks=b),
+                    i, o, hidden_features=h, context_features=ctx, num_blocks=b),
                 scale_activation=act))
         elif kind == "maf_affine":
             layers.append(transforms.MaskedAffineAutoregressiveTransform(

@@ -349,14 +349,28 @@ int fc_linear_debug_profile(unsigned long long* out16);
 #define FC_COND_BLOCK_FIRST 1  /* t = W relu(h) + b            (resnet.py:41-44) */
 #define FC_COND_BLOCK_SECOND 2 /* h = h + W relu(t) + b        (resnet.py:45-56) */
 #define FC_COND_FINAL 3        /* params = W h + b             (resnet.py:99, no activation in front) */
+/* Context terms (conditional nets, inference): a hidden layer may consume g = Wc ctx + bc, precomputed for the whole batch
+ * ([B, T] in the T128 layout, see FC_LINEAR_A_T128; fc_context_terms or fc_linear_apply with FC_LINEAR_OUT_T128).
+ * `terms` points at the layer's first column of that matrix (base + 128 * column floats, 16-byte aligned), `term_width`
+ * is T (a multiple of 16); column j of the layer's output consumes column j of `terms`.
+ *   ADD       block first of a residual MADE      t = W relu(h) + b + g                (made.py:170-181)
+ *   ADD_RELU  initial layer of a MADE             h = W x + b + relu(g)                (made.py:274-279)
+ *   GATE      block second of a ResidualNet       h = h + (W relu(t) + b) * sigmoid(g) (resnet.py:45-52: F.glu)
+ * A mode on another layer kind is FC_ERR_INVALID_ARGUMENT, a misaligned `terms` / term_width FC_ERR_UNSUPPORTED. */
+#define FC_COND_TERM_NONE 0
+#define FC_COND_TERM_ADD 1
+#define FC_COND_TERM_ADD_RELU 2
+#define FC_COND_TERM_GATE 3
 typedef struct fc_conditioner_layer {
   int32_t kind;      /* FC_COND_* */
   int32_t n_tiles;   /* N tiles: hidden / 128, or ceil(D_t / features per 96-column tile) for the final layer */
   int32_t relu_next; /* the following layer multiplies relu(result) */
-  int32_t reserved;
+  int32_t term_mode; /* FC_COND_TERM_* (0 for a net without context) */
   int64_t w_offset;  /* byte offset of the layer's packed weights inside `weights` (a multiple of 16) */
   const float* bias; /* device [n_tiles * bn] */
   const float* winv; /* device [2], see above */
+  const float* terms; /* device, T128 [B, term_width] from the layer's first column on; null with FC_COND_TERM_NONE */
+  int64_t term_width;
 } fc_conditioner_layer;
 typedef struct fc_conditioner {
   const void* weights; /* device, 16-byte aligned */
@@ -372,8 +386,10 @@ int fc_conditioner_pack_layer(const float* W, int64_t w_row_stride, const float*
                               int32_t n_pad, int32_t k_pad, int32_t bn, void* w_packed, float* bias_packed,
                               float* winv_packed, void* stream);
 /* a: the matrix the initial layer multiplies ([B, k_in], row stride lda; for a coupling layer the full-width inputs
- * with the identity-column gather folded into col_map, for a MADE the inputs).  x / y / logabsdet / tcols / ccols / cfg /
- * status exactly as for fc_linear_rqs_apply; y may alias x. */
+ * with the identity-column gather folded into col_map, for a MADE the inputs; for a conditional ResidualNet the context
+ * columns follow, [x | ctx]).  x / y / logabsdet / tcols / ccols / cfg / status exactly as for fc_linear_rqs_apply; y may
+ * alias x.  A conditional net (every fc_conditioner_*_apply): the layers with a term_mode read the context terms of this
+ * call (FC_COND_TERM_*, [B, T] in T128 from fc_context_terms or fc_linear_apply), bound in the layer table. */
 int fc_conditioner_rqs_apply(const fc_conditioner* net, const float* a, int64_t lda, int64_t B, const float* x,
                              int64_t x_row_stride, float* y, int64_t y_row_stride, float* logabsdet,
                              int32_t accumulate_logabsdet, int32_t D_t, fc_cols tcols, fc_cols ccols,
@@ -403,6 +419,12 @@ int fc_conditioner_affine_apply(const fc_conditioner* net, const float* a, int64
  * 96 columns. */
 int fc_conditioner_store_apply(const fc_conditioner* net, const float* a, int64_t lda, int64_t B, float* params,
                                int64_t params_row_stride, int32_t n_out, void* stream);
+/* The context terms of a conditional conditioner for narrow contexts (C <= 64, below the tensor-core GEMM's minimum
+ * reduction): out = ctx W^T + bias as [B, T] in the T128 layout (buffer of an even number of 128-row tiles; the rows
+ * beyond B of the last tiles are not written), fp32 FMA chains in k order.  ctx [B, C] (row stride ldc), W [T, C]
+ * row-major, bias [T]; T a multiple of 16. */
+int fc_context_terms(const float* ctx, int64_t ldc, int64_t B, int32_t C, const float* W, const float* bias, int32_t T,
+                     float* out, void* stream);
 /* Debugging aid: every barrier wait inside the kernel is bounded; if one ever times out the kernel ends early and leaves
  * a non-zero code (wait site + 100 * warp) here.  Synchronises the device.  Not part of the data path. */
 int fc_conditioner_error(int32_t* out);
