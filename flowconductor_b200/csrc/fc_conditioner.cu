@@ -1320,15 +1320,11 @@ static int cond_build_args(const fc_conditioner* net, const float* a, int64_t ld
   args.n_copy = ccols.n;
   args.D_t = D_t;
   args.status = status;
-  // Measured (scripts/sweep_cond_hand.sh): with two features per row thread and tile (8 bins) handing more to the
-  // bijection warps does not pay (cfg 2: 24.4 ms never, 24.9 every 2nd, 26.4 always), nor with 16-bin splines (cfg 3
-  // D-pass inverse 9.4 -> 10.8 ms at every 3rd tile); for the sum of sigmoids (one feature per thread and tile, the
-  // bijection warps would otherwise idle) every 3rd tile is best (cfg 4: 2.00 -> 1.90 ms).
-  static const int hand = [] {
-    const char* e = getenv("FC_COND_HAND");  // experiments: 0 = never hand everything over, n = every n-th final tile
-    return e && *e ? atoi(e) : -1;
-  }();
-  args.hand_period = hand >= 0 ? hand : hand_default;
+  // Measured: with two features per row thread and tile (8 bins) handing more to the bijection warps does not pay
+  // (cfg 2: 24.4 ms never, 24.9 every 2nd, 26.4 always), nor with 16-bin splines (cfg 3 D-pass inverse 9.4 -> 10.8 ms
+  // at every 3rd tile); for the sum of sigmoids (one feature per thread and tile, the bijection warps would otherwise
+  // idle) every 3rd tile is best (cfg 4: 2.00 -> 1.90 ms).
+  args.hand_period = hand_default;
   void* err_ptr = nullptr;
   if (cudaGetSymbolAddress(&err_ptr, g_cond_error) != cudaSuccess) return FC_ERR_CUDA;
   args.error = reinterpret_cast<int32_t*>(err_ptr);

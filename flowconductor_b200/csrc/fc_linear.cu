@@ -25,15 +25,16 @@
 // fp32 cuBLAS GEMM the reference runs (measured on K = 256 Gaussian operands, scripts/check_linear.py: rms error
 // 1.8e-6 undrained, 4.6e-7 at 64, 2.5e-7 at 32; cuBLAS fp32 2.9e-7).
 //
-// Kernel: persistent, one CTA per SM, 16 warps (register budget re-balanced with setmaxnreg):
+// Kernel: persistent, one CTA per SM, 16 warps (24 with the spline warps; register budget re-balanced with setmaxnreg):
 //   warp 0      TMA producer   : per stage one box of A (128 x BK) and the hi/lo boxes of W (BN x BK each)
 //   warp 1      UMMA issuer    : 3 x BK/8 tcgen05.mma (128 x BN x 8, kind::tf32) per stage, commit -> barriers
 //   warp 2      TMEM allocator
 //   warps 4-7   converters     : raw A tile -> (a_hi, a_lo)
 //   warps 8-15  epilogue       : tcgen05.ld each partial accumulator (double-buffered in TMEM, so draining chunk i
 //                                overlaps the MMAs of chunk i+1) into registers, then + bias and either
-//                                ReLU/residual/store, the rational-quadratic spline of 8 (K=8) / 4 (K=16)
-//                                features per 192-column tile, or the affine transform of 32 features per 64 columns.
+//                                ReLU/residual/store, the hand-over of the parameter tile to the spline warps, or the
+//                                affine transform of 32 features per 64 columns.
+//   warps 16-23 spline warps (EPI 1): the rational-quadratic spline of 8 (K=8) / 4 (K=16) features per 192-column tile.
 //   warp 3      staging manager (EPI 3): brings the skip connection into the staging tile and stores the finished tile —
 //                                one bulk copy for a T128 tile, four 2-D tensor-map boxes (128 rows x 32 columns,
 //                                128-byte swizzled rows) for a row-major result; split-K ranges land in consecutive
@@ -58,14 +59,20 @@ constexpr int kBM = 128;
 constexpr int kConvWarp0 = 4;
 constexpr int kEpiWarp0 = 8;
 constexpr int kNumConv = 128;  // converter threads (warps 4-7)
-// setmaxnreg budgets per warpgroup, EW epilogue warps (the register file holds 65536):
-//   EW = 8 : 512 threads launch with 128;  128*40 + 128*56 + 256*208 = 65536
-//   EW = 16: 768 threads launch with  80;  128*32 + 128*32 + 512*104 = 61440 (= 768 * 80, the CTA's pool)
-//   EW = 8 + 8 spline warps: 768 threads launch with 80;  128*32 + 128*64 + 256*120 + 256*72 = 61440
-template <int EW, int SW = 0>
+constexpr int kEpiWarps = 8;   // epilogue warps 8-15: two column groups, 4 warps (TMEM lane quarters) each
+
+// Kernel forms per epilogue (see the kernel comment): every kernel but the plain store (EPI 0) takes its activation
+// operand from tensor memory (TS), and the spline (EPI 1) runs on 8 warps of its own (SW).
+constexpr bool operand_in_tmem(int epi) { return epi != 0; }
+constexpr int spline_warps(int epi) { return epi == 1 ? 8 : 0; }
+
+// setmaxnreg budgets per warpgroup (the register file holds 65536):
+//   8 epilogue warps: 512 threads launch with 128;  128*40 + 128*56 + 256*208 = 65536
+//   8 epilogue + 8 spline warps: 768 threads launch with 80;  128*32 + 128*64 + 256*120 + 256*72 = 61440 (= 768 * 80,
+//   the CTA's pool)
+template <int SW>
 struct RegBudget {
-  static constexpr int kProducer = SW ? 32 : (EW == 8 ? 40 : 32), kConverter = SW ? 64 : (EW == 8 ? 56 : 32),
-                       kEpilogue = SW ? 120 : (EW == 8 ? 208 : 104), kSpline = 72;
+  static constexpr int kProducer = SW ? 32 : 40, kConverter = SW ? 64 : 56, kEpilogue = SW ? 120 : 208, kSpline = 72;
 };
 
 struct LinArgs {
@@ -113,15 +120,18 @@ struct RqsEpi {
   int activation;  // EPI 2 (affine): FC_SCALE_*; c.inverse carries the direction
 };
 
-template <int BN, int BK, int STAGES, int CTAS, bool TS = false, int SW = 0, bool STG = false>
+template <int EPI, int BN, int BK, int STAGES, int CTAS>
 struct LinSmem {
   static constexpr int A_BYTES = kBM * BK * 4;
   static constexpr int B_BYTES = (BN / CTAS) * BK * 4;  // a CTA pair splits the rows of every weight box
-  static constexpr int A_PLANES = TS ? 1 : 2;            // TS: the converted operand lives in tensor memory
+  static constexpr int A_PLANES = operand_in_tmem(EPI) ? 1 : 2;  // TS: the converted operand lives in tensor memory
   static constexpr int STAGE_BYTES = A_PLANES * A_BYTES + 2 * B_BYTES;
-  static constexpr int PARAMS_BYTES = (SW || STG) ? kBM * BN * 4 : 0;  // parameter tile (spline warps) / staging tile
+  // parameter tile (spline warps) / staging tile (EPI 3)
+  static constexpr int PARAMS_BYTES = (spline_warps(EPI) || EPI == 3) ? kBM * BN * 4 : 0;
   static constexpr int BAR_BYTES = 8 * (4 * STAGES + 6) + 16;
-  static constexpr int LAD_BYTES = (SW ? 2 : 2 * 3) * kBM * 4;  // per-row partial log-dets of the other column groups, x2
+  // per-row partial log-dets of the second thread group, double-buffered (spline warps: one row block per buffer; drain
+  // warps: buffers 3 row blocks apart, of which only the first is written)
+  static constexpr int LAD_BYTES = (spline_warps(EPI) ? 2 : 2 * 3) * kBM * 4;
   static constexpr int TOTAL = STAGES * STAGE_BYTES + PARAMS_BYTES + BAR_BYTES + LAD_BYTES + 1024;  // + alignment slack
   static_assert(A_BYTES % 1024 == 0 && B_BYTES % 1024 == 0, "operand tiles must keep 1024-byte alignment");
 };
@@ -173,37 +183,33 @@ __device__ __forceinline__ void drain_partial(uint32_t taddr, float* acc) {
 //          load and the result goes OUT by one TMA bulk store per 128 x 128 tile (contiguous 64 KB in the T128
 //          layout), issued by the otherwise idle warp 3; the epilogue warps never touch global memory.
 // RQS tile geometry: FEATS features of PPAD accumulator columns each (BN = FEATS * PPAD).
-// MODE 1: one CTA per SM, independent.
-// MODE 3: clusters of two CTAs work on two row tiles in lock step and SHARE the weight stream: each CTA fetches half
-//   of every weight box and TMA-multicasts it into both shared memories, which halves the L2 -> SM weight traffic
-//   (the weights are re-streamed for every 128-row tile: 512 KB per tile for a 256 x 256 layer, 1.5 MB for the final
-//   layer).  MMAs stay single-CTA; a ring slot is recycled once BOTH CTAs' MMAs have released it.
-// MODE 2: clusters of two CTAs (the two SMs of a TPC) that issue ONE tcgen05.mma.cta_group::2 (256 x BN x 8) per
+// Without PAIR every CTA works on its own row tile.
+// PAIR: clusters of two CTAs (the two SMs of a TPC) that issue ONE tcgen05.mma.cta_group::2 (256 x BN x 8) per
 //   product: each CTA stages its own 128 rows of A but only HALF of every weight box, so the weight traffic (L2 ->
 //   shared memory AND shared memory -> tensor core) per SM is halved and the ring is 1.5x deeper.  Rank 0 (the leader)
-//   issues the MMAs; rank 1's warp 1 relays "my stage is loaded and converted" to the leader.
-// TS: the converters write the (hi, lo) split of the activation tile into TENSOR MEMORY (tcgen05.st; ring of STAGES
-//   slots of 2*BK columns behind the two partial accumulators) and the MMAs take their A operand from there.  Per 8
-//   k-values the shared memory then serves 3 weight-tile reads + the TMA writes + one raw-tile read instead of 3 x
-//   (A + B) reads + TMA writes + raw read + two converted writes: 132 instead of 201 B/cycle at BN = 192 (the
+//   issues the MMAs; rank 1's converter and drain warps arrive on the leader's barriers.  Only TS kernels pair.
+// TS (EPI 1, 2, 3): the converters write the (hi, lo) split of the activation tile into TENSOR MEMORY (tcgen05.st; ring
+//   of STAGES slots of 2*BK columns behind the two partial accumulators) and the MMAs take their A operand from there.
+//   Per 8 k-values the shared memory then serves 3 weight-tile reads + the TMA writes + one raw-tile read instead of
+//   3 x (A + B) reads + TMA writes + raw read + two converted writes: 132 instead of 201 B/cycle at BN = 192 (the
 //   SMEM port delivers 128), and no generic->async proxy hand-off is needed.
-// SW > 0 (spline epilogue, with TS): the bijection moves to SW extra warps.  The drain warps only accumulate the
-//   partial sums and drop the finished parameter tile (128 rows x BN columns, column-major so that a warp's 32 rows are
-//   32 consecutive words) into shared memory; the spline warps evaluate it while the MMAs and drains of the NEXT tile
-//   run.  Without this the MMA warp can only run two partial accumulators ahead of the ~6k cycles the spline of a tile
-//   takes, and waits a third of the time.
-template <int EPI, int BN, int BK, int STAGES, int KC, int PPAD, int MODE, int EW, bool TS, int SW>
-__global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
+// SW (EPI 1): the bijection runs on 8 extra warps.  The drain warps only accumulate the partial sums and drop the
+//   finished parameter tile (128 rows x BN columns, column-major so that a warp's 32 rows are 32 consecutive words)
+//   into shared memory; the spline warps evaluate it while the MMAs and drains of the NEXT tile run.  Without this the
+//   MMA warp can only run two partial accumulators ahead of the ~6k cycles the spline of a tile takes, and waits a
+//   third of the time.
+template <int EPI, int BN, int BK, int STAGES, int KC, int PPAD, bool PAIR>
+__global__ void __launch_bounds__(kBaseThreads + 32 * (kEpiWarps + spline_warps(EPI)), 1)
     linear_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                          const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmR,
                          const LinArgs la, const StoreEpi se, const RqsEpi re) {
-  constexpr int CTAS = MODE == 2 ? 2 : 1;  // CTAs per MMA
-  constexpr bool MC = MODE == 3;           // weight boxes multicast inside the cluster
-  constexpr int CL = MODE == 1 ? 1 : 2;    // cluster size = row tiles per work unit
-  using SM = LinSmem<BN, BK, STAGES, CTAS, TS, SW, EPI == 3>;
-  static_assert(EPI != 3 || (TS && BN == 128 && EW == 8 && SW == 0 && MODE != 3), "staged store: 128-wide tiles, A in TMEM");
-  static_assert(SW == 0 || (EPI == 1 && EW == 8 && SW == 8), "spline warps: RQ epilogue, 8 + 8 warps");
-  static_assert(!TS || (MODE != 3 && 2 * BN + STAGES * 2 * BK <= 512), "TS: operand ring must fit behind the accumulators");
+  constexpr int CTAS = PAIR ? 2 : 1;  // CTAs per MMA = cluster size = row tiles per work unit
+  constexpr bool TS = operand_in_tmem(EPI);
+  constexpr int SW = spline_warps(EPI);
+  using SM = LinSmem<EPI, BN, BK, STAGES, CTAS>;
+  static_assert(EPI != 3 || BN == 128, "staged store: 128-wide tiles");
+  static_assert(!PAIR || TS, "CTA pairs take the activation operand from tensor memory");
+  static_assert(!TS || 2 * BN + STAGES * 2 * BK <= 512, "TS: operand ring must fit behind the accumulators");
   constexpr uint32_t kTmemA0 = 2 * BN;  // first column of the operand ring (TS)
   extern __shared__ unsigned char smem_raw[];
   const uint32_t raw_s = s32(smem_raw);
@@ -225,10 +231,10 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr uint32_t kTmemCols = 512;
   static_assert(2 * BN <= 512, "two partial accumulators must fit in tensor memory");
-  const int rank = CL == 2 ? (int)cluster_ctarank() : 0;
-  const int unit0 = (int)blockIdx.x / CL, unit_step = (int)gridDim.x / CL;  // cluster index / count
-  const int ks_n = la.k_slices;                                               // reduction ranges (split-K), else 1
-  const int n_units = ((la.num_m_tiles + CL - 1) / CL) * ks_n;               // work units: (row tile(s), range)
+  const int rank = CTAS == 2 ? (int)cluster_ctarank() : 0;
+  const int unit0 = (int)blockIdx.x / CTAS, unit_step = (int)gridDim.x / CTAS;  // cluster index / count
+  const int ks_n = la.k_slices;                                                   // reduction ranges (split-K), else 1
+  const int n_units = ((la.num_m_tiles + CTAS - 1) / CTAS) * ks_n;             // work units: (row tile(s), range)
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -236,16 +242,16 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(full_bar(s), 1);
       mbar_init(conv_bar(s), 4 * CTAS);  // one arrival per converter warp (of both CTAs of a pair, in the leader)
-      mbar_init(empty_bar(s), MC ? 2 : 1);
+      mbar_init(empty_bar(s), 1);
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), EW * CTAS);
+      mbar_init(tempty_bar(a), kEpiWarps * CTAS);
     }
     // SW: parameter tile full (drain warps) / empty (spline warps).  EPI 3: staging tile ready to be written (manager,
     // possibly through the skip connection's TMA bytes) / written by all epilogue warps
-    mbar_init(pfull_bar, EPI == 3 ? 1 : EW);
-    mbar_init(pempty_bar, EPI == 3 ? EW : (SW > 0 ? SW : 1));
+    mbar_init(pfull_bar, EPI == 3 ? 1 : kEpiWarps);
+    mbar_init(pempty_bar, EPI == 3 ? kEpiWarps : (SW > 0 ? SW : 1));
     fence_mbar_init();
   }
   if (warp == 2) {
@@ -256,8 +262,8 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
     }
   }
   tc_fence_before();
-  if (CL == 2) {
-    cluster_sync_all();  // barriers of both CTAs initialised before any remote arrive / multicast
+  if (CTAS == 2) {
+    cluster_sync_all();  // barriers of both CTAs initialised before any remote arrive
   } else {
     __syncthreads();
   }
@@ -270,14 +276,14 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
   const int n_chunks = (nk + chunk - 1) / chunk;
 
   if (warp < kConvWarp0) {
-    set_max_regs_dec<RegBudget<EW, SW>::kProducer>();
+    set_max_regs_dec<RegBudget<SW>::kProducer>();
     if (warp == 0) {
       // ---------------------------------------------------------------- TMA producer
       if (lane == 0) {
         int s = 0;
         uint32_t ph = 0;
         for (int mp = unit0; mp < n_units; mp += unit_step) {
-          const int mt = (mp / ks_n) * CL + rank;
+          const int mt = (mp / ks_n) * CTAS + rank;
           const int k_base = (mp % ks_n) * nk;  // first ring slot of this unit's reduction range (split-K)
           // The skip connection of the NEXT row tile of this CTA (one contiguous block in either layout) is pulled
           // into L2 slice by slice while this tile is computed: fetched by the epilogue in one burst from HBM it
@@ -285,7 +291,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
           const char* pf_base = nullptr;
           uint32_t pf_bytes = 0, pf_slice = 0;
           if (EPI == 0 && se.residual != nullptr) {
-            const int mt_next = ((mp + unit_step) / ks_n) * CL + rank;
+            const int mt_next = ((mp + unit_step) / ks_n) * CTAS + rank;
             if (mt_next < la.num_m_tiles) {
               const int64_t rows_left = (int64_t)la.M - (int64_t)mt_next * kBM;
               const int rows = se.tiled ? kBM : (rows_left < kBM ? (int)rows_left : kBM);
@@ -296,14 +302,14 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
           }
           uint32_t pf_done = 0;
           for (int nt = 0; nt < n_tiles; ++nt) {
-            const int brow = nt * BN + rank * (BN / CL);  // this CTA's share of the weight rows of the tile
+            const int brow = nt * BN + rank * (BN / CTAS);  // this CTA's share of the weight rows of the tile
             for (int kc = 0; kc < nk; ++kc) {
               if (pf_done < pf_bytes) {
                 const uint32_t nb = pf_bytes - pf_done < pf_slice ? pf_bytes - pf_done : pf_slice;
                 bulk_prefetch_l2(pf_base + pf_done, nb);
                 pf_done += nb;
               }
-              if (CL == 2) {
+              if (CTAS == 2) {
                 mbar_wait_cluster(empty_bar(s), ph ^ 1u);
               } else {
                 mbar_wait(empty_bar(s), ph ^ 1u);
@@ -317,16 +323,9 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
               } else {
                 tma_load_2d(st, &tmA, (k_base + kc) * BK, mt * kBM, full_bar(s));
               }
-              if (MC) {
-                const uint32_t half_off = (uint32_t)rank * (SM::B_BYTES / 2);
-                tma_load_2d_multicast(st + SM::A_PLANES * SM::A_BYTES + half_off, &tmB, (k_base + kc) * BK, brow, full_bar(s), 3);
-                tma_load_2d_multicast(st + SM::A_PLANES * SM::A_BYTES + SM::B_BYTES + half_off, &tmB, (k_base + kc) * BK, la.n_pad + brow,
-                                      full_bar(s), 3);
-              } else {
-                tma_load_2d(st + SM::A_PLANES * SM::A_BYTES, &tmB, (k_base + kc) * BK, brow, full_bar(s));
-                tma_load_2d(st + SM::A_PLANES * SM::A_BYTES + SM::B_BYTES, &tmB, (k_base + kc) * BK, la.n_pad + brow,
-                            full_bar(s));
-              }
+              tma_load_2d(st + SM::A_PLANES * SM::A_BYTES, &tmB, (k_base + kc) * BK, brow, full_bar(s));
+              tma_load_2d(st + SM::A_PLANES * SM::A_BYTES + SM::B_BYTES, &tmB, (k_base + kc) * BK, la.n_pad + brow,
+                          full_bar(s));
               if (++s == STAGES) {
                 s = 0;
                 ph ^= 1u;
@@ -341,7 +340,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
         constexpr uint32_t kTileBytes = kBM * BN * 4;
         uint32_t ph = 0;
         for (int mp = unit0; mp < n_units; mp += unit_step) {
-          const int mt = (mp / ks_n) * CL + rank;
+          const int mt = (mp / ks_n) * CTAS + rank;
           for (int nt = 0; nt < n_tiles; ++nt) {
             // a T128 tile of 128 rows x BN columns is contiguous: tile mt, column groups nt*BN/4 ..;
             // a row-major tile moves as BN/32 boxes of 128 rows x 32 columns (128-byte swizzled rows in the staging
@@ -450,10 +449,6 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
                         umma_tf32_ts(d, ta_hi, b_lo + o, idesc, 1u);
                         umma_tf32_ts(d, ta_hi, b_hi + o, idesc, 1u);
                       }
-                    } else if (CTAS == 2) {
-                      umma_tf32_ss_pair(d, a_lo + oa, b_hi + o, idesc, first);
-                      umma_tf32_ss_pair(d, a_hi + oa, b_lo + o, idesc, 1u);
-                      umma_tf32_ss_pair(d, a_hi + oa, b_hi + o, idesc, 1u);
                     } else {
                       umma_tf32_ss(d, a_lo + oa, b_hi + o, idesc, first);
                       umma_tf32_ss(d, a_hi + oa, b_lo + o, idesc, 1u);
@@ -462,8 +457,6 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
                   }
                   if (CTAS == 2) {
                     umma_commit_pair(empty_bar(s), 3);
-                  } else if (MC) {
-                    umma_commit_multicast(empty_bar(s), 3);
                   } else {
                     umma_commit(empty_bar(s));
                   }
@@ -500,7 +493,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
     }
   } else if (warp < kEpiWarp0) {
     // ------------------------------------------------------------------ converters: raw fp32 -> (hi, lo) tf32
-    set_max_regs_dec<RegBudget<EW, SW>::kConverter>();
+    set_max_regs_dec<RegBudget<SW>::kConverter>();
     const int ct = threadIdx.x - kConvWarp0 * 32;
     int s = 0;
     uint32_t ph = 0;
@@ -581,19 +574,11 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
           sts128(addr, h0, h1, h2, h3);
           sts128(addr + SM::A_BYTES, l0, l1, l2, l3);
         }
-        if (TS) {
-          // nothing was written to shared memory
-        } else if (CTAS == 2) {
-          fence_proxy_async_all();  // the reader is the leader's tensor core
-        } else {
-          fence_proxy_async_smem();
-        }
+        if (!TS) fence_proxy_async_smem();  // (TS: nothing was written to shared memory)
         __syncwarp();
         if (lane == 0) {
-          if (CTAS == 2 && TS) {
+          if (CTAS == 2) {
             mbar_arrive_remote_relaxed(conv_bar(s), 0);  // operand went to tensor memory: ordered by the tcgen05 fence
-          } else if (CTAS == 2) {
-            mbar_arrive_remote(conv_bar(s), 0);  // release.cluster: publishes this warp's part of the stage
           } else {
             mbar_arrive(conv_bar(s));
           }
@@ -609,7 +594,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
         }
       }
       if (TS && la.a_tiled == 2 && la.colsum != nullptr) {
-        const int mt = (mp / ks_n) * CL + rank;
+        const int mt = (mp / ks_n) * CTAS + rank;
         la.colsum[(int64_t)(mp % ks_n) * se.slice_stride + mt * kBM + (warp & 3) * 32 + lane] = csum;
       }
     }
@@ -617,24 +602,23 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
       g_lin_prof[12] = (unsigned long long)c_wait;
       g_lin_prof[13] = (unsigned long long)c_work;
     }
-  } else if (warp < kEpiWarp0 + EW) {
+  } else if (warp < kEpiWarp0 + kEpiWarps) {
     // ------------------------------------------------------------------ epilogue / drain warps
-    set_max_regs_inc<RegBudget<EW, SW>::kEpilogue>();
-    uint32_t pph = 0;  // phase of the parameter-tile hand-off (SW > 0)
-    constexpr int NG = EW / 4;               // column groups: 4 warps (one per TMEM lane quarter) each
-    constexpr int NCOL = BN / NG;            // accumulator columns (and registers) per thread
-    const int q = warp & 3;                  // TMEM lane quarter this warp may access
+    set_max_regs_inc<RegBudget<SW>::kEpilogue>();
+    uint32_t pph = 0;  // phase of the parameter-tile hand-off (SW > 0) / staging tile (EPI 3)
+    constexpr int NG = kEpiWarps / 4;          // column groups: 4 warps (one per TMEM lane quarter) each
+    constexpr int NCOL = BN / NG;              // accumulator columns (and registers) per thread
+    const int q = warp & 3;                    // TMEM lane quarter this warp may access
     const int half = (warp - kEpiWarp0) >> 2;  // which column group of the tile (columns / features)
     const uint32_t lane_sel = (uint32_t)(q * 32) << 16;
     int acc = 0;
     uint32_t aph = 0;
-    unsigned status = 0;
     int parity = 0;
     const bool eprof = FC_LINEAR_PROFILE && (la.debug & 4) && blockIdx.x == 0 && warp == kEpiWarp0;
     long long e_init = 0, e_wait = 0, e_drain = 0, e_final = 0, e_t = 0;
     const long long e_begin = clock64();
     for (int mp = unit0; mp < n_units; mp += unit_step) {
-      const int mt = (mp / ks_n) * CL + rank;
+      const int mt = (mp / ks_n) * CTAS + rank;
       const int64_t row = (int64_t)mt * kBM + q * 32 + lane;
       const bool valid = row < la.M;
       float lad_acc = 0.f;
@@ -642,12 +626,12 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
         float av[NCOL];
         if (eprof) e_t = clock64();
         // Start of the tile, while its first MMAs are still running: the register accumulators start from the bias
-        // (+ the skip connection), and the spline's inputs are fetched, so that no global-load latency is left
-        // between the last partial accumulator and the stores.
+        // (+ the skip connection), and the affine transform's inputs are fetched, so that no global-load latency is
+        // left between the last partial accumulator and the stores.
         const int rt = q * 32 + lane;
         int64_t o_base = 0, r_base = 0, n_mul = 1;
-        float xv[(EPI == 1 || EPI == 2) ? (BN / PPAD) / NG : 1];
-        int xcol[(EPI == 1 || EPI == 2) ? (BN / PPAD) / NG : 1];
+        float xv[EPI == 2 ? (BN / PPAD) / NG : 1];
+        int xcol[EPI == 2 ? (BN / PPAD) / NG : 1];
         if (EPI == 3) {
           const float4* b4 = reinterpret_cast<const float4*>(la.bias + nt * BN + half * NCOL);
 #pragma unroll
@@ -691,7 +675,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
         } else {
           constexpr int FEATS = BN / PPAD;
           constexpr int FH = FEATS / NG;
-          if (SW == 0 && nt == 0 && half == 0 && re.n_copy > 0 && re.y != re.x) {
+          if (EPI == 2 && nt == 0 && half == 0 && re.n_copy > 0 && re.y != re.x) {
             // identity columns (coupling.py:96-98): the warp copies its 32 rows one row per step (coalesced)
             const int64_t row0 = (int64_t)mt * kBM + q * 32;
             for (int i0 = 0; i0 < re.n_copy; i0 += 32) {
@@ -707,7 +691,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
             const int fl = half * FH + f;    // feature within the tile
             const int fg = nt * FEATS + fl;  // feature of the layer
             const bool live = fg < re.D_t;
-            if (SW == 0) {
+            if (EPI == 2) {
               xcol[f] = live ? (re.tcols ? __ldg(re.tcols + fg) : fg) : 0;
               xv[f] = (valid && live) ? __ldg(re.x + row * re.ldx + xcol[f]) : 0.f;
             }
@@ -822,7 +806,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
               *reinterpret_cast<float4*>(se.out + o_base + n * n_mul) = o;
             }
           }
-        } else if (SW > 0) {
+        } else if (EPI == 1) {
           // hand the finished parameter tile to the spline warps: column-major [BN][128 rows] words
           mbar_wait(pempty_bar, pph ^ 1u);
           const uint32_t pbase = params_s + (uint32_t)((half * NCOL) * kBM + q * 32 + lane) * 4u;
@@ -840,27 +824,21 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
             const int fg = nt * FEATS + half * FH + f;  // feature of the layer
             if (fg < re.D_t) {
               float yv, lv;
-              if constexpr (EPI == 2) {
-                affine_eval(xv[f], av[f * PPAD], av[f * PPAD + 1], re.activation, re.c.inverse, yv, lv);
-              } else {
-                rqs_eval<KC, true>(re.c, xv[f], av + f * PPAD, yv, lv, status);
-              }
+              affine_eval(xv[f], av[f * PPAD], av[f * PPAD + 1], re.activation, re.c.inverse, yv, lv);
               if (valid) re.y[row * re.ldy + xcol[f]] = yv;
               lad_acc += lv;
             }
           }
         }
       }
-      if ((EPI == 1 || EPI == 2) && SW == 0) {
+      if (EPI == 2) {
         // per-sample log|det J| (sum_except_batch, utils/torchutils.py:25-30): this thread summed its features in
         // order; the two column halves of a row are combined in a fixed order through shared memory
         float* ex = lad_x + parity * 3 * kBM;
-        if (half > 0) ex[(half - 1) * kBM + q * 32 + lane] = lad_acc;
-        named_barrier_sync(1, 32 * EW);
+        if (half > 0) ex[q * 32 + lane] = lad_acc;
+        named_barrier_sync(1, 32 * kEpiWarps);
         if (half == 0 && valid) {
-          float tot = lad_acc;
-#pragma unroll
-          for (int g = 1; g < NG; ++g) tot += ex[(g - 1) * kBM + q * 32 + lane];
+          const float tot = lad_acc + ex[q * 32 + lane];
           re.lad[row] = re.accumulate ? re.lad[row] + tot : tot;
         }
         parity ^= 1;
@@ -872,20 +850,19 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
       g_lin_prof[10] = (unsigned long long)e_wait;
       g_lin_prof[11] = (unsigned long long)e_drain;
     }
-    if ((EPI == 1 || EPI == 2) && status != 0 && re.status) atomicOr(re.status, (int)status);
   } else {
     // ------------------------------------------------------------------ spline warps (SW > 0)
     if constexpr (SW > 0) {
-      set_max_regs_dec<RegBudget<EW, SW>::kSpline>();
+      set_max_regs_dec<RegBudget<SW>::kSpline>();
       constexpr int FEATS = BN / PPAD;
       constexpr int FG = FEATS / 2;             // features per thread and tile: two thread groups of 128 rows
-      const int t = threadIdx.x - 32 * (kEpiWarp0 + EW);
+      const int t = threadIdx.x - 32 * (kEpiWarp0 + kEpiWarps);
       const int r = t & (kBM - 1), g = t >> 7;  // row of the tile, feature group
       uint32_t pph = 0;
       unsigned status = 0;
       int parity = 0;
       for (int mp = unit0; mp < n_units; mp += unit_step) {
-        const int mt = (mp / ks_n) * CL + rank;
+        const int mt = (mp / ks_n) * CTAS + rank;
         const int64_t row = (int64_t)mt * kBM + r;
         const bool valid = row < la.M;
         float lad_acc = 0.f;
@@ -954,7 +931,7 @@ __global__ void __launch_bounds__(kBaseThreads + 32 * (EW + SW), 1)
 
   __syncwarp();  // the role branches leave most warps diverged; the cluster barrier is warp-aligned
   tc_fence_before();
-  if (CL == 2) {
+  if (CTAS == 2) {
     cluster_sync_all();  // no CTA leaves (or frees tensor memory) while its partner can still signal it
   } else {
     __syncthreads();
@@ -1033,95 +1010,14 @@ static int make_map_t128(CUtensorMap* m, const float* ptr, uint64_t tiles, uint6
 
 // k-values per partial accumulator (see "Accumulation" at the top).  Short dot products leave less room between
 // the tensor core's truncation error and the (smaller) rounding noise of an fp32 FMA chain of the same length, so
-// they are drained after every stage.  FC_LINEAR_CHUNK_K overrides for experiments.
-static int chunk_k(int K) {
-  static int forced = [] {
-    const char* e = getenv("FC_LINEAR_CHUNK_K");
-    return e ? atoi(e) : 0;
-  }();
-  if (forced > 0) return forced < 16 ? 16 : forced;
-  return K <= 64 ? 16 : 32;
-}
+// they are drained after every stage.
+static int chunk_k(int K) { return K <= 64 ? 16 : 32; }
 
-// epilogue warps: 8 (two column groups, 208 registers each) or 16 (four column groups, 104 registers each)
-static int epilogue_warps() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_EW");
-    return e ? atoi(e) : 8;  // measured on cfg 2: 16 warps drain faster but take issue slots from the MMA warp; no gain
-  }();
-  return v == 16 ? 16 : 8;
-}
-
-// row-major results through the staged store kernel (TMA tensor-map stores); FC_LINEAR_STAGED_RM=0: direct stores from
-// the shared-memory-operand kernel
-static int staged_row_major() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_STAGED_RM");
-    return e ? atoi(e) : 1;
-  }();
-  return v != 0;
-}
-
-// activation operand in tensor memory (final-layer kernels, mode 1); FC_LINEAR_TS=0 switches back to shared memory
-static int operand_in_tmem() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_TS");
-    return e ? atoi(e) : 1;
-  }();
-  return v != 0;
-}
-
-// bijection on separate warps (FC_LINEAR_SW=0: inside the drain warps)
-static int spline_warps() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_SW");
-    return e ? atoi(e) : 1;
-  }();
-  return v != 0;
-}
-
-// cta_group::2 CTA pairs for the kernels whose operand lives in tensor memory (FC_LINEAR_PAIR=0: single CTAs)
-static int pair_mma() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_PAIR");
-    return e ? atoi(e) : 1;
-  }();
-  return v != 0;
-}
-
-// 32 k-values per ring slot in the staged pair kernel (FC_LINEAR_BK32=0: 16)
-static int wide_slots() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_BK32");
-    return e ? atoi(e) : 1;
-  }();
-  return v != 0;
-}
-
-// T128 outputs through the staged-store kernel (FC_LINEAR_STAGED=0: direct stores from the epilogue warps)
-static int staged_store() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_STAGED");
-    return e ? atoi(e) : 1;
-  }();
-  return v != 0;
-}
-
-// 1 = independent CTAs, 2 = CTA-pair MMAs (cta_group::2), 3 = weight multicast inside 2-CTA clusters
-static int cluster_mode() {
-  static int v = [] {
-    const char* e = getenv("FC_LINEAR_MODE");
-    return e ? atoi(e) : 1;
-  }();
-  return v >= 1 && v <= 3 ? v : 1;
-}
-
-template <int EPI, int BN, int BK, int STAGES, int KC, int PPAD, int MODE, int EW, bool TS = false, int SW = 0>
+template <int EPI, int BN, int BK, int STAGES, int KC, int PPAD, bool PAIR>
 static int launch_linear(const float* A, int64_t lda, int64_t M, int K, const fc_linear_weights* w, LinArgs la,
                          const StoreEpi& se, const RqsEpi& re, cudaStream_t stream) {
-  constexpr int CTAS = MODE == 2 ? 2 : 1;
-  constexpr int CL = MODE == 1 ? 1 : 2;
-  using SM = LinSmem<BN, BK, STAGES, CTAS, TS, SW, EPI == 3>;
+  constexpr int CTAS = PAIR ? 2 : 1;
+  using SM = LinSmem<EPI, BN, BK, STAGES, CTAS>;
   static_assert(SM::TOTAL <= 232448, "shared memory per CTA");
   if (w->n_pad % BN != 0 || w->k_pad % 32 != 0) return FC_ERR_INVALID_ARGUMENT;
   CUtensorMap tmA, tmB;
@@ -1129,7 +1025,7 @@ static int launch_linear(const float* A, int64_t lda, int64_t M, int K, const fc
            : la.a_tiled    ? make_map_t128(&tmA, A, (uint64_t)((M + kBM - 1) / kBM), (uint64_t)lda, BK)
                            : make_map(&tmA, A, (uint64_t)M, (uint64_t)K, (uint64_t)lda, kBM, BK);
   if (rc != FC_OK) return rc;
-  rc = make_map(&tmB, w->w, (uint64_t)2 * w->n_pad, (uint64_t)w->k_pad, (uint64_t)w->k_pad, BN / CL, BK);
+  rc = make_map(&tmB, w->w, (uint64_t)2 * w->n_pad, (uint64_t)w->k_pad, (uint64_t)w->k_pad, BN / CTAS, BK);
   if (rc != FC_OK) return rc;
   CUtensorMap tmO = tmA, tmR = tmA;  // only the staged store kernel with a row-major result reads these
   if (EPI == 3 && !se.tiled) {
@@ -1155,7 +1051,7 @@ static int launch_linear(const float* A, int64_t lda, int64_t M, int K, const fc
     return e ? atoi(e) : 0;
   }();
   la.debug = debug;
-  auto kern = linear_tf32x3_kernel<EPI, BN, BK, STAGES, KC, PPAD, MODE, EW, TS, SW>;
+  auto kern = linear_tf32x3_kernel<EPI, BN, BK, STAGES, KC, PPAD, PAIR>;
   // the opt-in shared-memory size is a per-device function attribute: set it once per (instantiation, device)
   static std::atomic<uint64_t> configured{0};
   int dev_id = 0;
@@ -1166,17 +1062,17 @@ static int launch_linear(const float* A, int64_t lda, int64_t M, int K, const fc
       return FC_ERR_CUDA;
     configured.fetch_or(dev_bit, std::memory_order_release);
   }
-  const int units = ((la.num_m_tiles + CL - 1) / CL) * la.k_slices;
-  const int max_units = device_info().sm_count / CL;
-  const int grid = (units < max_units ? units : max_units) * CL;
+  const int units = ((la.num_m_tiles + CTAS - 1) / CTAS) * la.k_slices;
+  const int max_units = device_info().sm_count / CTAS;
+  const int grid = (units < max_units ? units : max_units) * CTAS;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(kBaseThreads + 32 * (EW + SW));
+  cfg.blockDim = dim3(kBaseThreads + 32 * (kEpiWarps + spline_warps(EPI)));
   cfg.dynamicSmemBytes = SM::TOTAL;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
+  attr[0].val.clusterDim.x = CTAS;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
@@ -1217,11 +1113,9 @@ __global__ void pack_kernel(const float* __restrict__ W, int64_t ldw, const floa
   }
 }
 
-// Transposing producers for the split-K weight-gradient product: the reduction axis (the batch) has to be the contiguous
-// one for both operands.  128 x 32 tiles through shared memory, coalesced on both sides.
-//   kSplit = false: dst[c][r] = src[r][c]                       (grad_y [B, N] -> [N, B])
-//   kSplit = true : dst[0][c][r] = tf32_hi(src[r][c]), dst[1][c][r] = tf32(src[r][c] - hi)   (x [B, K] -> packed planes)
-template <bool kSplit>
+// Transposing weight producer for the split-K weight-gradient product: the reduction axis (the batch) has to be the
+// contiguous one.  128 x 32 tiles through shared memory, coalesced on both sides.
+//   dst[0][c][r] = tf32_hi(src[r][c]), dst[1][c][r] = tf32(src[r][c] - hi)   (x [B, K] -> packed planes)
 __global__ void __launch_bounds__(256) transpose_kernel(const float* __restrict__ src, int64_t lds, int64_t rows, int cols,
                                                         float* __restrict__ dst, int64_t ldd, int64_t plane_stride,
                                                         int relu) {
@@ -1253,24 +1147,20 @@ __global__ void __launch_bounds__(256) transpose_kernel(const float* __restrict_
     float hi[4], lo[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      if (kSplit) {
-        const uint32_t h = tc::to_tf32(e[j]);
-        hi[j] = __uint_as_float(h);
-        lo[j] = __uint_as_float(tc::to_tf32(e[j] - hi[j]));
-      } else {
-        hi[j] = e[j];
-      }
+      const uint32_t h = tc::to_tf32(e[j]);
+      hi[j] = __uint_as_float(h);
+      lo[j] = __uint_as_float(tc::to_tf32(e[j] - hi[j]));
     }
     float* d = dst + (int64_t)c * ldd + r;
     if (vec && r + 3 < rows) {
       *reinterpret_cast<float4*>(d) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-      if (kSplit) *reinterpret_cast<float4*>(d + plane_stride) = make_float4(lo[0], lo[1], lo[2], lo[3]);
+      *reinterpret_cast<float4*>(d + plane_stride) = make_float4(lo[0], lo[1], lo[2], lo[3]);
     } else {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         if (r + j < rows) {
           d[j] = hi[j];
-          if (kSplit) d[plane_stride + j] = lo[j];
+          d[plane_stride + j] = lo[j];
         }
       }
     }
@@ -1280,17 +1170,6 @@ __global__ void __launch_bounds__(256) transpose_kernel(const float* __restrict_
 }  // namespace fc
 
 using namespace fc;
-
-extern "C" int fc_linear_transpose(const float* src, int64_t src_row_stride, int64_t rows, int32_t cols, float* dst,
-                                   int64_t dst_row_stride, void* stream) {
-  if (rows < 0 || cols <= 0 || dst_row_stride < rows || src_row_stride < cols) return FC_ERR_INVALID_ARGUMENT;
-  if (rows == 0) return FC_OK;
-  if (!src || !dst) return FC_ERR_INVALID_ARGUMENT;
-  const dim3 grid((unsigned)((rows + 127) / 128), (unsigned)((cols + 31) / 32));
-  transpose_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(src, src_row_stride, rows, cols, dst, dst_row_stride, 0, 0);
-  FC_CHECK_LAUNCH();
-  return FC_OK;
-}
 
 extern "C" int fc_linear_pack_transposed(const float* X, int64_t x_row_stride, int64_t B, int32_t K, int32_t n_pad,
                                          int32_t k_pad, int32_t relu, float* w_packed, float* bias_packed,
@@ -1304,7 +1183,7 @@ extern "C" int fc_linear_pack_transposed(const float* X, int64_t x_row_stride, i
     return FC_ERR_CUDA;
   if (cudaMemsetAsync(bias_packed, 0, sizeof(float) * (size_t)n_pad, st) != cudaSuccess) return FC_ERR_CUDA;
   const dim3 grid((unsigned)((B + 127) / 128), (unsigned)((K + 31) / 32));
-  transpose_kernel<true><<<grid, 256, 0, st>>>(X, x_row_stride, B, K, w_packed, k_pad, (int64_t)n_pad * k_pad, relu);
+  transpose_kernel<<<grid, 256, 0, st>>>(X, x_row_stride, B, K, w_packed, k_pad, (int64_t)n_pad * k_pad, relu);
   FC_CHECK_LAUNCH();
   return FC_OK;
 }
@@ -1354,28 +1233,16 @@ extern "C" int fc_linear_apply(const float* A, int64_t lda, int64_t M, int32_t K
   if (w->n_pad % BN != 0) return FC_ERR_INVALID_ARGUMENT;
   la.num_n_tiles = (n_out + BN - 1) / BN;
   cudaStream_t st = (cudaStream_t)stream;
-  const bool experimental = cluster_mode() == 2 || cluster_mode() == 3 || epilogue_warps() == 16;
-  if (res_mask && experimental) return FC_ERR_UNSUPPORTED;
-  if (cluster_mode() == 2) return launch_linear<0, BN, 16, 6, 0, 32, 2, 8>(A, lda, M, K, w, la, se, re, st);
-  if (cluster_mode() == 3) return launch_linear<0, BN, 16, 4, 0, 32, 3, 8>(A, lda, M, K, w, la, se, re, st);
-  if (epilogue_warps() == 16) return launch_linear<0, BN, 16, 4, 0, 32, 1, 16>(A, lda, M, K, w, la, se, re, st);
-  if (o_tiled && staged_store() && n_out % 128 == 0 && (n_out == ldo) && (!residual || ldr == n_out)) {
-    // T128 output in whole 128-wide tiles: staged kernel (operand in TMEM, TMA bulk in / out)
-    la.num_n_tiles = n_out / 128;
-    // (short reductions keep 16-value slots: their partial accumulators are drained every 16 k-values)
-    if (pair_mma() && wide_slots() && K > 64)
-      return launch_linear<3, 128, 32, 4, 0, 32, 2, 8, true>(A, lda, M, K, w, la, se, re, st);
-    if (pair_mma()) return launch_linear<3, 128, 16, 8, 0, 32, 2, 8, true>(A, lda, M, K, w, la, se, re, st);
-    return launch_linear<3, 128, 16, 6, 0, 32, 1, 8, true>(A, lda, M, K, w, la, se, re, st);
-  }
-  if (!o_tiled && staged_store() && staged_row_major() && pair_mma() && w->n_pad % 128 == 0) {
-    // row-major result: same kernel, the staging tile leaves (and the skip connection arrives) through 2-D tensor maps
+  if (!o_tiled || n_out % 128 == 0) {
+    // staged kernel (operand in TMEM, CTA pairs): a T128 output in whole 128-wide tiles leaves by TMA bulk copies, a
+    // row-major one (the staging tile and the skip connection) through 2-D tensor maps
     la.num_n_tiles = (n_out + 127) / 128;
-    if (wide_slots() && K > 64) return launch_linear<3, 128, 32, 4, 0, 32, 2, 8, true>(A, lda, M, K, w, la, se, re, st);
-    return launch_linear<3, 128, 16, 8, 0, 32, 2, 8, true>(A, lda, M, K, w, la, se, re, st);
+    // (short reductions keep 16-value slots: their partial accumulators are drained every 16 k-values)
+    if (K > 64) return launch_linear<3, 128, 32, 4, 0, 32, true>(A, lda, M, K, w, la, se, re, st);
+    return launch_linear<3, 128, 16, 8, 0, 32, true>(A, lda, M, K, w, la, se, re, st);
   }
   if (res_mask) return FC_ERR_UNSUPPORTED;  // only the staged kernel gates
-  return launch_linear<0, BN, 16, 4, 0, 32, 1, 8>(A, lda, M, K, w, la, se, re, st);
+  return launch_linear<0, BN, 16, 4, 0, 32, false>(A, lda, M, K, w, la, se, re, st);
 }
 
 extern "C" int fc_linear_rqs_apply(const float* hidden, int64_t ldh, int64_t B, int32_t H, const fc_linear_weights* w,
@@ -1399,26 +1266,14 @@ extern "C" int fc_linear_rqs_apply(const float* hidden, int64_t ldh, int64_t B, 
   la.a_tiled = a_tiled;
   StoreEpi se{};
   RqsEpi re{x, x_row_stride, y, y_row_stride, logabsdet, accumulate_logabsdet, tcols.idx, ccols.idx, ccols.n, D_t, c, status};
+  if (c.K != 8 && c.K != 16) return FC_ERR_UNSUPPORTED;
   constexpr int BN = 192;
+  const int feats = BN / (3 * c.K);  // features per tile: 3K - 1 parameters padded to PP = 3K columns each
+  la.num_n_tiles = (D_t + feats - 1) / feats;
+  if (w->n_pad < la.num_n_tiles * BN) return FC_ERR_INVALID_ARGUMENT;
   cudaStream_t st = (cudaStream_t)stream;
-#define FC_RQS_DISPATCH(KBINS, PP)                                                                                       \
-  {                                                                                                                     \
-    la.num_n_tiles = (D_t + BN / PP - 1) / (BN / PP);                                                                   \
-    if (w->n_pad < la.num_n_tiles * BN) return FC_ERR_INVALID_ARGUMENT;                                                 \
-    if (cluster_mode() == 2) return launch_linear<1, BN, 16, 7, KBINS, PP, 2, 8>(hidden, ldh, B, H, w, la, se, re, st);  \
-    if (cluster_mode() == 3) return launch_linear<1, BN, 16, 5, KBINS, PP, 3, 8>(hidden, ldh, B, H, w, la, se, re, st);  \
-    if (epilogue_warps() == 16) return launch_linear<1, BN, 16, 5, KBINS, PP, 1, 16>(hidden, ldh, B, H, w, la, se, re, st); \
-    if (operand_in_tmem() && spline_warps() && pair_mma())                                                               \
-      return launch_linear<1, BN, 16, 4, KBINS, PP, 2, 8, true, 8>(hidden, ldh, B, H, w, la, se, re, st);               \
-    if (operand_in_tmem() && spline_warps())                                                                             \
-      return launch_linear<1, BN, 16, 4, KBINS, PP, 1, 8, true, 8>(hidden, ldh, B, H, w, la, se, re, st);               \
-    if (operand_in_tmem()) return launch_linear<1, BN, 16, 4, KBINS, PP, 1, 8, true>(hidden, ldh, B, H, w, la, se, re, st); \
-    return launch_linear<1, BN, 16, 5, KBINS, PP, 1, 8>(hidden, ldh, B, H, w, la, se, re, st);                           \
-  }
-  if (c.K == 8) FC_RQS_DISPATCH(8, 24)
-  if (c.K == 16) FC_RQS_DISPATCH(16, 48)
-#undef FC_RQS_DISPATCH
-  return FC_ERR_UNSUPPORTED;
+  if (c.K == 8) return launch_linear<1, BN, 16, 4, 8, 24, true>(hidden, ldh, B, H, w, la, se, re, st);
+  return launch_linear<1, BN, 16, 4, 16, 48, true>(hidden, ldh, B, H, w, la, se, re, st);
 }
 
 extern "C" int fc_linear_affine_apply(const float* hidden, int64_t ldh, int64_t B, int32_t H, const fc_linear_weights* w,
@@ -1444,9 +1299,7 @@ extern "C" int fc_linear_affine_apply(const float* hidden, int64_t ldh, int64_t 
   constexpr int BN = 64;  // 32 features per tile: the affine final layer is narrow (2 columns per feature)
   la.num_n_tiles = (2 * D_t + BN - 1) / BN;
   if (w->n_pad < la.num_n_tiles * BN) return FC_ERR_INVALID_ARGUMENT;
-  if (operand_in_tmem())
-    return launch_linear<2, BN, 16, 8, 0, 2, 1, 8, true>(hidden, ldh, B, H, w, la, se, re, (cudaStream_t)stream);
-  return launch_linear<2, BN, 16, 8, 0, 2, 1, 8>(hidden, ldh, B, H, w, la, se, re, (cudaStream_t)stream);
+  return launch_linear<2, BN, 16, 8, 0, 2, false>(hidden, ldh, B, H, w, la, se, re, (cudaStream_t)stream);
 }
 
 // Weight-gradient form of the split-K product: At is the A operand TRANSPOSED, [K, M] row-major (grad_y [B, N] as the
@@ -1474,25 +1327,5 @@ extern "C" int fc_linear_splitk_t_apply(const float* At, int64_t ldat, int64_t M
   StoreEpi se{partials, ldo, nullptr, 0, n_out, 0, 0, 0, slice_rows};
   RqsEpi re{};
   la.num_n_tiles = (n_out + 127) / 128;
-  return launch_linear<3, 128, 32, 4, 0, 32, 2, 8, true>(At, ldat, M, (int)K, w, la, se, re, (cudaStream_t)stream);
-}
-
-extern "C" int fc_linear_splitk_apply(const float* A, int64_t lda, int64_t M, int32_t K, const fc_linear_weights* w,
-                                      int32_t k_slices, float* partials, int64_t slice_stride, int64_t ldo,
-                                      int32_t n_out, void* stream) {
-  int rc = check_operand(A, lda, M, K, w, 0);
-  if (rc != FC_OK) return rc;
-  if (M == 0) return FC_OK;
-  if (!partials || n_out <= 0 || n_out > w->n_pad || k_slices < 1) return FC_ERR_INVALID_ARGUMENT;
-  if ((n_out & 3) || (ldo & 3) || (slice_stride & 3) || (reinterpret_cast<uintptr_t>(partials) & 15))
-    return FC_ERR_UNSUPPORTED;
-  if (slice_stride < M * ldo) return FC_ERR_INVALID_ARGUMENT;
-  LinArgs la{};
-  la.k_slices = k_slices;
-  StoreEpi se{partials, ldo, nullptr, 0, n_out, 0, 0, 0, slice_stride};
-  RqsEpi re{};
-  constexpr int BN = 256;
-  if (w->n_pad % BN != 0) return FC_ERR_INVALID_ARGUMENT;
-  la.num_n_tiles = (n_out + BN - 1) / BN;
-  return launch_linear<0, BN, 16, 4, 0, 32, 1, 8>(A, lda, M, K, w, la, se, re, (cudaStream_t)stream);
+  return launch_linear<3, 128, 32, 4, 0, 32, true>(At, ldat, M, (int)K, w, la, se, re, (cudaStream_t)stream);
 }

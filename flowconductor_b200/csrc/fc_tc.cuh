@@ -61,19 +61,9 @@ __device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity)
         : "memory");
   } while (!ok);
 }
-// arrive on the mbarrier at the same shared-memory offset in CTA `cta_rank` of this cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t cta_rank) {
-  asm volatile(
-      "{\n"
-      ".reg .b32 ra;\n"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n"
-      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n"
-      "}\n" ::"r"(bar),
-      "r"(cta_rank)
-      : "memory");
-}
-// same without memory ordering: for hand-offs whose data moves through tensor memory / the async proxy and is
-// ordered by tcgen05 fences (a cluster-scope release is a full fence and costs ~1k cycles)
+// arrive on the mbarrier at the same shared-memory offset in CTA `cta_rank` of this cluster, without memory ordering:
+// for hand-offs whose data moves through tensor memory / the async proxy and is ordered by tcgen05 fences (a
+// cluster-scope release is a full fence and costs ~1k cycles)
 __device__ __forceinline__ void mbar_arrive_remote_relaxed(uint32_t bar, uint32_t cta_rank) {
   asm volatile(
       "{\n"
@@ -92,7 +82,6 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 __device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 // generic-proxy writes to shared memory -> visible to the async proxy (TMA / UMMA operand reads)
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -106,17 +95,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* t, 
   asm volatile(
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
       "l"(t), "r"(c0), "r"(c1), "r"(bar)
-      : "memory");
-}
-
-// 2-D tiled load delivered to the same shared-memory offset (and signalled on the same barrier offset) in every
-// CTA of the cluster named in `cta_mask`
-__device__ __forceinline__ void tma_load_2d_multicast(uint32_t dst, const CUtensorMap* t, int c0, int c1, uint32_t bar,
-                                                      uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], "
-      "[%4], %5;" ::"r"(dst),
-      "l"(t), "r"(c0), "r"(c1), "r"(bar), "h"(cta_mask)
       : "memory");
 }
 // asynchronous prefetch of a contiguous global range into L2 (size a multiple of 16 bytes, 16-byte aligned)
@@ -176,30 +154,12 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-// single-CTA MMAs, but the arrival is delivered to the barrier at this offset in every CTA of `cta_mask`
-__device__ __forceinline__ void umma_commit_multicast(uint32_t bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(cta_mask)
-               : "memory");
-}
-// same, issued by the leader CTA of a pair: arrives on the barrier at this offset in every CTA of `cta_mask`
+// same for the MMAs of a CTA pair, issued by the leader: arrives on the barrier at this offset in every CTA of
+// `cta_mask`
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t cta_mask) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
                "h"(cta_mask)
                : "memory");
-}
-// 256 x N x 8 across a CTA pair (leader issues): each CTA supplies its 128 rows of A and N/2 rows of B from the
-// same shared-memory offsets, and receives its 128 accumulator rows (all N columns) in its own tensor memory
-__device__ __forceinline__ void umma_tf32_ss_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                                  uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(d_tmem),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
 }
 // D[tmem] (+)= A[tmem] * B[smem]^T: the A operand (128 rows = lanes, 8 tf32 values = 8 consecutive 32-bit columns)
 // is read from tensor memory

@@ -211,31 +211,6 @@ def linear_affine(hidden, packed, x, y, logabsdet, accumulate, d_t, tcols, ccols
     return y, logabsdet
 
 
-def linear_splitk(a, packed, k_slices=None):
-    """a @ W.T for a long reduction and a small output (fc_linear_splitk_apply): the reduction is cut into k_slices
-    ranges that run as independent work units; returns the sum of the partial products, [M, n_out].
-    `packed` must carry a zero bias."""
-    _cabi.require_cuda_f32(a, "activations")
-    L = _cabi.lib()
-    a, ap, lda = _cabi.rows(a)
-    M, K = a.shape
-    if K != packed.k_in:
-        raise ValueError("activations have {} columns, the packed layer expects {}".format(K, packed.k_in))
-    n4 = (packed.n_out + 3) // 4 * 4
-    if k_slices is None:
-        # enough (row tile, range) units for ~2 per SM, at least 2048 reduction steps each
-        tiles = (M + 127) // 128
-        sms = torch.cuda.get_device_properties(a.device).multi_processor_count
-        k_slices = max(1, min((2 * sms + tiles - 1) // tiles, K // 2048))
-    partials = torch.empty((k_slices, M, n4), dtype=torch.float32, device=a.device)
-    with torch.cuda.device(a.device), _cabi.launch("fc_linear_splitk_apply", a.device):
-        rc = L.fc_linear_splitk_apply(ap, lda, M, K, ctypes.byref(packed.struct), k_slices, partials.data_ptr(),
-                                      M * n4, n4, n4, _cabi.stream_ptr(a.device))
-    _cabi.check(rc, "fc_linear_splitk_apply")
-    out = partials[0] if k_slices == 1 else partials.sum(0)
-    return out if n4 == packed.n_out else out[:, :packed.n_out]
-
-
 def linear_splitk_t(a_t, packed, k_slices=None, column_sums=False):
     """a_t.T @ W.T for a_t given TRANSPOSED ([K, M] row-major, e.g. grad_y [B, N]) — fc_linear_splitk_t_apply: the
     weight-gradient product without a transposed copy of grad_y.  Returns [M, n_out]; `packed` must carry a zero bias.
@@ -268,21 +243,8 @@ def linear_splitk_t(a_t, packed, k_slices=None, column_sums=False):
     return out
 
 
-def transpose(t):
-    """[rows, cols] -> [cols, rows] (fc_linear_transpose; coalesced on both sides)."""
-    _cabi.require_cuda_f32(t, "matrix")
-    L = _cabi.lib()
-    t, tp, ld = _cabi.rows(t)
-    rows, cols = t.shape
-    out = torch.empty((cols, rows), dtype=torch.float32, device=t.device)
-    with torch.cuda.device(t.device), _cabi.launch("fc_linear_transpose", t.device):
-        rc = L.fc_linear_transpose(tp, ld, rows, cols, out.data_ptr(), rows, _cabi.stream_ptr(t.device))
-    _cabi.check(rc, "fc_linear_transpose")
-    return out
-
-
 def pack_transposed(x, n_tile=N_TILE_STORE, relu=False):
-    """Packed hi / lo planes of x^T (zero bias) for linear_splitk: x [B, K] -> PackedLinear with n_out = K, k_in = B.
+    """Packed hi / lo planes of x^T (zero bias) for linear_splitk_t: x [B, K] -> PackedLinear with n_out = K, k_in = B.
     relu=True packs max(x, 0)."""
     _cabi.require_cuda_f32(x, "activations")
     L = _cabi.lib()

@@ -7,7 +7,7 @@ flowcon/transforms/made.py:71-72) as an autograd function whose forward and inpu
     forward   y  = x  @ (W*mask)^T + b          tensor cores
     backward  gx = gy @ (W*mask)                tensor cores (the packed operand is the transposed weight)
               gW = (gy^T @ x) * mask            tensor cores, split-K: the reduction runs over the batch, so it is cut
-              gb = gy.sum(0)                    into ranges that run as independent work units (fc_linear_splitk_apply)
+              gb = gy.sum(0)                    into ranges that run as independent work units (fc_linear_splitk_t_apply)
 
 The weights change every optimizer step, so they are re-packed on every call (two tiny kernels per layer).
 Anything the kernel does not cover (CPU tensors, other dtypes, misaligned operands) takes F.linear.
@@ -18,12 +18,6 @@ from torch.nn import functional as F
 from .. import linear as fl
 
 ENABLED = True
-# Weight gradients through fc_linear_splitk_apply: grad_y and x are transposed by fc_linear_transpose /
-# fc_linear_pack_transposed (the batch has to be the contiguous reduction axis; x is split into its hi / lo planes on the
-# way), then one split-K product.  Measured over 262144 rows: 256 x 256: 0.60 ms (0.135 + 0.19 + 0.28) vs 0.77 ms for the
-# cuBLAS fp32 torch.mm; 752 x 256: 1.40 vs 2.03 ms.
-WGRAD_TC = True
-WGRAD_T = True  # grad_y enters the weight-gradient product untransposed (fc_linear_splitk_t_apply)
 # Shortest reduction the tensor-core GEMM is used for.  Every 3xTF32 product carries ~2^-22 relative error (dropped
 # lo*lo term, truncation inside the MMA); an fp32 FMA chain rounds at 2^-24 per step, so its error grows with the
 # chain length.  Measured (scripts/check_linear.py, Gaussian operands): at K = 32 the tensor-core result is 1.3x
@@ -75,7 +69,7 @@ def _wgrad(gy, x, weight, mask, want_bias, relu_x=False):
     """(grad_W, grad_b or None) of y = relu?(x) @ (W*mask)^T + b for upstream gy."""
     gb = None
     # (the reduction runs over the batch, so a narrow layer input does not shorten it: no MIN_K condition here)
-    if (WGRAD_TC and WGRAD_T and x.shape[0] >= 4096 and x.shape[0] % 4 == 0 and gy.shape[1] % 4 == 0
+    if (x.shape[0] >= 4096 and x.shape[0] % 4 == 0 and gy.shape[1] % 4 == 0
             and x.stride(1) == 1 and x.stride(0) % 4 == 0 and x.data_ptr() % 16 == 0):
         xt = fl.pack_transposed(x, relu=relu_x)
         if want_bias:
@@ -176,7 +170,7 @@ class _TCWgradLinear(torch.autograd.Function):
 
 def linear(x, weight, bias=None, mask=None):
     if not _eligible(x, weight) or gy_misaligned(weight):
-        if (ENABLED and WGRAD_TC and WGRAD_T and x.is_cuda and x.dtype == torch.float32 and x.dim() == 2
+        if (ENABLED and x.is_cuda and x.dtype == torch.float32 and x.dim() == 2
                 and weight.dtype == torch.float32 and x.shape[0] >= 4096 and x.shape[0] % 4 == 0
                 and weight.shape[0] % 4 == 0 and weight.shape[0] >= MIN_K and weight.requires_grad
                 and torch.is_grad_enabled()):

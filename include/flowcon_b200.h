@@ -259,21 +259,13 @@ int fc_linear_apply(const float* A, int64_t lda, int64_t M, int32_t K, const fc_
 /*
  * Split-K form for products whose reduction is long and whose output is small — the weight gradient of a dense
  * layer, grad_W[N, K_in] = grad_y^T[N, B] * x[B, K_in]^T-packed, reduces over the whole batch (autograd of
- * resnet.py:26-28 / made.py:71-72; the reference leaves it to torch.mm).  The reduction range [0, K) is cut into
- * k_slices ranges, every (row tile, range) pair is one work unit, and range s writes its partial product to
- * partials + s * slice_stride (row stride ldo); the caller sums the k_slices partial results.  `w` must have been packed
- * with a zero bias.  A: row-major [M, K], 16-byte aligned rows.
- */
-int fc_linear_splitk_apply(const float* A, int64_t lda, int64_t M, int32_t K, const fc_linear_weights* w,
-                           int32_t k_slices, float* partials, int64_t slice_stride, int64_t ldo, int32_t n_out,
-                           void* stream);
-
-/*
- * The same product with the A operand given TRANSPOSED: At is [K, M] row-major with row stride ldat — for a weight
- * gradient simply grad_y [B, N] as the backward pass holds it, so no transposed copy of grad_y is written
- * (fc_linear_transpose is not needed).  Range s writes rows [s * slice_rows, s * slice_rows + M) of the row-major
- * matrix `partials` ([k_slices * slice_rows, ldo]); slice_rows >= M must be a multiple of 256 (rows M.. of a range
- * are scratch).  `w` as above (fc_linear_pack_transposed of x), zero bias.  colsum: NULL, or [k_slices][slice_rows]
+ * resnet.py:26-28 / made.py:71-72; the reference leaves it to torch.mm).  The A operand is given TRANSPOSED: At is
+ * [K, M] row-major with row stride ldat — for a weight gradient simply grad_y [B, N] as the backward pass holds it, so
+ * no transposed copy of grad_y is written.  The reduction range [0, K) is cut into k_slices ranges, every (row tile,
+ * range) pair is one work unit, and range s writes its partial product to rows [s * slice_rows, s * slice_rows + M) of
+ * the row-major matrix `partials` ([k_slices * slice_rows, ldo]); the caller sums the k_slices partial results.
+ * slice_rows >= M must be a multiple of 256 (rows M.. of a range are scratch).  `w` is x packed by
+ * fc_linear_pack_transposed (zero bias).  colsum: NULL, or [k_slices][slice_rows]
  * floats that receive, per range, the column sums of At (entry s * slice_rows + m = sum over the range's rows k of
  * At[k][m]); their sum over s is grad_y.sum(0), the bias gradient, for free.
  */
@@ -281,10 +273,8 @@ int fc_linear_splitk_t_apply(const float* At, int64_t ldat, int64_t M, int64_t K
                              int32_t k_slices, float* partials, int64_t slice_rows, int64_t ldo, int32_t n_out,
                              float* colsum, void* stream);
 
-/* Operand producers for fc_linear_splitk_apply (the batch has to be the contiguous reduction axis of both operands):
- * dst[c, r] = src[r, c], and the packed hi / lo planes of X^T (zero bias): packed row c = column c of X. */
-int fc_linear_transpose(const float* src, int64_t src_row_stride, int64_t rows, int32_t cols, float* dst,
-                        int64_t dst_row_stride, void* stream);
+/* Weight operand for fc_linear_splitk_t_apply (the batch has to be its contiguous reduction axis): the packed hi / lo
+ * planes of X^T (zero bias): packed row c = column c of X. */
 int fc_linear_pack_transposed(const float* X, int64_t x_row_stride, int64_t B, int32_t K, int32_t n_pad, int32_t k_pad,
                               int32_t relu /* pack max(X, 0): the layer's input went through F.relu */,
                               float* w_packed, float* bias_packed, void* stream);

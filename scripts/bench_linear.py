@@ -1,5 +1,5 @@
-"""Micro-benchmark of the two tensor-core kernels on cfg-2 shapes (env knobs: FC_LINEAR_CTAS, FC_LINEAR_CHUNK_K,
-FC_LINEAR_DEBUG)."""
+"""Micro-benchmark of the two tensor-core kernels on cfg-2 shapes (FC_LINEAR_DEBUG=4 with a profiling build also prints
+the wait-cycle counters)."""
 import math, os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -51,9 +51,7 @@ print("  " + "  ".join("{} {:.3f}".format(k, t) for k, t in v.items()))
 t2 = timeit(lambda: fl.linear_rqs(a, pkf, x, y, lad, False, d_t, tcols, ccols, cfg, None))
 t2i = timeit(lambda: fl.linear_rqs(at, pkf, x, x, lad, False, d_t, tcols, ccols, cfg, None))
 print("final+spline in place, T128 hidden: {:.3f} ms".format(t2i))
-print("mode={} chunk={} debug={}: hidden {:.3f} ms   final+spline {:.3f} ms".format(
-    os.environ.get("FC_LINEAR_MODE", "-"), os.environ.get("FC_LINEAR_CHUNK_K", "-"), os.environ.get("FC_LINEAR_DEBUG", "0"),
-    t1, t2))
+print("hidden {:.3f} ms   final+spline {:.3f} ms".format(t1, t2))
 
 if int(os.environ.get("FC_LINEAR_DEBUG", "0")) & 4:
     import ctypes

@@ -1,4 +1,4 @@
-"""Weight-gradient product grad_W = grad_y^T x over 262144 rows: the three implementations side by side."""
+"""Weight-gradient product grad_W = grad_y^T x: torch.mm against the split-K tensor-core product, and its k-slice sweep."""
 import os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -25,15 +25,12 @@ for B, N, K in [(262144, 256, 256), (262144, 752, 256), (32768, 256, 256)]:
     gy = torch.randn(B, N, generator=g, device=dev)
     x = torch.randn(B, K, generator=g, device=dev)
     t_mm = timeit(lambda: gy.t().mm(x))
-    t_old = timeit(lambda: fl.linear_splitk(fl.transpose(gy), fl.pack_transposed(x)))
     t_new = timeit(lambda: fl.linear_splitk_t(gy, fl.pack_transposed(x)))
     t_pack = timeit(lambda: fl.pack_transposed(x))
-    t_tr = timeit(lambda: fl.transpose(gy))
     pk = fl.pack_transposed(x)
     t_gemm = timeit(lambda: fl.linear_splitk_t(gy, pk))
-    print("B={} N={} K={}: torch.mm {:.3f} ms | transposes + split-K {:.3f} | untransposed grad_y {:.3f} "
-          "(pack x^T {:.3f}, product + slice sum {:.3f}; transpose of grad_y was {:.3f})".format(
-              B, N, K, t_mm, t_old, t_new, t_pack, t_gemm, t_tr), flush=True)
+    print("B={} N={} K={}: torch.mm {:.3f} ms | split-K {:.3f} (pack x^T {:.3f}, product + slice sum {:.3f})".format(
+        B, N, K, t_mm, t_new, t_pack, t_gemm), flush=True)
 
 # reduction ranges per product at a small per-GPU shard (the 8-GPU cfg-3 step: 32768 rows per rank)
 B, N, K = 32768, 256, 256

@@ -228,7 +228,6 @@ def main():
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     gen = torch.Generator(device=dev).manual_seed(0)
-    print("variant", os.environ.get("FC_LINEAR_VARIANT", "0"))
     ok = True
     t0 = time.time()
     ok &= check_store(128, 32, 256, False, False, False, gen, dev)

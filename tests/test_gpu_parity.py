@@ -500,16 +500,13 @@ def test_linear_store_kernels(dev, M, K, N, relu_in, relu_out, res, a_t, o_t):
 
 @pytest.mark.parametrize("N,K,B,slices", [(256, 256, 8192, None), (752, 256, 20000, 7), (64, 100, 4096, 1),
                                           (256, 256, 131072, None)])  # 148 ranges: two work units per CTA pair
-def test_linear_splitk_weight_gradient_shape(dev, N, K, B, slices):
-    """fc_linear_splitk_apply: grad_W = grad_y^T @ x as a split-K product over the batch, against fp64."""
+def test_linear_splitk_t_weight_gradient_shape(dev, N, K, B, slices):
+    """fc_linear_splitk_t_apply: grad_W = grad_y^T @ x as a split-K product over the batch, against fp64."""
     from flowconductor_b200 import linear as fl
 
     g = torch.Generator(device=dev).manual_seed(N + B)
     gy = torch.randn(B, N, generator=g, device=dev)
     x = torch.randn(B, K, generator=g, device=dev)
-    got = fl.linear_splitk(gy.t().contiguous(), fl.pack(x.t().contiguous(), None), k_slices=slices)
-    got2 = fl.linear_splitk(fl.transpose(gy), fl.pack_transposed(x), k_slices=slices)  # the fused operand producers
-    assert torch.equal(got, got2)
     # grad_y untransposed (operand via TMEM), bias gradient accumulated on the way
     got3, colsum = fl.linear_splitk_t(gy, fl.pack_transposed(x), k_slices=slices, column_sums=True)
     assert torch.equal(got3, fl.linear_splitk_t(gy, fl.pack_transposed(x), k_slices=slices))
@@ -519,8 +516,7 @@ def test_linear_splitk_weight_gradient_shape(dev, N, K, B, slices):
         2e-6 * want_cs.abs().max()
     want = gy.double().t() @ x.double()
     ref32 = gy.t() @ x
-    assert got.shape == (N, K) and got3.shape == (N, K)
-    assert _gemm_err(got, want) <= 2.0 * _gemm_err(ref32, want) + 2e-7
+    assert got3.shape == (N, K)
     assert _gemm_err(got3, want) <= 2.0 * _gemm_err(ref32, want) + 2e-7
 
 
@@ -831,13 +827,12 @@ def test_short_reduction_layer_keeps_tensor_core_weight_gradient(dev, monkeypatc
 
 
 @pytest.mark.parametrize("rows,cols", [(4099, 100), (128, 32), (1000, 256), (5, 3)])
-def test_transposing_operand_producers(dev, rows, cols):
-    """fc_linear_transpose / fc_linear_pack_transposed on ragged shapes (vector and scalar store paths)."""
+def test_pack_transposed_ragged_shapes(dev, rows, cols):
+    """fc_linear_pack_transposed on ragged shapes (vector and scalar store paths)."""
     from flowconductor_b200 import linear as fl
 
     g = torch.Generator(device=dev).manual_seed(rows)
     x = torch.randn(rows, cols, generator=g, device=dev)
-    assert torch.equal(fl.transpose(x), x.t().contiguous())
     for relu in (False, True):
         pk = fl.pack_transposed(x, relu=relu)
         planes = pk.w  # [2, n_pad, k_pad]: tf32 hi / lo planes of x^T, zero padded
