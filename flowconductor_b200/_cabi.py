@@ -23,7 +23,7 @@ LINEAR_A_T128, LINEAR_OUT_T128, LINEAR_RESIDUAL_GATES = 1, 2, 4
 
 EXPORTS = ["fc_rqs_apply", "fc_rqs_backward", "fc_rqs_bins", "fc_linspline_apply", "fc_linspline_backward",
            "fc_quadspline_apply", "fc_quadspline_backward", "fc_cubicspline_apply", "fc_cubicspline_backward", "fc_affine_apply", "fc_affine_backward", "fc_sos_apply",
-           "fc_sos_backward", "fc_stdnormal_log_prob", "fc_linear_pack", "fc_linear_apply", "fc_linear_rqs_apply",
+           "fc_sos_backward", "fc_sos_inverse_backward", "fc_stdnormal_log_prob", "fc_linear_pack", "fc_linear_apply", "fc_linear_rqs_apply",
            "fc_linear_affine_apply", "fc_linear_splitk_t_apply", "fc_linear_pack_transposed",
            "fc_linear_debug_profile",
            "fc_elementwise_last_path", "fc_conditioner_layer_bytes", "fc_conditioner_pack_layer", "fc_conditioner_rqs_apply", "fc_conditioner_sos_apply", "fc_conditioner_affine_apply", "fc_conditioner_store_apply", "fc_context_terms", "fc_conditioner_error", "fc_conditioner_profile",
@@ -119,6 +119,7 @@ def lib():
                                          i32, i32, vp]
         L.fc_sos_apply.argtypes = [vp, i64, vp, i64, vp, i64, vp, i32, i64, i32, i32, f32, i32, i32, f32, vp]
         L.fc_sos_backward.argtypes = [vp, i64, vp, i64, vp, i64, vp, vp, i64, vp, i64, i64, i32, i32, vp]
+        L.fc_sos_inverse_backward.argtypes = L.fc_sos_backward.argtypes
         L.fc_stdnormal_log_prob.argtypes = [vp, i64, vp, vp, i64, i32, vp]
         L.fc_linear_pack.argtypes = [vp, i64, vp, i64, vp, i32, i32, vp, vp, i32, i32, vp, vp, vp]
         L.fc_linear_apply.argtypes = [vp, i64, i64, i32, ctypes.POINTER(LinearWeights), i32, vp, i64, i32, i32, vp,

@@ -1186,7 +1186,13 @@ FC_HD void sos_backward_esp(float x, float er, float& j_esp, float& dj_dx, float
   dj_ds = -dsp - dsn;
 }
 
-template <int NC>
+// kInverse: the adjoint of the numerical inverse (fc_sos_inverse_backward).  x is then the inverse's output, z = f(x),
+// gy and gl are the upstream gradients of x and of the inverse's log-derivative -log J(x).  With J_x = d log J / dx,
+//   dL/dz = (gy - gl J_x) / J,
+// and since dx/dtheta = -(df/dtheta) / J, the raw-parameter gradient is the forward adjoint at x with upstream
+// (gy, gl) := (-dL/dz, -gl).  Pass 1 (the totals) does not depend on the upstream gradients, so the swap happens
+// between the two passes; gx receives dL/dz.
+template <int NC, bool kInverse = false>
 FC_HD void sos_backward_elem_t(float x, const float* raw, int n_runtime, float gy, float gl, float& gx, float* graw) {
   if constexpr (NC > 0 && (NC % 2 == 0)) {
     // MUFU-lean path: two passes instead of three (the softmax dot product sum_j p_j dL/dw_j is linear in the
@@ -1221,8 +1227,14 @@ FC_HD void sos_backward_elem_t(float x, const float* raw, int n_runtime, float g
     float j_esp, dj_esp_dx, dy_esp_ds, dj_esp_ds, ds_der;
     sos_backward_esp(x, raw[3 * NC], j_esp, dj_esp_dx, dy_esp_ds, dj_esp_ds, ds_der);
     const float J = fmaxf(jac + j_esp, 1e-37f);
-    const float gJ = gl * fc_rcp(J);
-    gx = gy * (jac + j_esp) + gJ * (djac_dx + dj_esp_dx);
+    float gJ = gl * fc_rcp(J);
+    if constexpr (kInverse) {  // see the comment above sos_backward_elem_t
+      gx = (gy - gJ * (djac_dx + dj_esp_dx)) * fc_rcp(J);
+      gy = -gx;
+      gJ = -gJ;
+    } else {
+      gx = gy * (jac + j_esp) + gJ * (djac_dx + dj_esp_dx);
+    }
     graw[3 * NC] = (gy * dy_esp_ds + gJ * dj_esp_ds) * ds_der;
     const float dot = (gy * (S1 - ysum * P) + gJ * S2) * inv_wsum;
 #pragma unroll
@@ -1290,8 +1302,14 @@ FC_HD void sos_backward_elem_t(float x, const float* raw, int n_runtime, float g
   const float dy_esp_ds = -sp + sn;
   const float dj_esp_ds = -dsp - dsn;
   const float J = fmaxf(jac + j_esp, 1e-37f);  // total derivative
-  const float gJ = gl * fc_rcp(J);
-  gx = gy * (jac + j_esp) + gJ * (djac_dx + dj_esp_dx);
+  float gJ = gl * fc_rcp(J);
+  if constexpr (kInverse) {
+    gx = (gy - gJ * (djac_dx + dj_esp_dx)) * fc_rcp(J);
+    gy = -gx;
+    gJ = -gJ;
+  } else {
+    gx = gy * (jac + j_esp) + gJ * (djac_dx + dj_esp_dx);
+  }
   graw[3 * n] = (gy * dy_esp_ds + gJ * dj_esp_ds) * ds_der;
 
   // pass 2: per-sigmoid parameter gradients

@@ -42,6 +42,21 @@ struct SosOpT {
 
 using SosOp = SosOpT<0>;
 
+// adjoint of the numerical inverse: x is the inverse's output (sos_backward_elem_t<NC, true>)
+struct SosInverseAdjointOp {
+  static constexpr int kTileBwdWarps = 8, kTileBwdMaxWarps = 16;
+  int n;
+  __device__ __forceinline__ int P() const { return 3 * n + 1; }
+  __device__ __forceinline__ void backward(float x, const float* p, float gy, float gl, float& gx, float* gp) const {
+    // gp may alias p: the same read-before-write order as SosOpT::backward
+    if (n == 10) {
+      sos_backward_elem_t<10, true>(x, p, n, gy, gl, gx, gp);
+    } else {
+      sos_backward_elem_t<0, true>(x, p, n, gy, gl, gx, gp);
+    }
+  }
+};
+
 // the numerical inverse is its own kernel instantiation: its register-resident constants must not raise the
 // register count of the forward kernel
 struct SosInverseOp {
@@ -140,10 +155,11 @@ extern "C" int fc_sos_apply(const float* x, int64_t x_row_stride, const float* p
   return launch_apply(a, op, smem, (cudaStream_t)stream);
 }
 
-extern "C" int fc_sos_backward(const float* x, int64_t x_row_stride, const float* params, int64_t params_row_stride,
-                               const float* grad_y, int64_t gy_row_stride, const float* grad_logabsdet, float* grad_x,
-                               int64_t gx_row_stride, float* grad_params, int64_t gp_row_stride, int64_t B, int32_t D,
-                               int32_t n_sigmoids, void* stream) {
+template <class Op>
+static int sos_backward_launch(const Op& op, const float* x, int64_t x_row_stride, const float* params,
+                               int64_t params_row_stride, const float* grad_y, int64_t gy_row_stride,
+                               const float* grad_logabsdet, float* grad_x, int64_t gx_row_stride, float* grad_params,
+                               int64_t gp_row_stride, int64_t B, int32_t D, int32_t n_sigmoids, void* stream) {
   fc_cols none = {nullptr, 0};
   int rc = check_layer_args(x, params, grad_x, B, D, none, none);
   if (rc != FC_OK) return rc;
@@ -151,16 +167,34 @@ extern "C" int fc_sos_backward(const float* x, int64_t x_row_stride, const float
   if (!grad_y || !grad_params) return FC_ERR_INVALID_ARGUMENT;
   if (n_sigmoids < 1) return FC_ERR_INVALID_ARGUMENT;
   if (n_sigmoids > FC_SOS_MAX_SIGMOIDS) return FC_ERR_UNSUPPORTED;
-  if (B == 0) return FC_OK;
   LayerBwdArgs a;
   a.x = x; a.params = params; a.gy = grad_y; a.gl = grad_logabsdet; a.gx = grad_x; a.gp = grad_params;
   a.x_stride = x_row_stride; a.p_stride = params_row_stride; a.gy_stride = gy_row_stride;
   a.gx_stride = gx_row_stride; a.gp_stride = gp_row_stride;
   a.B = B; a.D_t = D; a.n_copy = 0; a.tcols = nullptr; a.ccols = nullptr;
-  SosOp op;
-  op.n = n_sigmoids; op.offset = 0.f;
   const size_t smem = plan_tiles(a, 3 * n_sigmoids + 1);
   const int piped = try_launch_pipelined_backward(a, op, 3 * n_sigmoids + 1, (int)x_row_stride, (cudaStream_t)stream);
   if (piped != 0) return piped < 0 ? piped : FC_OK;
   return launch_backward(a, op, smem, (cudaStream_t)stream);
+}
+
+extern "C" int fc_sos_backward(const float* x, int64_t x_row_stride, const float* params, int64_t params_row_stride,
+                               const float* grad_y, int64_t gy_row_stride, const float* grad_logabsdet, float* grad_x,
+                               int64_t gx_row_stride, float* grad_params, int64_t gp_row_stride, int64_t B, int32_t D,
+                               int32_t n_sigmoids, void* stream) {
+  SosOp op;
+  op.n = n_sigmoids; op.offset = 0.f;
+  return sos_backward_launch(op, x, x_row_stride, params, params_row_stride, grad_y, gy_row_stride, grad_logabsdet,
+                             grad_x, gx_row_stride, grad_params, gp_row_stride, B, D, n_sigmoids, stream);
+}
+
+extern "C" int fc_sos_inverse_backward(const float* x, int64_t x_row_stride, const float* params,
+                                       int64_t params_row_stride, const float* grad_y, int64_t gy_row_stride,
+                                       const float* grad_logabsdet, float* grad_x, int64_t gx_row_stride,
+                                       float* grad_params, int64_t gp_row_stride, int64_t B, int32_t D,
+                                       int32_t n_sigmoids, void* stream) {
+  SosInverseAdjointOp op;
+  op.n = n_sigmoids;
+  return sos_backward_launch(op, x, x_row_stride, params, params_row_stride, grad_y, gy_row_stride, grad_logabsdet,
+                             grad_x, gx_row_stride, grad_params, gp_row_stride, B, D, n_sigmoids, stream);
 }

@@ -577,9 +577,7 @@ def _(x, params, n_sigmoids, offset, inverse, bisection_iterations, lim):
     return torch.empty_like(x), x.new_empty((x.shape[0],))
 
 
-@torch.library.custom_op("flowcon_b200::sos_layer_backward", mutates_args=())
-def sos_layer_backward(x: Tensor, params: Tensor, grad_y: Tensor, grad_lad: Optional[Tensor],
-                       n_sigmoids: int) -> Tuple[Tensor, Tensor]:
+def _sos_adjoint(entry, x, params, grad_y, grad_lad, n_sigmoids):
     L = _cabi.lib()
     x, xp, xs = _cabi.rows(x)
     params, pp, ps = _cabi.rows(params)
@@ -591,11 +589,17 @@ def sos_layer_backward(x: Tensor, params: Tensor, grad_y: Tensor, grad_lad: Opti
     if grad_lad is not None:
         grad_lad = grad_lad.contiguous()
         glp = grad_lad.data_ptr()
-    with torch.cuda.device(x.device), _cabi.launch("fc_sos_backward", x.device):
-        rc = L.fc_sos_backward(xp, xs, pp, ps, gyp, gys, glp, gx.data_ptr(), D, gp.data_ptr(), gp.shape[1], B, D,
+    with torch.cuda.device(x.device), _cabi.launch(entry, x.device):
+        rc = getattr(L, entry)(xp, xs, pp, ps, gyp, gys, glp, gx.data_ptr(), D, gp.data_ptr(), gp.shape[1], B, D,
                                n_sigmoids, _cabi.stream_ptr(x.device))
-    _cabi.check(rc, "fc_sos_backward")
+    _cabi.check(rc, entry)
     return gx, gp
+
+
+@torch.library.custom_op("flowcon_b200::sos_layer_backward", mutates_args=())
+def sos_layer_backward(x: Tensor, params: Tensor, grad_y: Tensor, grad_lad: Optional[Tensor],
+                       n_sigmoids: int) -> Tuple[Tensor, Tensor]:
+    return _sos_adjoint("fc_sos_backward", x, params, grad_y, grad_lad, n_sigmoids)
 
 
 @sos_layer_backward.register_fake
@@ -603,20 +607,33 @@ def _(x, params, grad_y, grad_lad, n_sigmoids):
     return torch.empty_like(x), torch.empty_like(params)
 
 
+@torch.library.custom_op("flowcon_b200::sos_layer_inverse_backward", mutates_args=())
+def sos_layer_inverse_backward(x_out: Tensor, params: Tensor, grad_out: Tensor, grad_lad: Optional[Tensor],
+                               n_sigmoids: int) -> Tuple[Tensor, Tensor]:
+    """Adjoint of `sos_layer(..., inverse=True)`: x_out is the inverse's output.  Returns the gradients of the inverse's
+    input z and of the raw parameters (the offset, iteration count and bracket do not enter)."""
+    return _sos_adjoint("fc_sos_inverse_backward", x_out, params, grad_out, grad_lad, n_sigmoids)
+
+
+@sos_layer_inverse_backward.register_fake
+def _(x_out, params, grad_out, grad_lad, n_sigmoids):
+    return torch.empty_like(x_out), torch.empty_like(params)
+
+
 def _sos_setup(ctx, inputs, output):
     x, params, n_sigmoids, offset, inverse = inputs[:5]
-    ctx.save_for_backward(x, params)
+    # the inverse's adjoint is evaluated at its own output: saving it spares a second numerical solve
+    ctx.save_for_backward(output[0] if inverse else x, params)
     ctx.n_sigmoids = n_sigmoids
     ctx.inverse = inverse
 
 
 def _sos_backward(ctx, gy, gl):
-    if ctx.inverse:
-        raise NotImplementedError("gradients through the numerical sum-of-sigmoids inverse are not implemented")
     x, params = ctx.saved_tensors
     if gy is None:
         gy = torch.zeros_like(x)
-    gx, gp = sos_layer_backward(x, params, gy, gl, ctx.n_sigmoids)
+    adjoint = sos_layer_inverse_backward if ctx.inverse else sos_layer_backward
+    gx, gp = adjoint(x, params, gy, gl, ctx.n_sigmoids)
     return gx, gp, None, None, None, None, None
 
 

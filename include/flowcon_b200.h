@@ -203,6 +203,17 @@ int fc_sos_backward(const float* x, int64_t x_row_stride, const float* params, i
                     float* grad_x, int64_t gx_row_stride, float* grad_params, int64_t gp_row_stride,
                     int64_t B, int32_t D, int32_t n_sigmoids, void* stream);
 
+/*
+ * Adjoint of the numerical inverse (fc_sos_apply with inverse = 1).  x is the inverse's OUTPUT; grad_y and
+ * grad_logabsdet (may be NULL) are the gradients of that output and of the inverse's logabsdet.  Writes the gradient of
+ * the inverse's input (grad_x) and of the raw parameters.  Arguments and validation as fc_sos_backward; the offset,
+ * the iteration count and the bracket do not enter.
+ */
+int fc_sos_inverse_backward(const float* x, int64_t x_row_stride, const float* params, int64_t params_row_stride,
+                            const float* grad_y, int64_t gy_row_stride, const float* grad_logabsdet,
+                            float* grad_x, int64_t gx_row_stride, float* grad_params, int64_t gp_row_stride,
+                            int64_t B, int32_t D, int32_t n_sigmoids, void* stream);
+
 /* Base density tail: out[r] = -0.5 * sum_j z[r,j]^2 - 0.5*D*ln(2*pi) + logabsdet[r]
  * (StandardNormal._log_prob distributions/normal.py:23-33 + flows/base.py:48). logabsdet may be NULL. */
 int fc_stdnormal_log_prob(const float* z, int64_t z_row_stride, const float* logabsdet, float* out,
