@@ -75,11 +75,21 @@ class Conditioner(ctypes.Structure):
                 ("k_in", ctypes.c_int32), ("hidden_k", ctypes.c_int32), ("layers", ConditionerLayer * COND_MAX_LAYERS)]
 
 
+MADE_MAX_TERM_ARRAYS = 8
+
+
+class MadeTermArray(ctypes.Structure):
+    """struct fc_made_term_array"""
+    _fields_ = [("array", ctypes.c_int32), ("column", ctypes.c_int32), ("b_off", ctypes.c_int32), ("relu", ctypes.c_int32)]
+
+
 class MadeProgramStruct(ctypes.Structure):
     """struct fc_made_program"""
     _fields_ = [("phases", ctypes.c_void_p), ("weights", ctypes.c_void_p), ("bias", ctypes.c_void_p),
                 ("n_phases", ctypes.c_int32), ("features", ctypes.c_int32), ("params_per_feature", ctypes.c_int32),
-                ("n_arrays", ctypes.c_int32), ("hidden", ctypes.c_int32), ("n_bias", ctypes.c_int32)]
+                ("n_arrays", ctypes.c_int32), ("hidden", ctypes.c_int32), ("n_bias", ctypes.c_int32),
+                ("terms", ctypes.c_void_p), ("term_width", ctypes.c_int32), ("n_term_arrays", ctypes.c_int32),
+                ("term_arrays", MadeTermArray * MADE_MAX_TERM_ARRAYS)]
 
 
 class LibraryMissing(RuntimeError):

@@ -61,8 +61,6 @@ class ContextPlan:
 def pack_context(net):
     """ContextPlan of a conditional ResidualNet (a gate per block, resnet.py:45-52) or residual MADE (initial layer
     made.py:274-279, the first layer of every block made.py:170-181); None for a net without context layers."""
-    from . import linear as fl
-
     blocks = list(net.blocks)
     if hasattr(net, "context_layer"):  # MADE
         src = [(0, _cabi.COND_TERM_ADD_RELU, net.context_layer)]
@@ -71,24 +69,39 @@ def pack_context(net):
         src = [(2 + 2 * i, _cabi.COND_TERM_GATE, b.context_layer) for i, b in enumerate(blocks)]
     else:
         return None
-    hp = padded_hidden(net.initial_layer.weight.shape[0])
+    return stack_context(src, padded_hidden(net.initial_layer.weight.shape[0]))
+
+
+def stack_context(src, stride, order=None):
+    """ContextPlan of the context layers `src` [(consumer, FC_COND_TERM_* mode, nn.Linear)]: layer i's outputs at
+    columns i * stride + j, taken in the order `order` (an index into the outputs) when given; the width is padded to a
+    multiple of 16 and the padding columns have zero weights and bias.  The incremental MADE inverse (made_inverse.py)
+    stacks its context layers here too, in the degree order of its hidden units."""
+    from . import linear as fl
+
     ref = src[0][2].weight
     C = ref.shape[1]
-    weight = torch.zeros((hp * len(src), C), dtype=torch.float32, device=ref.device)
-    bias = torch.zeros((hp * len(src),), dtype=torch.float32, device=ref.device)
+    width = _ceil_to(stride * len(src), 16)
+    weight = torch.zeros((width, C), dtype=torch.float32, device=ref.device)
+    bias = torch.zeros((width,), dtype=torch.float32, device=ref.device)
     layers = []
     for i, (layer, mode, lin) in enumerate(src):
-        n = lin.weight.shape[0]
-        weight[i * hp:i * hp + n] = lin.weight.detach()
-        if lin.bias is not None:
-            bias[i * hp:i * hp + n] = lin.bias.detach()
-        layers.append((layer, mode, i * hp))
+        w = lin.weight.detach()
+        b = lin.bias.detach() if lin.bias is not None else None
+        if order is not None:
+            w = w[order]
+            b = b[order] if b is not None else None
+        n = w.shape[0]
+        weight[i * stride:i * stride + n] = w
+        if b is not None:
+            bias[i * stride:i * stride + n] = b
+        layers.append((layer, mode, i * stride))
     linear = None
-    if C >= MIN_K_TC:
+    if C >= MIN_K_TC and ref.is_cuda:  # (a plan of CPU modules only serves host-side tests of the stacking)
         c4 = _ceil_to(C, 4)
         cm = None if c4 == C else torch.arange(C, dtype=torch.int32, device=ref.device)
         linear = fl.pack(weight, bias, col_map=cm, k_in=c4)
-    return ContextPlan(weight, bias, layers, weight.shape[0], linear)
+    return ContextPlan(weight, bias, layers, width, linear)
 
 
 def context_terms(packed, ctx):

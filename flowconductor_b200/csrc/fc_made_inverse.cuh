@@ -33,6 +33,9 @@
 //     task stores its units.  One CTA barrier per phase.
 //   * warp 0 then inverts the feature (same element arithmetic as the layer kernels: fc_math.cuh) and the next pass
 //     starts.  log|det J| is the sum of the per-feature terms (what the reference's last pass returns).
+//   * a conditional MADE (kCtx): the context enters as precomputed terms Wc ctx + bc, which do not depend on x; the
+//     hidden arrays that consume them are prefilled with bias + act(term) when a row tile starts, and the program's tasks
+//     accumulate onto that value.  Nothing else changes.
 //
 // This header holds the kernel and its launch plumbing; every bijection family instantiates it in its own .cu with an Op
 //   struct Op { __device__ void eval(float z, const float* pc, float& x, float& lad, unsigned& status) const; }
@@ -56,7 +59,7 @@ constexpr int kMSlotFloats = kMSlotBytes / 4;
 constexpr int kMPhaseInt4 = (4 + 12 * kMW) / 4;  // one fc_made_phase = header + 8 tasks = 25 x int4
 constexpr int kMRecFloats = FC_MADE_RECORD_FLOATS;  // the phase record at the head of the phase's weights (padded to 512 B)
 
-struct MadeArgs {
+struct MadeKernelArgs {
   const int4* phases;  // fc_made_phase[n_phases]
   int n_phases;
   const float* weights;
@@ -72,6 +75,16 @@ struct MadeArgs {
   long long M;
   int num_tiles;
   int32_t* status;
+};
+// Conditional MADE (kCtx): this call's context terms [M, term_width] in T128 and the hidden arrays that start from them.
+// A kernel parameter of its own, so that the context-free kernels keep their parameter layout and code.
+struct MadeTerms {
+  const float* terms;
+  int term_width, n_term_arrays;
+  int4 arrays[FC_MADE_MAX_TERM_ARRAYS];  // (array, first column in `terms`, bias offset, relu)
+};
+struct MadeArgs : MadeKernelArgs {
+  MadeTerms ctx;
 };
 
 // Experiments only (-DFC_MADE_PROFILE=1: FC_LINEAR_PROFILE_BUILD=1 python -m flowconductor_b200.build --force): cycles warps 0
@@ -157,8 +170,8 @@ struct MadeSmem {
   }
 };
 
-template <class Op>
-__global__ void __launch_bounds__(kMThreads, 1) made_inverse_kernel(const MadeArgs a, const Op op) {
+template <class Op, bool kCtx>
+__global__ void __launch_bounds__(kMThreads, 1) made_inverse_kernel(const MadeKernelArgs a, const Op op, const MadeTerms ct) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const uint32_t raw_s = tc::s32(smem_raw);
   const uint32_t base = (raw_s + 127u) & ~127u;
@@ -236,6 +249,28 @@ __global__ void __launch_bounds__(kMThreads, 1) made_inverse_kernel(const MadeAr
     for (int i = tid; i < kMR * D; i += kMW * 32) {
       const int r = i / D, f = i - r * D;
       X[f * kMR + r] = (row0 + r < a.M) ? __ldg(a.z + (row0 + r) * a.ldz + f) : 0.f;
+    }
+    if constexpr (kCtx) {
+      // The context terms do not depend on x: every unit of a context array starts the tile at bias + act(term) (MADE
+      // initial layer: act = ReLU, made.py:138-140; first layer of a block: identity, made.py:100-102), and the tasks that
+      // write those units accumulate onto it (the host clears FC_MADE_INIT_BIAS on them).  Lane = row: one float4 of the
+      // T128 matrix per (row, 4 units), 512 contiguous bytes per warp, conflict-free [unit][32 rows] stores.  Rows past M
+      // get the bias alone (the T128 rows there were never written).
+      const int groups = (a.hidden + 3) >> 2;
+      const float* tile_terms = ct.terms + (row0 >> 7) * 128ll * ct.term_width + (row0 & 127) * 4;
+      for (int i = tid; i < ct.n_term_arrays * groups * kMR; i += kMW * 32) {
+        const int r = i & (kMR - 1), q = i >> 5, g = q % groups;
+        const int4 ta = ct.arrays[q / groups];
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (row0 + r < a.M) v = __ldg(reinterpret_cast<const float4*>(tile_terms + (size_t)((ta.y >> 2) + g) * 512 + r * 4));
+        if (ta.w) v = make_float4(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f), fmaxf(v.z, 0.f), fmaxf(v.w, 0.f));
+        const float t[4] = {v.x, v.y, v.z, v.w};
+        const int j0 = 4 * g, n = a.hidden - j0 < 4 ? a.hidden - j0 : 4;
+        float* h = H + (size_t)(ta.x - 1) * arr_floats + (size_t)j0 * kMR + r;
+#pragma unroll
+        for (int e = 0; e < 4; ++e)
+          if (e < n) h[e * kMR] = BS[ta.z + j0 + e] + t[e];
+      }
     }
     float lad_acc = 0.f;
     tc::named_barrier_sync(1, kMW * 32);
@@ -401,6 +436,24 @@ inline int made_check(const fc_made_program* prog, const float* z, int64_t ldz, 
   a.lad = lad;
   a.M = B;
   a.num_tiles = (int)((B + kMR - 1) / kMR);
+  const int nt = prog->n_term_arrays;
+  if (nt < 0 || nt > FC_MADE_MAX_TERM_ARRAYS) return FC_ERR_INVALID_ARGUMENT;
+  if (nt > 0) {
+    if (!prog->terms || (reinterpret_cast<uintptr_t>(prog->terms) & 15) || prog->term_width <= 0 || prog->term_width % 16)
+      return FC_ERR_INVALID_ARGUMENT;
+    for (int t = 0; t < nt; ++t) {
+      const fc_made_term_array& ta = prog->term_arrays[t];
+      if (ta.array < 1 || ta.array > prog->n_arrays) return FC_ERR_INVALID_ARGUMENT;
+      for (int u = 0; u < t; ++u)
+        if (prog->term_arrays[u].array == ta.array) return FC_ERR_INVALID_ARGUMENT;
+      if (ta.column < 0 || ta.column % 4 || (int64_t)ta.column + prog->hidden > prog->term_width) return FC_ERR_INVALID_ARGUMENT;
+      if (ta.b_off < 0 || (int64_t)ta.b_off + prog->hidden > prog->n_bias) return FC_ERR_INVALID_ARGUMENT;
+      a.ctx.arrays[t] = make_int4(ta.array, ta.column, ta.b_off, ta.relu != 0);
+    }
+    a.ctx.terms = prog->terms;
+    a.ctx.term_width = prog->term_width;
+  }
+  a.ctx.n_term_arrays = nt;
   a.stages = made_stages(a.D, a.P, a.n_arrays, a.hidden, a.n_bias);
   if (a.stages < 2) return FC_ERR_UNSUPPORTED;
   return FC_OK;
@@ -408,12 +461,12 @@ inline int made_check(const fc_made_program* prog, const float* z, int64_t ldz, 
 
 template <class Op>
 inline int launch_made(const MadeArgs& a, const Op& op, cudaStream_t stream) {
-  auto kern = made_inverse_kernel<Op>;
+  auto kern = a.ctx.n_term_arrays > 0 ? made_inverse_kernel<Op, true> : made_inverse_kernel<Op, false>;
   const size_t smem = MadeSmem::total(a.stages, a.D, a.P, a.n_arrays, a.hidden, a.n_bias);
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return FC_ERR_CUDA;
   const int sms = device_info().sm_count;
   const int grid = a.num_tiles < sms ? a.num_tiles : sms;
-  kern<<<grid, kMThreads, smem, stream>>>(a, op);
+  kern<<<grid, kMThreads, smem, stream>>>(a, op, a.ctx);
   FC_CHECK_LAUNCH();
   return FC_OK;
 }

@@ -7,6 +7,12 @@ of the layer below; pass f then computes only the units that become valid with f
 feature f, after which the kernel inverts that feature.  The schedule is derived from the MASKS, not from the degree
 formula: any mask pattern with the prefix property compiles, anything else returns None (the D-pass inverse runs).
 
+A conditional MADE (`context_features`) compiles to the same program.  Its context layers (initial layer made.py:138-140,
+first layer of every block made.py:100-102) do not depend on x: they are stacked into one `conditioner.ContextPlan`, rows
+in the program's degree order, and each call evaluates them for the whole batch in one launch
+(`conditioner.context_terms`).  The kernel starts the hidden arrays that consume them from bias + act(term), so the tasks
+that write those arrays accumulate instead of initialising from the bias.
+
 No fallback inside: `apply_*` needs CUDA fp32 tensors and the library.
 """
 import ctypes
@@ -14,7 +20,7 @@ import ctypes
 import numpy as np
 import torch
 
-from . import _cabi
+from . import _cabi, conditioner
 
 MAX_NJ = 24      # FC_MADE_MAX_NJ
 TASKS = 8        # FC_MADE_TASKS
@@ -33,17 +39,24 @@ TASK_FIELDS = ("in_array", "out_array", "k0", "kn", "j0", "nj", "c0", "flags", "
 class MadeProgram:
     """Compiled program + its device buffers (`phases`, `weights`, `bias` keep the memory alive)."""
 
-    def __init__(self, phases_np, weights, bias, features, params_per_feature, n_arrays, hidden, device):
+    def __init__(self, phases_np, weights, bias, features, params_per_feature, n_arrays, hidden, device, context=None,
+                 term_arrays=()):
         self.phases_np = phases_np  # [n_phases, 100] int32 (host copy: tests, debugging)
         self.phases = torch.from_numpy(phases_np.copy()).to(device)
         self.weights, self.bias = weights, bias
         self.features, self.params_per_feature, self.n_arrays, self.hidden = features, params_per_feature, n_arrays, hidden
+        # conditional MADE: the stacked context layers, and per consuming hidden array (array, column, b_off, relu)
+        self.context, self.term_arrays = context, list(term_arrays)
         self.struct = None
         if weights.is_cuda:
             st = _cabi.MadeProgramStruct()
             st.phases, st.weights, st.bias = self.phases.data_ptr(), weights.data_ptr(), bias.data_ptr()
             st.n_phases, st.features, st.params_per_feature = phases_np.shape[0], features, params_per_feature
             st.n_arrays, st.hidden, st.n_bias = n_arrays, hidden, bias.numel()
+            if context is not None:
+                st.term_width, st.n_term_arrays = context.width, len(self.term_arrays)
+                for i, t in enumerate(self.term_arrays):
+                    st.term_arrays[i].array, st.term_arrays[i].column, st.term_arrays[i].b_off, st.term_arrays[i].relu = t
             self.struct = st
 
     @property
@@ -80,15 +93,17 @@ def _prefix_counts(mask):
 
 
 def supported_made(net):
-    """Structure the compiler handles: residual blocks, ReLU, no context / batch norm / active dropout."""
+    """Structure the compiler handles: residual blocks, ReLU, no batch norm / active dropout; context layers on the initial
+    layer and every block, or none."""
     from .nn import tensorcore
 
-    if not getattr(net, "use_residual_blocks", False) or hasattr(net, "context_layer"):
+    if not getattr(net, "use_residual_blocks", False):
         return False
     if not tensorcore._is_relu(net.activation):
         return False
+    ctx = hasattr(net, "context_layer")
     for blk in net.blocks:
-        if getattr(blk, "use_batch_norm", False) or not tensorcore._is_relu(blk.activation) or hasattr(blk, "context_layer"):
+        if getattr(blk, "use_batch_norm", False) or not tensorcore._is_relu(blk.activation) or hasattr(blk, "context_layer") != ctx:
             return False
         if blk.dropout.p > 0 and blk.training:
             return False
@@ -125,6 +140,11 @@ def compile_made(net, params_per_feature):
     n_arrays = 1 + 2 * nb
     if smem_bytes(D, P, n_arrays, H) > SMEM_LIMIT:
         return None
+    conditional = hasattr(net, "context_layer")
+    if conditional and 1 + nb > _cabi.MADE_MAX_TERM_ARRAYS:
+        return None
+    # hidden arrays that start from bias + act(context term): the initial layer's (ReLU) and each block's first layer's
+    ctx_arrays = {1} | {2 * b + 2 for b in range(nb)} if conditional else set()
     with torch.no_grad():
         deg = init.degrees.detach().cpu()
         for blk in net.blocks:
@@ -172,7 +192,7 @@ def compile_made(net, params_per_feature):
             c0 = 0
             for li, j_lo, nj, k0, kn, init_bias, final, j_base in tasks:
                 _, in_a, out_a, relu_in, res_a = layers[li]
-                flags = (RELU_IN if relu_in else 0) | (INIT_BIAS if init_bias else 0)
+                flags = (RELU_IN if relu_in else 0) | (INIT_BIAS if init_bias and out_a not in ctx_arrays else 0)
                 rec += [in_a, out_a, k0, kn, j_lo - j_base, nj, c0, flags, res_a if final else 0, bias_base[li] + j_lo, 0, 0]
                 if kn > 0:
                     mat[:kn, c0:c0 + nj] = sorted_w[li][j_lo:j_lo + nj, k0:k0 + kn].t()
@@ -258,7 +278,16 @@ def compile_made(net, params_per_feature):
         phases_np = np.asarray(phases, dtype=np.int32).reshape(-1, PHASE_INTS)
         weights = torch.cat(blocks) if blocks else torch.zeros((4,), dtype=torch.float32, device=dev)
         bias = torch.cat(bias_parts).contiguous()
-    return MadeProgram(phases_np, weights.contiguous(), bias, D, P, n_arrays, H, dev)
+        context, term_arrays = None, []
+        if conditional:
+            # columns i * ceil4(H) + j: sorted unit j of the i-th consuming array (the kernel reads whole float4 groups)
+            src = [(1, _cabi.COND_TERM_ADD_RELU, net.context_layer)]
+            src += [(2 * b + 2, _cabi.COND_TERM_ADD, blk.context_layer) for b, blk in enumerate(net.blocks)]
+            context = conditioner.stack_context(src, (H + 3) // 4 * 4, order=perm)
+            b_off = {1: bias_base[0]}
+            b_off.update({2 * b + 2: bias_base[1 + 2 * b] for b in range(nb)})
+            term_arrays = [(arr, col, b_off[arr], int(mode == _cabi.COND_TERM_ADD_RELU)) for arr, mode, col in context.layers]
+    return MadeProgram(phases_np, weights.contiguous(), bias, D, P, n_arrays, H, dev, context, term_arrays)
 
 
 def _io(prog, z):
@@ -271,13 +300,37 @@ def _io(prog, z):
     return z, zp, ldz, x, lad
 
 
-def _apply(entry, prog, z, *tail):
+def _bind_terms(prog, context, B):
+    """The context terms of this call (one launch, conditioner.context_terms), bound into the program struct; None for a
+    MADE without context layers.  The binding is valid for one launch only: the caller keeps the result alive until the
+    launch is enqueued and then clears `prog.struct.terms` (the buffer goes back to the caching allocator)."""
+    if prog.context is None:
+        if context is not None:
+            raise ValueError("a context was given for a MADE without context layers")
+        prog.struct.terms = None
+        return None
+    if context is None:
+        raise ValueError("a MADE with context layers needs its context")
+    if context.dim() != 2 or context.shape[0] != B:
+        raise ValueError("context has shape {}, expected [{}, {}]".format(tuple(context.shape), B, prog.context.features))
+    terms = conditioner.context_terms(prog.context, context)
+    if terms.width != prog.context.width:  # the kernel addresses the T128 tiles with the plan's width
+        raise ValueError("context terms are {} wide, the program expects {}".format(terms.width, prog.context.width))
+    prog.struct.terms = terms.buf.data_ptr()
+    return terms
+
+
+def _apply(entry, prog, z, context, *tail):
     """Shared launch plumbing of the fc_made_inverse_* entry points: (x, logabsdet)."""
     L = _cabi.lib()
     z, zp, ldz, x, lad = _io(prog, z)
-    with torch.cuda.device(z.device), _cabi.launch(entry, z.device):
-        rc = getattr(L, entry)(ctypes.byref(prog.struct), zp, ldz, x.data_ptr(), x.stride(0), lad.data_ptr(), 0,
-                               z.shape[0], *tail, _cabi.stream_ptr(z.device))
+    terms = _bind_terms(prog, context, z.shape[0])  # noqa: F841 (alive until the launch is enqueued)
+    try:
+        with torch.cuda.device(z.device), _cabi.launch(entry, z.device):
+            rc = getattr(L, entry)(ctypes.byref(prog.struct), zp, ldz, x.data_ptr(), x.stride(0), lad.data_ptr(), 0,
+                                   z.shape[0], *tail, _cabi.stream_ptr(z.device))
+    finally:
+        prog.struct.terms = None  # a later direct use of the struct must bind its own terms
     _cabi.check(rc, entry)
     return x, lad
 
@@ -286,32 +339,33 @@ def _sptr(status):
     return status.data_ptr() if status is not None else None
 
 
-def apply_rqs(prog, z, cfg, status=None):
-    """Inverse of a MAF layer with rational-quadratic splines: (x, logabsdet) = layer.inverse(z)."""
-    return _apply("fc_made_inverse_rqs", prog, z, ctypes.byref(cfg), _sptr(status))
+def apply_rqs(prog, z, cfg, status=None, context=None):
+    """Inverse of a MAF layer with rational-quadratic splines: (x, logabsdet) = layer.inverse(z, context).  `context`:
+    the [B, C] context of a conditional MADE (required exactly when the program has context layers); likewise below."""
+    return _apply("fc_made_inverse_rqs", prog, z, context, ctypes.byref(cfg), _sptr(status))
 
 
-def apply_affine(prog, z, activation):
+def apply_affine(prog, z, activation, context=None):
     """Inverse of a MaskedAffineAutoregressiveTransform layer."""
-    return _apply("fc_made_inverse_affine", prog, z, int(activation))
+    return _apply("fc_made_inverse_affine", prog, z, context, int(activation))
 
 
-def apply_sos(prog, z, n_sigmoids, offset, iterations, lim):
+def apply_sos(prog, z, n_sigmoids, offset, iterations, lim, context=None):
     """Inverse of a MaskedSumOfSigmoidsTransform layer (numerical inverse per feature, as fc_sos_apply)."""
-    return _apply("fc_made_inverse_sos", prog, z, int(n_sigmoids), float(offset), int(iterations), float(lim))
+    return _apply("fc_made_inverse_sos", prog, z, context, int(n_sigmoids), float(offset), int(iterations), float(lim))
 
 
-def apply_linspline(prog, z, num_bins, tails, lo, hi, status=None):
-    return _apply("fc_made_inverse_linspline", prog, z, int(num_bins), int(tails), float(lo), float(hi), float(lo), float(hi),
-                  _sptr(status))
+def apply_linspline(prog, z, num_bins, tails, lo, hi, status=None, context=None):
+    return _apply("fc_made_inverse_linspline", prog, z, context, int(num_bins), int(tails), float(lo), float(hi), float(lo),
+                  float(hi), _sptr(status))
 
 
-def apply_quadspline(prog, z, cfg, status=None):
-    return _apply("fc_made_inverse_quadspline", prog, z, ctypes.byref(cfg), _sptr(status))
+def apply_quadspline(prog, z, cfg, status=None, context=None):
+    return _apply("fc_made_inverse_quadspline", prog, z, context, ctypes.byref(cfg), _sptr(status))
 
 
-def apply_cubicspline(prog, z, cfg, status=None):
-    return _apply("fc_made_inverse_cubicspline", prog, z, ctypes.byref(cfg), _sptr(status))
+def apply_cubicspline(prog, z, cfg, status=None, context=None):
+    return _apply("fc_made_inverse_cubicspline", prog, z, context, ctypes.byref(cfg), _sptr(status))
 
 
 PROFILE_FIELDS = ("phase record", "wait weights", "multiply", "store units", "phase barrier", "invert feature", "total",
@@ -334,8 +388,9 @@ ENABLED = True  # False: every autoregressive inverse takes the D-pass path
 
 
 def program_for(net, params_per_feature):
-    """Compiled program of `net`, cached on the module with the same key rules as the packed tensor-core weights
-    (nn/tensorcore.py: data pointer + in-place version of every parameter).  None if the net does not compile."""
+    """Compiled program of `net` (with the stacked context layers of a conditional MADE), cached on the module with the
+    same key rules as the packed tensor-core weights (nn/tensorcore.py: data pointer + in-place version of every parameter,
+    the context layers' included).  None if the net does not compile."""
     from .nn import tensorcore
 
     key = (tensorcore._param_key(net), params_per_feature, bool(net.training))
@@ -349,12 +404,19 @@ def program_for(net, params_per_feature):
 
 
 def usable(net, inputs, context):
-    """Should this inverse call take the incremental kernel?"""
+    """Should this inverse call take the incremental kernel?  A call with a context does when the net has context layers
+    and the fused conditioner does not cover the call (there the D-pass inverse runs one fused launch per pass:
+    AutoregressiveTransform.inverse)."""
     from .nn import tensorcore
     from .transforms import made as made_module
 
-    if not ENABLED or context is not None or not isinstance(net, made_module.MADE):
+    if not ENABLED or not isinstance(net, made_module.MADE) or hasattr(net, "context_layer") != (context is not None):
         return False
-    if tensorcore.wants_grad(net, inputs):
+    if tensorcore.wants_grad(net, inputs, context):
         return False
-    return inputs.is_cuda and inputs.dtype == torch.float32 and inputs.dim() == 2 and inputs.shape[0] > 0
+    if not (inputs.is_cuda and inputs.dtype == torch.float32 and inputs.dim() == 2 and inputs.shape[0] > 0):
+        return False
+    if context is None:
+        return True
+    return (context.is_cuda and context.dtype == torch.float32 and context.dim() == 2
+            and context.shape[0] == inputs.shape[0] and not tensorcore.usable(net, inputs, context, inputs))

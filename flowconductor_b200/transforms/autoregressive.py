@@ -32,7 +32,7 @@ class AutoregressiveTransform(Transform):
 
     def inverse(self, inputs, context=None):
         if made_inverse.usable(self.autoregressive_net, inputs, context):
-            result = self._incremental_inverse(inputs)
+            result = self._incremental_inverse(inputs, context)
             if result is not None:
                 return result
         outputs = torch.zeros_like(inputs)
@@ -56,8 +56,9 @@ class AutoregressiveTransform(Transform):
             return self._elementwise_inverse(inputs, params)
         return self._elementwise_forward(inputs, params)
 
-    def _incremental_inverse(self, inputs):
-        """(outputs, logabsdet) from the incremental-MADE kernel, or None if this layer / network is not covered."""
+    def _incremental_inverse(self, inputs, context=None):
+        """(outputs, logabsdet) from the incremental-MADE kernel, or None if this layer / network is not covered.
+        `context`: the context of a conditional MADE (made_inverse.usable has checked it)."""
         return None
 
     def _output_dim_multiplier(self):
@@ -99,11 +100,11 @@ class MaskedAffineAutoregressiveTransform(AutoregressiveTransform):
         return ops.affine_layer(inputs, autoregressive_params, None, None, _cabi.AFFINE_INTERLEAVED,
                                 _cabi.SCALE_SOFTPLUS_EPS, True)
 
-    def _incremental_inverse(self, inputs):
+    def _incremental_inverse(self, inputs, context=None):
         prog = made_inverse.program_for(self.autoregressive_net, 2)
         if prog is None:
             return None
-        return made_inverse.apply_affine(prog, inputs, _cabi.SCALE_SOFTPLUS_EPS)
+        return made_inverse.apply_affine(prog, inputs, _cabi.SCALE_SOFTPLUS_EPS, context)
 
     def _tensorcore_layer(self, conditioner_inputs, inputs, inverse, context=None, terms=None):
         net = self.autoregressive_net
@@ -135,11 +136,11 @@ class MaskedSumOfSigmoidsTransform(AutoregressiveTransform):
     def _elementwise_inverse(self, inputs, autoregressive_params):
         return ops.sos_layer(inputs, autoregressive_params, self.n_sigmoids, -0.5, True, 50, 120.0)
 
-    def _incremental_inverse(self, inputs):
+    def _incremental_inverse(self, inputs, context=None):
         prog = made_inverse.program_for(self.autoregressive_net, self._output_dim_multiplier())
         if prog is None:
             return None
-        return made_inverse.apply_sos(prog, inputs, self.n_sigmoids, -0.5, 50, 120.0)
+        return made_inverse.apply_sos(prog, inputs, self.n_sigmoids, -0.5, 50, 120.0, context)
 
     def _tensorcore_layer(self, conditioner_inputs, inputs, inverse, context=None, terms=None):
         net = self.autoregressive_net
@@ -183,7 +184,7 @@ class MaskedPiecewiseRationalQuadraticAutoregressiveTransform(AutoregressiveTran
     def _elementwise_inverse(self, inputs, autoregressive_params):
         return self._elementwise(inputs, autoregressive_params, inverse=True)
 
-    def _incremental_inverse(self, inputs):
+    def _incremental_inverse(self, inputs, context=None):
         prog = made_inverse.program_for(self.autoregressive_net, self._spline.params_per_feature())
         if prog is None:
             return None
@@ -191,7 +192,7 @@ class MaskedPiecewiseRationalQuadraticAutoregressiveTransform(AutoregressiveTran
         cfg, tails = self._spline.config(True, hidden)
         status = torch.zeros((1,), dtype=torch.int32, device=inputs.device) if tails == _cabi.TAILS_NONE or splines.STRICT \
             else None
-        outputs, logabsdet = made_inverse.apply_rqs(prog, inputs, cfg, status)
+        outputs, logabsdet = made_inverse.apply_rqs(prog, inputs, cfg, status, context)
         if status is not None:
             splines.check_status(status, tails)
         return outputs, logabsdet
@@ -236,13 +237,13 @@ class MaskedPiecewiseLinearAutoregressiveTransform(AutoregressiveTransform):
     def _elementwise_inverse(self, inputs, autoregressive_params):
         return self._spline.apply(inputs, autoregressive_params, None, None, True)
 
-    def _incremental_inverse(self, inputs):
+    def _incremental_inverse(self, inputs, context=None):
         prog = made_inverse.program_for(self.autoregressive_net, self._output_dim_multiplier())
         if prog is None:
             return None
         tails, lo, hi = self._spline.domain()
         status = _status_for(inputs, tails)
-        out = made_inverse.apply_linspline(prog, inputs, self.num_bins, tails, lo, hi, status)
+        out = made_inverse.apply_linspline(prog, inputs, self.num_bins, tails, lo, hi, status, context)
         if status is not None:
             splines.check_status(status, tails)
         return out
@@ -278,13 +279,13 @@ class MaskedPiecewiseQuadraticAutoregressiveTransform(AutoregressiveTransform):
     def _elementwise_inverse(self, inputs, autoregressive_params):
         return self._spline.apply(inputs, autoregressive_params, None, None, True, None)
 
-    def _incremental_inverse(self, inputs):
+    def _incremental_inverse(self, inputs, context=None):
         prog = made_inverse.program_for(self.autoregressive_net, self._output_dim_multiplier())
         if prog is None:
             return None
         cfg, tails = self._spline.config(True, None)
         status = _status_for(inputs, tails)
-        out = made_inverse.apply_quadspline(prog, inputs, cfg, status)
+        out = made_inverse.apply_quadspline(prog, inputs, cfg, status, context)
         if status is not None:
             splines.check_status(status, tails)
         return out
@@ -312,13 +313,13 @@ class MaskedPiecewiseCubicAutoregressiveTransform(AutoregressiveTransform):
     def _elementwise_inverse(self, inputs, autoregressive_params):
         return self._spline.apply(inputs, autoregressive_params, None, None, True, None)
 
-    def _incremental_inverse(self, inputs):
+    def _incremental_inverse(self, inputs, context=None):
         prog = made_inverse.program_for(self.autoregressive_net, self._output_dim_multiplier())
         if prog is None:
             return None
         cfg, tails = self._spline.config(True, None)
         status = _status_for(inputs, tails)
-        out = made_inverse.apply_cubicspline(prog, inputs, cfg, status)
+        out = made_inverse.apply_cubicspline(prog, inputs, cfg, status, context)
         if status is not None:
             splines.check_status(status, tails)
         return out

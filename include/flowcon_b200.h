@@ -441,8 +441,8 @@ int fc_conditioner_profile(unsigned long long* out32);
  * The INVERSE of a masked autoregressive layer in one kernel, MADE evaluated incrementally (csrc/fc_made_inverse.cu;
  * SURVEY 8(f) n2).  Replaces AutoregressiveTransform.inverse (flowcon/transforms/autoregressive/autoregressive.py:44-53:
  * D passes of the whole conditioner, flowcon/transforms/made.py:274-283, each followed by the element-wise inverse) for
- * a residual MADE without context: pass f computes only the hidden units that become valid with feature f - 1 and the
- * parameters of feature f.  The caller (flowconductor_b200/made_inverse.py) compiles the network into a program of
+ * a residual MADE, with or without context layers: pass f computes only the hidden units that become valid with feature
+ * f - 1 and the parameters of feature f.  The caller (flowconductor_b200/made_inverse.py) compiles the network into a program of
  * PHASES; a phase is a [rows x width] fp32 weight matrix at `weights + 4 * w_off4 + FC_MADE_RECORD_FLOATS` (row-major, masked,
  * zero-padded; the FC_MADE_RECORD_FLOATS words in front of it are a bit copy of the phase's own record, which the kernel
  * receives through its weight ring instead of reading `phases` on the serial chain; width <= 1920) whose
@@ -458,12 +458,23 @@ int fc_conditioner_profile(unsigned long long* out32);
  * feature >= 0 the bijection's inverse of that feature is evaluated from the parameter tile.  Shared memory bounds the
  * network: fc_made_inverse_smem_bytes(...) must not exceed the device's opt-in limit (FC_ERR_UNSUPPORTED otherwise: run the
  * D-pass inverse).
+ *
+ * Context (a MADE with context_features): the context terms do not depend on x, so they are computed for the whole batch
+ * first — `terms` is this call's [B, term_width] matrix g = Wc ctx + bc in the T128 layout (fc_context_terms or
+ * fc_linear_apply with FC_LINEAR_OUT_T128).  Each of the n_term_arrays entries names a hidden array whose units start
+ * every row tile from bias[b_off + j] + act(terms[row][column + j]) instead of being written with FC_MADE_INIT_BIAS:
+ *   relu = 1  MADE initial layer             h = W x + b + relu(Wc ctx + bc)      (made.py:138-140)
+ *   relu = 0  first layer of a residual block t = W0 relu(h) + b0 + Wc ctx + bc  (made.py:100-102)
+ * so the tasks that write such an array must not set FC_MADE_INIT_BIAS.  term_width is a multiple of 16, column a multiple
+ * of 4 with column + hidden <= term_width, b_off + hidden <= n_bias, each array 1 .. n_arrays at most once, `terms`
+ * 16-byte aligned; anything else is FC_ERR_INVALID_ARGUMENT.  n_term_arrays = 0 (terms NULL): a MADE without context.
  */
 #define FC_MADE_MAX_NJ 24
 #define FC_MADE_TASKS 8
 #define FC_MADE_RECORD_FLOATS 128 /* the phase's record, struct fc_made_phase padded to 512 bytes, precedes its matrix in `weights` */
 #define FC_MADE_RELU_IN 1
 #define FC_MADE_INIT_BIAS 2
+#define FC_MADE_MAX_TERM_ARRAYS 8
 typedef struct fc_made_task {
   int32_t in_array, out_array, k0, kn;
   int32_t j0, nj, c0, flags;
@@ -473,12 +484,21 @@ typedef struct fc_made_phase {
   int32_t rows, width, w_off4, feature;
   fc_made_task tasks[FC_MADE_TASKS];
 } fc_made_phase;
+typedef struct fc_made_term_array {
+  int32_t array;  /* hidden array 1 .. n_arrays whose units start from bias + act(term) */
+  int32_t column; /* first column of its units in `terms` (a multiple of 4): unit j reads column + j */
+  int32_t b_off;  /* the layer's bias inside `bias` */
+  int32_t relu;   /* 1: act = ReLU (MADE initial layer), 0: identity (first layer of a block) */
+} fc_made_term_array;
 typedef struct fc_made_program {
   const fc_made_phase* phases; /* device, 16-byte aligned */
   const float* weights;        /* device, 16-byte aligned */
   const float* bias;           /* device */
   int32_t n_phases, features, params_per_feature, n_arrays, hidden;
   int32_t n_bias;              /* floats in `bias` (staged in shared memory) */
+  const float* terms;          /* device, this call's context terms [B, term_width] in T128; NULL when n_term_arrays == 0 */
+  int32_t term_width, n_term_arrays;
+  fc_made_term_array term_arrays[FC_MADE_MAX_TERM_ARRAYS];
 } fc_made_program;
 /* Debugging aid (library built with -DFC_MADE_PROFILE=1, else all zero): cycles warp 0 ([0..6]) and warp 5 ([8..14]) of CTA 0
  * spent in the last fc_made_inverse_* launch: [0] reading phase records, [1] waiting for weight slots, [2] multiplying,
