@@ -549,6 +549,83 @@ actnorm_layer.register_autograd(_actnorm_backward, setup_context=_actnorm_setup)
 
 
 # ------------------------------------------------------------------------------------------------
+# dense D x D row map of LULinear (D < 64): y = x M^T + c, logabsdet = logdet on every row
+# ------------------------------------------------------------------------------------------------
+def _lu_operands(M, c, D):
+    if M.shape != (D, D) or c.numel() != D:
+        raise ValueError("M must be [{0}, {0}] and c must have {0} entries".format(D))
+    return M.contiguous(), c.contiguous()
+
+
+@torch.library.custom_op("flowcon_b200::lulinear_layer", mutates_args=())
+def lulinear_layer(x: Tensor, M: Tensor, c: Tensor, logdet: Tensor) -> Tuple[Tensor, Tensor]:
+    _cabi.require_cuda_f32(x, "inputs")
+    _cabi.require_cuda_f32(M, "M")
+    _cabi.require_cuda_f32(c, "c")
+    _cabi.require_cuda_f32(logdet, "logdet")
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    B, D = x.shape
+    M, c = _lu_operands(M, c, D)
+    logdet = logdet.reshape(()).contiguous()
+    y = torch.empty((B, D), dtype=x.dtype, device=x.device)
+    lad = torch.empty((B,), dtype=x.dtype, device=x.device)
+    with torch.cuda.device(x.device), _cabi.launch("fc_lulinear_apply", x.device):
+        rc = L.fc_lulinear_apply(xp, xs, M.data_ptr(), c.data_ptr(), logdet.data_ptr(), y.data_ptr(), D, lad.data_ptr(),
+                                 0, B, D, _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_lulinear_apply")
+    return y, lad
+
+
+@lulinear_layer.register_fake
+def _(x, M, c, logdet):
+    return x.new_empty(x.shape), x.new_empty((x.shape[0],))
+
+
+@torch.library.custom_op("flowcon_b200::lulinear_layer_backward", mutates_args=())
+def lulinear_layer_backward(x: Tensor, M: Tensor, grad_y: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    """(grad_x, grad_M, grad_c) of y = x M^T + c; grad_logdet = sum(grad_logabsdet) is left to the caller."""
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    grad_y, gyp, gys = _cabi.rows(_cabi.require_cuda_f32(grad_y, "grad outputs"))
+    B, D = x.shape
+    M = M.contiguous()
+    gx = torch.empty((B, D), dtype=x.dtype, device=x.device)
+    gM = torch.empty((D, D), dtype=x.dtype, device=x.device)
+    gc = torch.empty((D,), dtype=x.dtype, device=x.device)
+    ws = torch.empty((max(int(L.fc_lulinear_workspace_floats(B, D)), 1),), dtype=x.dtype, device=x.device)
+    with torch.cuda.device(x.device), _cabi.launch("fc_lulinear_backward", x.device):
+        rc = L.fc_lulinear_backward(xp, xs, M.data_ptr(), gyp, gys, gx.data_ptr(), D, gM.data_ptr(), gc.data_ptr(),
+                                    ws.data_ptr(), B, D, _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_lulinear_backward")
+    return gx, gM, gc
+
+
+@lulinear_layer_backward.register_fake
+def _(x, M, grad_y):
+    D = x.shape[1]
+    return x.new_empty(x.shape), x.new_empty((D, D)), x.new_empty((D,))
+
+
+def _lulinear_setup(ctx, inputs, output):
+    x, M, c, logdet = inputs
+    ctx.save_for_backward(x, M)
+    ctx.c_shape, ctx.logdet_shape = c.shape, logdet.shape
+
+
+def _lulinear_backward(ctx, gy, gl):
+    x, M = ctx.saved_tensors
+    if gy is None:
+        gy = torch.zeros_like(x)
+    gx, gM, gc = lulinear_layer_backward(x, M, gy)
+    gld = gl.sum() if gl is not None else x.new_zeros(())
+    return gx, gM, gc.reshape(ctx.c_shape), gld.reshape(ctx.logdet_shape)
+
+
+lulinear_layer.register_autograd(_lulinear_backward, setup_context=_lulinear_setup)
+
+
+# ------------------------------------------------------------------------------------------------
 # sum-of-sigmoids layer
 # ------------------------------------------------------------------------------------------------
 @torch.library.custom_op("flowcon_b200::sos_layer", mutates_args=())

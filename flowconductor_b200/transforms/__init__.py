@@ -17,6 +17,7 @@ from .coupling import (AdditiveCouplingTransform, AffineCouplingTransform, Coupl
 from .made import MADE, MaskedLinear  # noqa: F401
 from .nonlinearities import (PiecewiseCubicCDF, PiecewiseLinearCDF, PiecewiseQuadraticCDF,  # noqa: F401
                             PiecewiseRationalQuadraticCDF)
+from .lu import LULinear  # noqa: F401
 from .normalization import ActNorm  # noqa: F401
 from .permutations import Permutation, RandomPermutation, ReversePermutation  # noqa: F401
 from . import splines  # noqa: F401

@@ -29,6 +29,15 @@ def _maf_prq_stack(features, num_layers, num_bins, hidden, tail_bound=3.0):
     return layers
 
 
+def _nsf_lu_stack(features, num_layers, num_bins, hidden, tail_bound=3.0):
+    """Neural spline flow (Durkan et al. 2019): every coupling layer followed by LULinear(features, identity_init=True)."""
+    layers = []
+    for layer in _prq_coupling_stack(features, num_layers, num_bins, hidden, tail_bound):
+        layers.append(layer)
+        layers.append({"kind": "lu_linear", "identity_init": True})
+    return layers
+
+
 WORKLOADS = {
     # cfg 1: README.md:86-98 model (MAF(2, 4) + RandomPermutation), evaluated on 2-D toy batches
     "cfg1": {"features": 2, "context_features": None, "batch": 10000,
@@ -119,6 +128,9 @@ WORKLOADS = {
                                    "layers": [{"kind": "prq_coupling", "mask": "mid_split", "num_bins": 5,
                                                "tails": None, "tail_bound": 1.0, "hidden_features": 16,
                                                "num_blocks": 2}]},
+    # LU-factorised linear layers between the couplings (flowcon/transforms/lu.py): cfg 2's stack at D = 32
+    "nsf_lu": {"features": 32, "context_features": None, "batch": 1 << 20, "layers": _nsf_lu_stack(32, 8, 8, 256)},
+    "nsf_lu_small": {"features": 6, "context_features": None, "batch": 64, "layers": _nsf_lu_stack(6, 2, 8, 16)},
 }
 
 
@@ -192,6 +204,13 @@ def trained_like_(state, workload, seed=1, weight_gain=8.0):
                 state[key] = state[key] + std * torch.randn(state[key].numel(), generator=g, dtype=torch.float32).to(
                     state[key].dtype)
             continue
+        if kind == "lu_linear":  # a trained LULinear is far from the identity: entries at the non-identity init scale
+            for name in ("bias", "lower_entries", "upper_entries", "unconstrained_upper_diag"):
+                key = layer_prefix(i) + name
+                bound = 1.0 / workload["features"] ** 0.5
+                u = torch.rand(state[key].numel(), generator=g, dtype=torch.float32) * 2.0 - 1.0
+                state[key] = (bound * u).to(state[key].dtype)
+            continue
         net = {"prq_coupling": "transform_net", "affine_coupling": "transform_net", "maf_affine": "autoregressive_net",
                "maf_prq": "autoregressive_net", "maf_sos": "autoregressive_net", "cond_sos": "conditional_net",
                "cond_prq": "conditional_net", "plin_coupling": "transform_net", "maf_plin": "autoregressive_net",
@@ -231,6 +250,8 @@ def build_flow(workload, seed=0):
             layers.append(cls(features))
         elif kind == "actnorm":
             layers.append(transforms.ActNorm(features))
+        elif kind == "lu_linear":
+            layers.append(transforms.LULinear(features, identity_init=layer.get("identity_init", True)))
         elif kind == "prq_coupling":
             hidden, blocks = layer["hidden_features"], layer["num_blocks"]
             layers.append(transforms.PiecewiseRationalQuadraticCouplingTransform(

@@ -549,6 +549,25 @@ int fc_actnorm_backward(const float* x, int64_t x_row_stride, const float* log_s
                         float* grad_log_scale, float* grad_shift, float* workspace, int64_t B, int32_t D, int32_t inverse,
                         void* stream);
 
+/*
+ * Dense D x D row map of the LU-factorised linear layer (csrc/fc_lulinear.cu; LULinear, flowcon/transforms/lu.py on top of
+ * flowcon/transforms/linear.py) for 1 <= D <= 63:  y = x · Mᵀ + c,  logabsdet[b] = *logdet (written, or added to with
+ * accumulate_logabsdet).  M: device [D, D] row-major, c: device [D], logdet: device scalar — the caller composes them from
+ * the LU factors (forward M = L U, c = bias; inverse M = U⁻¹ L⁻¹, c = -M bias), so nothing is read back to the host and
+ * the call can be captured into a CUDA graph.  x and y are [B, D] with their own row strides (>= D), so column slices of
+ * wider tensors work; any B.  D outside [1, 63] returns FC_ERR_INVALID_ARGUMENT (wider maps are tensor-core GEMMs).
+ * The backward reads (x, grad_y) once and writes grad_x = grad_y · M, grad_M = grad_yᵀ · x and grad_c = Σ_b grad_y[b]
+ * (per-CTA partial sums summed in a fixed order: deterministic); workspace: fc_lulinear_workspace_floats(B, D) floats of
+ * device scratch.  grad_logdet = Σ_b grad_logabsdet[b] is left to the caller.
+ */
+int fc_lulinear_apply(const float* x, int64_t x_row_stride, const float* M, const float* c, const float* logdet, float* y,
+                      int64_t y_row_stride, float* logabsdet, int32_t accumulate_logabsdet, int64_t B, int32_t D,
+                      void* stream);
+int64_t fc_lulinear_workspace_floats(int64_t B, int32_t D);
+int fc_lulinear_backward(const float* x, int64_t x_row_stride, const float* M, const float* grad_y, int64_t gy_row_stride,
+                         float* grad_x, int64_t gx_row_stride, float* grad_M, float* grad_c, float* workspace, int64_t B,
+                         int32_t D, void* stream);
+
 /* Library / build info (also used by the loader test). */
 const char* fc_version(void);
 int fc_built_for_sm(void); /* 100 */
