@@ -18,6 +18,7 @@ STATUS_INPUT_OUTSIDE_DOMAIN = 1
 STATUS_NEGATIVE_DISCRIMINANT = 2
 TAILS_NONE, TAILS_LINEAR = 0, 1
 AFFINE_BLOCKED, AFFINE_INTERLEAVED = 0, 1
+BATCHNORM_TRAIN, BATCHNORM_EVAL_FORWARD, BATCHNORM_EVAL_INVERSE = 0, 1, 2
 SCALE_SIGMOID2, SCALE_SOFTPLUS_CLAMP3, SCALE_SOFTPLUS_EPS = 0, 1, 2
 LINEAR_A_T128, LINEAR_OUT_T128, LINEAR_RESIDUAL_GATES = 1, 2, 4
 
@@ -29,6 +30,7 @@ EXPORTS = ["fc_rqs_apply", "fc_rqs_backward", "fc_rqs_bins", "fc_linspline_apply
            "fc_elementwise_last_path", "fc_conditioner_layer_bytes", "fc_conditioner_pack_layer", "fc_conditioner_rqs_apply", "fc_conditioner_sos_apply", "fc_conditioner_affine_apply", "fc_conditioner_store_apply", "fc_context_terms", "fc_conditioner_error", "fc_conditioner_profile",
            "fc_actnorm_apply", "fc_actnorm_workspace_floats", "fc_actnorm_backward",
            "fc_lulinear_apply", "fc_lulinear_workspace_floats", "fc_lulinear_backward",
+           "fc_batchnorm_workspace_floats", "fc_batchnorm_stats", "fc_batchnorm_apply", "fc_batchnorm_backward",
            "fc_made_inverse_smem_bytes", "fc_made_inverse_profile", "fc_made_inverse_rqs", "fc_made_inverse_affine",
            "fc_made_inverse_sos", "fc_made_inverse_linspline", "fc_made_inverse_quadspline", "fc_made_inverse_cubicspline",
            "fc_version", "fc_built_for_sm"]
@@ -159,6 +161,11 @@ def lib():
         L.fc_lulinear_apply.argtypes = [vp, i64, vp, vp, vp, vp, i64, vp, i32, i64, i32, vp]
         L.fc_lulinear_workspace_floats.argtypes = [i64, i32]
         L.fc_lulinear_backward.argtypes = [vp, i64, vp, vp, i64, vp, i64, vp, vp, vp, i64, i32, vp]
+        L.fc_batchnorm_workspace_floats.argtypes = [i64, i32]
+        L.fc_batchnorm_stats.argtypes = [vp, i64, vp, vp, vp, i64, i32, vp]
+        L.fc_batchnorm_apply.argtypes = [vp, i64, vp, vp, vp, vp, f32, vp, i64, vp, i64, i32, i32, vp]
+        L.fc_batchnorm_backward.argtypes = [vp, i64, vp, vp, vp, vp, f32, vp, i64, vp, vp, i64, vp, vp, vp, i64, i32,
+                                            i32, vp]
         L.fc_made_inverse_smem_bytes.argtypes = [i32, i32, i32, i32, i32]
         L.fc_made_inverse_profile.argtypes = [ctypes.POINTER(ctypes.c_uint64)]
         L.fc_made_inverse_rqs.argtypes = [ctypes.POINTER(MadeProgramStruct), vp, i64, vp, i64, vp, i32, i64,
@@ -179,6 +186,7 @@ def lib():
         L.fc_made_inverse_smem_bytes.restype = ctypes.c_int64
         L.fc_actnorm_workspace_floats.restype = ctypes.c_int64
         L.fc_lulinear_workspace_floats.restype = ctypes.c_int64
+        L.fc_batchnorm_workspace_floats.restype = ctypes.c_int64
         _lib = L
     return _lib
 

@@ -137,8 +137,8 @@ class GraphedTrainStep:
     * the optimizer must be capturable (`torch.optim.Adam(..., capturable=True)`): its step counter lives on the device;
     * `sync_gradients` (e.g. `distributed.allreduce_gradients`) is captured with the rest — NCCL collectives are
       graph-capturable;
-    * the warm-up steps needed before capture run on the example batch and are UNDONE afterwards (parameters and
-      optimizer state are restored in place), so constructing the object does not train.
+    * the warm-up steps needed before capture run on the example batch and are UNDONE afterwards (parameters, running
+      statistics and optimizer state are restored in place), so constructing the object does not train.
     `step(*inputs)` copies the batch into the static buffers, replays, and returns the (static) loss tensor."""
 
     def __init__(self, module, optimizer, loss_fn, *example_inputs, sync_gradients=None, warmup=3):
@@ -152,6 +152,9 @@ class GraphedTrainStep:
         self.device = self._static_in[0].device
         params = [p for p in module.parameters()]
         saved_params = [p.detach().clone() for p in params]
+        # running statistics (BatchNorm) move during the warm-up too
+        buffers = [b for b in module.buffers() if b.is_floating_point()]
+        saved_buffers = [b.clone() for b in buffers]
         # optimizer state that already exists (training resumed) is restored; state created by the warm-up is zeroed
         prior = {id(t): t.detach().clone() for st in optimizer.state.values() for t in st.values()
                  if isinstance(t, torch.Tensor)}
@@ -179,7 +182,7 @@ class GraphedTrainStep:
             # undo the warm-up (and the capture itself does not execute): parameters back to their values, optimizer
             # state back to "zero steps taken"
             with torch.no_grad():
-                for p, s0 in zip(params, saved_params):
+                for p, s0 in zip(params + buffers, saved_params + saved_buffers):
                     p.copy_(s0)
                 for st in optimizer.state.values():
                     for t in st.values():

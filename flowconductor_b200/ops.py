@@ -626,6 +626,149 @@ lulinear_layer.register_autograd(_lulinear_backward, setup_context=_lulinear_set
 
 
 # ------------------------------------------------------------------------------------------------
+# batch normalisation (BatchNorm): per-feature statistics of the batch (training) or running buffers (eval)
+# ------------------------------------------------------------------------------------------------
+def _bn_vectors(D, **named):
+    for name, t in named.items():
+        _cabi.require_cuda_f32(t, name)
+        if t.numel() != D:
+            raise ValueError("{} must have {} entries".format(name, D))
+    return [t.contiguous() for t in named.values()]
+
+
+def _bn_apply(x, mean, var, uw, bias, eps, inverse):
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    B, D = x.shape
+    y = torch.empty((B, D), dtype=x.dtype, device=x.device)
+    lad = torch.empty((B,), dtype=x.dtype, device=x.device)
+    with torch.cuda.device(x.device), _cabi.launch("fc_batchnorm_apply", x.device):
+        rc = L.fc_batchnorm_apply(xp, xs, mean.data_ptr(), var.data_ptr(), uw.data_ptr(), bias.data_ptr(), eps,
+                                  y.data_ptr(), D, lad.data_ptr(), B, D, int(inverse), _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_batchnorm_apply")
+    return y, lad
+
+
+def _bn_workspace(L, B, D, device):
+    n = int(L.fc_batchnorm_workspace_floats(B, D))
+    if n < 0:
+        _cabi.check(n, "fc_batchnorm_workspace_floats")
+    return torch.empty((max(n, 1),), dtype=torch.float32, device=device)
+
+
+@torch.library.custom_op("flowcon_b200::batchnorm_train", mutates_args=())
+def batchnorm_train(x: Tensor, unconstrained_weight: Tensor, bias: Tensor,
+                    eps: float) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """Training-mode BatchNorm: (y, logabsdet, batch mean, unbiased batch variance).  Three launches: the statistics
+    (per-CTA Welford, then a fixed-order merge) and the forward pass.  The statistics outputs carry no gradient."""
+    _cabi.require_cuda_f32(x, "inputs")
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    B, D = x.shape
+    uw, bias = _bn_vectors(D, unconstrained_weight=unconstrained_weight, bias=bias)
+    mean = torch.empty((D,), dtype=x.dtype, device=x.device)
+    var = torch.empty((D,), dtype=x.dtype, device=x.device)
+    ws = _bn_workspace(L, B, D, x.device)
+    with torch.cuda.device(x.device), _cabi.launch("fc_batchnorm_stats", x.device):
+        rc = L.fc_batchnorm_stats(xp, xs, mean.data_ptr(), var.data_ptr(), ws.data_ptr(), B, D,
+                                  _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_batchnorm_stats")
+    y, lad = _bn_apply(x, mean, var, uw, bias, eps, False)
+    return y, lad, mean, var
+
+
+@batchnorm_train.register_fake
+def _(x, unconstrained_weight, bias, eps):
+    D = x.shape[1]
+    return torch.empty_like(x), x.new_empty((x.shape[0],)), x.new_empty((D,)), x.new_empty((D,))
+
+
+@torch.library.custom_op("flowcon_b200::batchnorm_eval", mutates_args=())
+def batchnorm_eval(x: Tensor, running_mean: Tensor, running_var: Tensor, unconstrained_weight: Tensor, bias: Tensor,
+                   eps: float, inverse: bool) -> Tuple[Tensor, Tensor]:
+    """Eval-mode BatchNorm in either direction, from the running buffers: (y, logabsdet).  One launch."""
+    _cabi.require_cuda_f32(x, "inputs")
+    D = x.shape[1]
+    rm, rv, uw, bias = _bn_vectors(D, running_mean=running_mean, running_var=running_var,
+                                   unconstrained_weight=unconstrained_weight, bias=bias)
+    return _bn_apply(x, rm, rv, uw, bias, eps, inverse)
+
+
+@batchnorm_eval.register_fake
+def _(x, running_mean, running_var, unconstrained_weight, bias, eps, inverse):
+    return torch.empty_like(x), x.new_empty((x.shape[0],))
+
+
+@torch.library.custom_op("flowcon_b200::batchnorm_backward", mutates_args=())
+def batchnorm_backward(x: Tensor, mean: Tensor, var: Tensor, unconstrained_weight: Tensor, bias: Tensor, eps: float,
+                       grad_y: Tensor, grad_lad: Optional[Tensor], mode: int) -> Tuple[Tensor, Tensor, Tensor]:
+    """(grad_x, grad_unconstrained_weight, grad_bias); mode _cabi.BATCHNORM_TRAIN differentiates through the batch
+    statistics (mean, var), the eval modes treat them as constants."""
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    grad_y, gyp, gys = _cabi.rows(_cabi.require_cuda_f32(grad_y, "grad outputs"))
+    B, D = x.shape
+    mean, var, uw, bias = (t.contiguous() for t in (mean, var, unconstrained_weight, bias))
+    gx = torch.empty((B, D), dtype=x.dtype, device=x.device)
+    guw = torch.empty((D,), dtype=x.dtype, device=x.device)
+    gb = torch.empty((D,), dtype=x.dtype, device=x.device)
+    ws = _bn_workspace(L, B, D, x.device)
+    glp = None
+    if grad_lad is not None:
+        grad_lad = grad_lad.contiguous()
+        glp = grad_lad.data_ptr()
+    with torch.cuda.device(x.device), _cabi.launch("fc_batchnorm_backward", x.device):
+        rc = L.fc_batchnorm_backward(xp, xs, mean.data_ptr(), var.data_ptr(), uw.data_ptr(), bias.data_ptr(), eps, gyp,
+                                     gys, glp, gx.data_ptr(), D, guw.data_ptr(), gb.data_ptr(), ws.data_ptr(), B, D,
+                                     int(mode), _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_batchnorm_backward")
+    return gx, guw, gb
+
+
+@batchnorm_backward.register_fake
+def _(x, mean, var, unconstrained_weight, bias, eps, grad_y, grad_lad, mode):
+    D = x.shape[1]
+    return torch.empty_like(x), x.new_empty((D,)), x.new_empty((D,))
+
+
+def _bn_train_setup(ctx, inputs, output):
+    x, uw, bias, eps = inputs
+    _, _, mean, var = output
+    ctx.save_for_backward(x, mean, var, uw, bias)
+    ctx.eps = eps
+    ctx.mark_non_differentiable(mean, var)
+
+
+def _bn_train_backward(ctx, gy, gl, _gmean, _gvar):
+    x, mean, var, uw, bias = ctx.saved_tensors
+    if gy is None:
+        gy = torch.zeros_like(x)
+    gx, guw, gb = batchnorm_backward(x, mean, var, uw, bias, ctx.eps, gy, gl, _cabi.BATCHNORM_TRAIN)
+    return gx, guw.reshape(uw.shape), gb.reshape(bias.shape), None
+
+
+batchnorm_train.register_autograd(_bn_train_backward, setup_context=_bn_train_setup)
+
+
+def _bn_eval_setup(ctx, inputs, output):
+    x, rm, rv, uw, bias, eps, inverse = inputs
+    ctx.save_for_backward(x, rm, rv, uw, bias)
+    ctx.eps, ctx.inverse = eps, inverse
+
+
+def _bn_eval_backward(ctx, gy, gl):
+    x, rm, rv, uw, bias = ctx.saved_tensors
+    if gy is None:
+        gy = torch.zeros_like(x)
+    mode = _cabi.BATCHNORM_EVAL_INVERSE if ctx.inverse else _cabi.BATCHNORM_EVAL_FORWARD
+    gx, guw, gb = batchnorm_backward(x, rm, rv, uw, bias, ctx.eps, gy, gl, mode)
+    return gx, None, None, guw.reshape(uw.shape), gb.reshape(bias.shape), None, None
+
+
+batchnorm_eval.register_autograd(_bn_eval_backward, setup_context=_bn_eval_setup)
+
+
+# ------------------------------------------------------------------------------------------------
 # sum-of-sigmoids layer
 # ------------------------------------------------------------------------------------------------
 @torch.library.custom_op("flowcon_b200::sos_layer", mutates_args=())

@@ -18,7 +18,7 @@ from .made import MADE, MaskedLinear  # noqa: F401
 from .nonlinearities import (PiecewiseCubicCDF, PiecewiseLinearCDF, PiecewiseQuadraticCDF,  # noqa: F401
                             PiecewiseRationalQuadraticCDF)
 from .lu import LULinear  # noqa: F401
-from .normalization import ActNorm  # noqa: F401
+from .normalization import ActNorm, BatchNorm  # noqa: F401
 from .permutations import Permutation, RandomPermutation, ReversePermutation  # noqa: F401
 from . import splines  # noqa: F401
 from .splines import (cubic_spline, linear_spline, quadratic_spline, rational_quadratic_spline,  # noqa: F401

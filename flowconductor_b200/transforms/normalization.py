@@ -1,12 +1,65 @@
-"""`ActNorm` with the API and state_dict of flowcon/transforms/normalization.py:144-218 (2-D inputs): a per-feature affine
-map whose scale and shift are learnable and, in training mode, initialised from the first batch so that the outputs have
-zero mean and unit variance.  Forward / inverse / gradients run in csrc/fc_actnorm.cu (SURVEY.md 8(f) n4)."""
+"""`BatchNorm` and `ActNorm` with the API and state_dict of flowcon/transforms/normalization.py (2-D inputs).
+
+`BatchNorm` normalises every feature with the statistics of the batch in training mode (mean and UNBIASED variance, also
+folded into the running buffers with `momentum`) and with the running buffers in eval mode, then applies a learnable
+positive scale and a shift; its inverse exists in eval mode only.  Statistics, forward / inverse and gradients run in
+csrc/fc_batchnorm.cu.
+
+`ActNorm` is a per-feature affine map whose scale and shift are learnable and, in training mode, initialised from the
+first batch so that the outputs have zero mean and unit variance.  Forward / inverse / gradients run in csrc/fc_actnorm.cu
+(SURVEY.md 8(f) n4)."""
+import numpy as np
 import torch
 from torch import nn
+from torch.nn import functional as F
 
 from .. import ops
 from ..utils import typechecks as check
-from .base import Transform
+from .base import InverseNotAvailable, Transform
+
+
+class BatchNorm(Transform):
+    """`affine` is accepted and unused, as in the reference."""
+
+    def __init__(self, features, eps=1e-5, momentum=0.1, affine=True):
+        if not check.is_positive_int(features):
+            raise TypeError("Number of features must be a positive integer.")
+        super().__init__()
+        self.momentum = momentum
+        self.eps = eps
+        constant = np.log(np.exp(1 - eps) - 1)
+        self.unconstrained_weight = nn.Parameter(constant * torch.ones(features))
+        self.bias = nn.Parameter(torch.zeros(features))
+        self.register_buffer("running_mean", torch.zeros(features))
+        self.register_buffer("running_var", torch.zeros(features))
+
+    @property
+    def weight(self):
+        return F.softplus(self.unconstrained_weight) + self.eps
+
+    @staticmethod
+    def _check(inputs):
+        if inputs.dim() != 2:
+            raise ValueError("Expected 2-dim inputs, got inputs of shape: {}".format(inputs.shape))
+
+    def forward(self, inputs, context=None):
+        self._check(inputs)
+        if not self.training:
+            return ops.batchnorm_eval(inputs, self.running_mean, self.running_var, self.unconstrained_weight, self.bias,
+                                      self.eps, False)
+        outputs, logabsdet, mean, var = ops.batchnorm_train(inputs, self.unconstrained_weight, self.bias, self.eps)
+        # the reference's own in-place update, so the running buffers round exactly as there (six launches on [D])
+        with torch.no_grad():
+            self.running_mean.mul_(1 - self.momentum).add_(mean * self.momentum)
+            self.running_var.mul_(1 - self.momentum).add_(var * self.momentum)
+        return outputs, logabsdet
+
+    def inverse(self, inputs, context=None):
+        if self.training:
+            raise InverseNotAvailable("Batch norm inverse is only available in eval mode, not in training mode.")
+        self._check(inputs)
+        return ops.batchnorm_eval(inputs, self.running_mean, self.running_var, self.unconstrained_weight, self.bias,
+                                  self.eps, True)
 
 
 class ActNorm(Transform):

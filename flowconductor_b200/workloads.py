@@ -38,6 +38,27 @@ def _nsf_lu_stack(features, num_layers, num_bins, hidden, tail_bound=3.0):
     return layers
 
 
+def _maf_bn_stack(num_layers, hidden, num_blocks=2):
+    """flows.MaskedAutoregressiveFlow(..., batch_norm_between_layers=True): reverse permutation, MAF-affine, BatchNorm."""
+    layers = []
+    for _ in range(num_layers):
+        layers.append({"kind": "permutation", "mode": "reverse"})
+        layers.append({"kind": "maf_affine", "hidden_features": hidden, "num_blocks": num_blocks})
+        layers.append({"kind": "batchnorm"})
+    return layers
+
+
+def _realnvp_bn_stack(num_layers, hidden, num_blocks=2):
+    """flows.SimpleRealNVP(..., batch_norm_between_layers=True): affine couplings on the odd, then the even features
+    (the reference's mask[::2] = -1, negated after every layer), each followed by BatchNorm."""
+    layers = []
+    for i in range(num_layers):
+        layers.append({"kind": "affine_coupling", "mask": "alternating_odd" if i % 2 == 0 else "alternating_even",
+                       "hidden_features": hidden, "num_blocks": num_blocks, "scale_activation": "sigmoid2"})
+        layers.append({"kind": "batchnorm"})
+    return layers
+
+
 WORKLOADS = {
     # cfg 1: README.md:86-98 model (MAF(2, 4) + RandomPermutation), evaluated on 2-D toy batches
     "cfg1": {"features": 2, "context_features": None, "batch": 10000,
@@ -131,6 +152,11 @@ WORKLOADS = {
     # LU-factorised linear layers between the couplings (flowcon/transforms/lu.py): cfg 2's stack at D = 32
     "nsf_lu": {"features": 32, "context_features": None, "batch": 1 << 20, "layers": _nsf_lu_stack(32, 8, 8, 256)},
     "nsf_lu_small": {"features": 6, "context_features": None, "batch": 64, "layers": _nsf_lu_stack(6, 2, 8, 16)},
+    # BatchNorm between layers (flowcon/flows/autoregressive.py, flowcon/flows/realnvp.py): the packaged flows'
+    # layering; maf_bn is a MAF-affine training workload at D = 43, so the BatchNorm kernels take their unaligned path
+    "maf_bn_small": {"features": 6, "context_features": None, "batch": 128, "layers": _maf_bn_stack(2, 16)},
+    "realnvp_bn_small": {"features": 6, "context_features": None, "batch": 128, "layers": _realnvp_bn_stack(2, 16)},
+    "maf_bn": {"features": 43, "context_features": None, "batch": 262144, "layers": _maf_bn_stack(5, 256)},
 }
 
 
@@ -204,6 +230,12 @@ def trained_like_(state, workload, seed=1, weight_gain=8.0):
                 state[key] = state[key] + std * torch.randn(state[key].numel(), generator=g, dtype=torch.float32).to(
                     state[key].dtype)
             continue
+        if kind == "batchnorm":  # trained: weights away from 1, a shift, running statistics of a non-white input
+            p = layer_prefix(i)
+            for name, std in (("unconstrained_weight", 0.4), ("bias", 0.5), ("running_mean", 0.8)):
+                state[p + name] = state[p + name] + std * torch.randn(state[p + name].numel(), generator=g)
+            state[p + "running_var"] = torch.exp(0.6 * torch.randn(state[p + "running_var"].numel(), generator=g))
+            continue
         if kind == "lu_linear":  # a trained LULinear is far from the identity: entries at the non-identity init scale
             for name in ("bias", "lower_entries", "upper_entries", "unconstrained_upper_diag"):
                 key = layer_prefix(i) + name
@@ -250,6 +282,8 @@ def build_flow(workload, seed=0):
             layers.append(cls(features))
         elif kind == "actnorm":
             layers.append(transforms.ActNorm(features))
+        elif kind == "batchnorm":
+            layers.append(transforms.BatchNorm(features))
         elif kind == "lu_linear":
             layers.append(transforms.LULinear(features, identity_init=layer.get("identity_init", True)))
         elif kind == "prq_coupling":

@@ -568,6 +568,38 @@ int fc_lulinear_backward(const float* x, int64_t x_row_stride, const float* M, c
                          float* grad_x, int64_t gx_row_stride, float* grad_M, float* grad_c, float* workspace, int64_t B,
                          int32_t D, void* stream);
 
+/*
+ * Batch normalisation as a flow layer (csrc/fc_batchnorm.cu; BatchNorm, flowcon/transforms/normalization.py, 2-D inputs)
+ * for 1 <= D <= 4096 in every entry (wider: FC_ERR_UNSUPPORTED).  With w = softplus(unconstrained_weight) + eps and
+ * σ = sqrt(var + eps) per feature:
+ *   forward  y = w · ((x − mean) / σ) + bias,     logabsdet[b] = Σ_d (log w_d − ½ log(var_d + eps))
+ *   inverse  y = σ · ((x − bias) / w) + mean,     logabsdet[b] = −Σ_d (log w_d − ½ log(var_d + eps))
+ * The mean is subtracted (the bias, inverse) before the scale is applied, never folded into one shift.  mean, var,
+ * unconstrained_weight, bias: device [D], read by the kernels (a captured graph sees later updates of them).
+ * fc_batchnorm_stats writes the batch mean and the UNBIASED variance (B - 1; NaN for B = 1, as torch.var) of x [B, D],
+ * B >= 1: Welford per thread, Chan merges in a fixed order, no atomics — two calls are bitwise equal.
+ * fc_batchnorm_backward, mode FC_BATCHNORM_TRAIN (mean / var are the batch statistics of x, differentiated through),
+ * FC_BATCHNORM_EVAL_FORWARD or FC_BATCHNORM_EVAL_INVERSE (running buffers, constants): grad_x, and the gradients of
+ * unconstrained_weight and bias (deterministic, per-CTA partial sums summed in a fixed order); grad_logabsdet may be
+ * null.  Training mode reads x and grad_y twice (column sums, then grad_x: three launches), eval mode once (two).
+ * workspace: fc_batchnorm_workspace_floats(B, D) floats of device scratch, for the statistics and the backward.
+ * x, y and the gradients are [B, D] with their own row strides (>= D); any B >= 0 (stats: B >= 1).
+ */
+#define FC_BATCHNORM_TRAIN 0
+#define FC_BATCHNORM_EVAL_FORWARD 1
+#define FC_BATCHNORM_EVAL_INVERSE 2
+int64_t fc_batchnorm_workspace_floats(int64_t B, int32_t D);
+int fc_batchnorm_stats(const float* x, int64_t x_row_stride, float* mean, float* var, float* workspace, int64_t B,
+                       int32_t D, void* stream);
+int fc_batchnorm_apply(const float* x, int64_t x_row_stride, const float* mean, const float* var,
+                       const float* unconstrained_weight, const float* bias, float eps, float* y, int64_t y_row_stride,
+                       float* logabsdet, int64_t B, int32_t D, int32_t inverse, void* stream);
+int fc_batchnorm_backward(const float* x, int64_t x_row_stride, const float* mean, const float* var,
+                          const float* unconstrained_weight, const float* bias, float eps, const float* grad_y,
+                          int64_t gy_row_stride, const float* grad_logabsdet, float* grad_x, int64_t gx_row_stride,
+                          float* grad_unconstrained_weight, float* grad_bias, float* workspace, int64_t B, int32_t D,
+                          int32_t mode, void* stream);
+
 /* Library / build info (also used by the loader test). */
 const char* fc_version(void);
 int fc_built_for_sm(void); /* 100 */
