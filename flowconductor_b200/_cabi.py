@@ -31,6 +31,8 @@ EXPORTS = ["fc_rqs_apply", "fc_rqs_backward", "fc_rqs_bins", "fc_linspline_apply
            "fc_actnorm_apply", "fc_actnorm_workspace_floats", "fc_actnorm_backward",
            "fc_lulinear_apply", "fc_lulinear_workspace_floats", "fc_lulinear_backward",
            "fc_batchnorm_workspace_floats", "fc_batchnorm_stats", "fc_batchnorm_apply", "fc_batchnorm_backward",
+           "fc_diagnormal_log_prob", "fc_diagnormal_log_prob_backward", "fc_diagnormal_sample",
+           "fc_diagnormal_sample_backward", "fc_diagnormal_workspace_floats",
            "fc_made_inverse_smem_bytes", "fc_made_inverse_profile", "fc_made_inverse_rqs", "fc_made_inverse_affine",
            "fc_made_inverse_sos", "fc_made_inverse_linspline", "fc_made_inverse_quadspline", "fc_made_inverse_cubicspline",
            "fc_version", "fc_built_for_sm"]
@@ -166,6 +168,11 @@ def lib():
         L.fc_batchnorm_apply.argtypes = [vp, i64, vp, vp, vp, vp, f32, vp, i64, vp, i64, i32, i32, vp]
         L.fc_batchnorm_backward.argtypes = [vp, i64, vp, vp, vp, vp, f32, vp, i64, vp, vp, i64, vp, vp, vp, i64, i32,
                                             i32, vp]
+        L.fc_diagnormal_log_prob.argtypes = [vp, i64, vp, i64, vp, vp, i64, i32, i64, vp]
+        L.fc_diagnormal_log_prob_backward.argtypes = [vp, i64, vp, i64, vp, vp, i64, vp, vp, i64, i32, i64, vp]
+        L.fc_diagnormal_sample.argtypes = [vp, i64, vp, i64, vp, i64, i64, i32, i64, vp]
+        L.fc_diagnormal_sample_backward.argtypes = [vp, i64, vp, i64, vp, i64, vp, vp, i64, i32, i64, vp]
+        L.fc_diagnormal_workspace_floats.argtypes = [i64, i32, i64]
         L.fc_made_inverse_smem_bytes.argtypes = [i32, i32, i32, i32, i32]
         L.fc_made_inverse_profile.argtypes = [ctypes.POINTER(ctypes.c_uint64)]
         L.fc_made_inverse_rqs.argtypes = [ctypes.POINTER(MadeProgramStruct), vp, i64, vp, i64, vp, i32, i64,
@@ -187,6 +194,7 @@ def lib():
         L.fc_actnorm_workspace_floats.restype = ctypes.c_int64
         L.fc_lulinear_workspace_floats.restype = ctypes.c_int64
         L.fc_batchnorm_workspace_floats.restype = ctypes.c_int64
+        L.fc_diagnormal_workspace_floats.restype = ctypes.c_int64
         _lib = L
     return _lib
 

@@ -1,2 +1,2 @@
 from .base import Distribution, NoMeanException  # noqa: F401
-from .normal import StandardNormal  # noqa: F401
+from .normal import ConditionalDiagonalNormal, DiagonalNormal, StandardNormal  # noqa: F401

@@ -5,7 +5,7 @@ from inspect import signature
 import torch.nn
 
 from ..distributions.base import Distribution
-from ..distributions.normal import StandardNormal
+from ..distributions.normal import ConditionalDiagonalNormal, DiagonalNormal, StandardNormal
 from ..utils import torchutils
 
 __all__ = ["Flow"]
@@ -30,6 +30,8 @@ class Flow(Distribution):
         noise, logabsdet = self._transform(inputs, context=embedded)
         if type(self._distribution) is StandardNormal:
             return self._distribution.log_prob_plus(noise, logabsdet)  # fused base density + logabsdet
+        if type(self._distribution) in (DiagonalNormal, ConditionalDiagonalNormal):
+            return self._distribution.log_prob_plus(noise, logabsdet, context=embedded)
         if self._context_used_in_base:
             return self._distribution.log_prob(noise, context=embedded) + logabsdet
         return self._distribution.log_prob(noise) + logabsdet

@@ -897,3 +897,144 @@ def _sn_backward(ctx, g):
 
 
 stdnormal_log_prob.register_autograd(_sn_backward, setup_context=_sn_setup)
+
+
+# ------------------------------------------------------------------------------------------------
+# diagonal Gaussian base densities (DiagonalNormal, ConditionalDiagonalNormal): params [C, 2D] = [means | log stds],
+# data row r uses parameter row r // group
+# ------------------------------------------------------------------------------------------------
+def _dn_operands(rows, params, D, group):
+    _cabi.require_cuda_f32(params, "base density params")
+    if params.dim() != 2 or params.shape[1] != 2 * D:
+        raise ValueError("base density params must be [C, {}], got {}".format(2 * D, tuple(params.shape)))
+    want = max(1, -(-rows // group)) if group >= 1 else -1  # an empty batch still has its one shared row
+    if params.shape[0] != want:
+        raise ValueError("{} rows in groups of {} need {} parameter rows, got {}".format(
+            rows, group, want, params.shape[0]))
+    return _cabi.rows(params)
+
+
+def _dn_workspace(L, R, D, group, device):
+    n = int(L.fc_diagnormal_workspace_floats(R, D, group))
+    if n < 0:
+        _cabi.check(n, "fc_diagnormal_workspace_floats")
+    return torch.empty((max(n, 1),), dtype=torch.float32, device=device)
+
+
+@torch.library.custom_op("flowcon_b200::diagnormal_log_prob", mutates_args=())
+def diagnormal_log_prob(x: Tensor, params: Tensor, group: int, logabsdet: Optional[Tensor]) -> Tensor:
+    """log N(x; m, diag e^{2s}) per row (+ logabsdet) in one pass; row r reads parameter row r // group."""
+    _cabi.require_cuda_f32(x, "inputs")
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    R, D = x.shape
+    params, pp, ps = _dn_operands(R, params, D, group)
+    out = torch.empty((R,), dtype=x.dtype, device=x.device)
+    ladp = None
+    if logabsdet is not None:
+        logabsdet = _cabi.require_cuda_f32(logabsdet, "logabsdet").contiguous()
+        ladp = logabsdet.data_ptr()
+    with torch.cuda.device(x.device), _cabi.launch("fc_diagnormal_log_prob", x.device):
+        rc = L.fc_diagnormal_log_prob(xp, xs, pp, ps, ladp, out.data_ptr(), R, D, group, _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_diagnormal_log_prob")
+    return out
+
+
+@diagnormal_log_prob.register_fake
+def _(x, params, group, logabsdet):
+    return x.new_empty((x.shape[0],))
+
+
+@torch.library.custom_op("flowcon_b200::diagnormal_log_prob_backward", mutates_args=())
+def diagnormal_log_prob_backward(x: Tensor, params: Tensor, group: int, grad_out: Tensor) -> Tuple[Tensor, Tensor]:
+    """(grad_x [R, D], grad_params [C, 2D]); the parameter gradients are group sums taken in a fixed order."""
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    R, D = x.shape
+    params, pp, ps = _dn_operands(R, params, D, group)
+    grad_out = _cabi.require_cuda_f32(grad_out, "grad outputs").contiguous()
+    gx = torch.empty((R, D), dtype=x.dtype, device=x.device)
+    gp = (torch.empty if R > 0 else torch.zeros)((params.shape[0], 2 * D), dtype=x.dtype, device=x.device)
+    ws = _dn_workspace(L, R, D, group, x.device)
+    with torch.cuda.device(x.device), _cabi.launch("fc_diagnormal_log_prob_backward", x.device):
+        rc = L.fc_diagnormal_log_prob_backward(xp, xs, pp, ps, grad_out.data_ptr(), gx.data_ptr(), D, gp.data_ptr(),
+                                               ws.data_ptr(), R, D, group, _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_diagnormal_log_prob_backward")
+    return gx, gp
+
+
+@diagnormal_log_prob_backward.register_fake
+def _(x, params, group, grad_out):
+    return torch.empty_like(x), params.new_empty((params.shape[0], 2 * x.shape[1]))
+
+
+def _dn_lp_setup(ctx, inputs, output):
+    x, params, group, lad = inputs
+    ctx.save_for_backward(x, params)
+    ctx.group = group
+    ctx.has_lad = lad is not None
+
+
+def _dn_lp_backward(ctx, g):
+    x, params = ctx.saved_tensors
+    gx, gp = diagnormal_log_prob_backward(x, params, ctx.group, g)
+    return gx, gp, None, (g if ctx.has_lad else None)
+
+
+diagnormal_log_prob.register_autograd(_dn_lp_backward, setup_context=_dn_lp_setup)
+
+
+@torch.library.custom_op("flowcon_b200::diagnormal_sample", mutates_args=())
+def diagnormal_sample(noise: Tensor, params: Tensor, group: int) -> Tensor:
+    """m + e^{s} · noise per row; row r reads parameter row r // group (no repeated copies of the parameters)."""
+    _cabi.require_cuda_f32(noise, "noise")
+    L = _cabi.lib()
+    noise, np_, ns = _cabi.rows(noise)
+    R, D = noise.shape
+    params, pp, ps = _dn_operands(R, params, D, group)
+    y = torch.empty((R, D), dtype=noise.dtype, device=noise.device)
+    with torch.cuda.device(noise.device), _cabi.launch("fc_diagnormal_sample", noise.device):
+        rc = L.fc_diagnormal_sample(np_, ns, pp, ps, y.data_ptr(), D, R, D, group, _cabi.stream_ptr(noise.device))
+    _cabi.check(rc, "fc_diagnormal_sample")
+    return y
+
+
+@diagnormal_sample.register_fake
+def _(noise, params, group):
+    return torch.empty_like(noise)
+
+
+@torch.library.custom_op("flowcon_b200::diagnormal_sample_backward", mutates_args=())
+def diagnormal_sample_backward(noise: Tensor, params: Tensor, group: int, grad_samples: Tensor) -> Tensor:
+    """grad_params [C, 2D]: group sums of grad_samples and of grad_samples · e^{s} · noise, in a fixed order."""
+    L = _cabi.lib()
+    noise, np_, ns = _cabi.rows(noise)
+    R, D = noise.shape
+    params, pp, ps = _dn_operands(R, params, D, group)
+    grad_samples, gsp, gss = _cabi.rows(_cabi.require_cuda_f32(grad_samples, "grad outputs"))
+    gp = (torch.empty if R > 0 else torch.zeros)((params.shape[0], 2 * D), dtype=noise.dtype, device=noise.device)
+    ws = _dn_workspace(L, R, D, group, noise.device)
+    with torch.cuda.device(noise.device), _cabi.launch("fc_diagnormal_sample_backward", noise.device):
+        rc = L.fc_diagnormal_sample_backward(np_, ns, pp, ps, gsp, gss, gp.data_ptr(), ws.data_ptr(), R, D, group,
+                                             _cabi.stream_ptr(noise.device))
+    _cabi.check(rc, "fc_diagnormal_sample_backward")
+    return gp
+
+
+@diagnormal_sample_backward.register_fake
+def _(noise, params, group, grad_samples):
+    return params.new_empty((params.shape[0], 2 * noise.shape[1]))
+
+
+def _dn_sample_setup(ctx, inputs, output):
+    noise, params, group = inputs
+    ctx.save_for_backward(noise, params)
+    ctx.group = group
+
+
+def _dn_sample_backward(ctx, gy):
+    noise, params = ctx.saved_tensors
+    return None, diagnormal_sample_backward(noise, params, ctx.group, gy), None
+
+
+diagnormal_sample.register_autograd(_dn_sample_backward, setup_context=_dn_sample_setup)

@@ -157,6 +157,24 @@ WORKLOADS = {
     "maf_bn_small": {"features": 6, "context_features": None, "batch": 128, "layers": _maf_bn_stack(2, 16)},
     "realnvp_bn_small": {"features": 6, "context_features": None, "batch": 128, "layers": _realnvp_bn_stack(2, 16)},
     "maf_bn": {"features": 43, "context_features": None, "batch": 262144, "layers": _maf_bn_stack(5, 256)},
+    # Gaussian bases with learned parameters (flowcon/distributions/normal.py): `base` names the base density, the
+    # default being StandardNormal.  A conditional one reads its means and log standard deviations from a linear
+    # encoder of the context (nn.Linear(context_features, 2 D)).
+    "cond_prq_diag_small": {"features": 6, "context_features": 4, "batch": 64,
+                            "layers": [{"kind": "cond_prq", "num_bins": 8, "tails": "linear", "tail_bound": 3.0,
+                                        "hidden_features": 16, "num_blocks": 2}],
+                            "base": {"kind": "conditional_diagonal_normal", "encoder": "linear"}},
+    "maf_diag_small": {"features": 6, "context_features": None, "batch": 128,
+                       "layers": [{"kind": "permutation", "mode": "reverse"},
+                                  {"kind": "maf_affine", "hidden_features": 16, "num_blocks": 2},
+                                  {"kind": "permutation", "mode": "reverse"},
+                                  {"kind": "maf_affine", "hidden_features": 16, "num_blocks": 2}],
+                       "base": {"kind": "diagonal_normal"}},
+    # cfg 4's shape (D = 32, context 8, 262 144 rows) with a context-dependent base
+    "cond_sos_diag": {"features": 32, "context_features": 8, "batch": 262144,
+                      "layers": [{"kind": "cond_sos", "n_sigmoids": 10, "hidden_features": 64, "num_blocks": 2}
+                                 for _ in range(3)],
+                      "base": {"kind": "conditional_diagonal_normal", "encoder": "linear"}},
 }
 
 
@@ -262,13 +280,40 @@ def trained_like_(state, workload, seed=1, weight_gain=8.0):
             std = std.reshape(-1)
         state[wkey] = state[wkey] * weight_gain
         state[bkey] = state[bkey] + (noise * std).to(state[bkey].dtype)
+    base = workload.get("base", {}).get("kind")
+    if base == "diagonal_normal":  # a trained base is shifted and scaled per feature
+        for name, std in (("mean_", 0.5), ("log_std_", 0.3)):
+            key = "_distribution." + name
+            state[key] = state[key] + std * torch.randn(state[key].shape, generator=g)
+    elif base == "conditional_diagonal_normal":
+        key = "_distribution._context_encoder.bias"
+        state[key] = state[key] + 0.3 * torch.randn(state[key].shape, generator=g)
     return state
+
+
+def build_base(workload):
+    """The workload's base density: `base` {"kind": "diagonal_normal"} or {"kind": "conditional_diagonal_normal",
+    "encoder": "linear"}; StandardNormal without one."""
+    from . import distributions
+
+    features = workload["features"]
+    base = workload.get("base")
+    if base is None:
+        return distributions.StandardNormal([features])
+    if base["kind"] == "diagonal_normal":
+        return distributions.DiagonalNormal([features])
+    if base["kind"] == "conditional_diagonal_normal":
+        encoder = None
+        if base.get("encoder") == "linear":
+            encoder = torch.nn.Linear(workload["context_features"], 2 * features)
+        return distributions.ConditionalDiagonalNormal([features], context_encoder=encoder)
+    raise ValueError(base["kind"])
 
 
 def build_flow(workload, seed=0):
     """Instantiate the workload with this package's drop-in classes (random init, CPU tensors;
     move with `.to('cuda')`)."""
-    from . import distributions, flows, transforms
+    from . import flows, transforms
     from .nn import nets
 
     torch.manual_seed(seed)
@@ -365,4 +410,4 @@ def build_flow(workload, seed=0):
                 num_blocks=layer["num_blocks"]))
         else:
             raise ValueError(kind)
-    return flows.Flow(transforms.CompositeTransform(layers), distributions.StandardNormal([features]))
+    return flows.Flow(transforms.CompositeTransform(layers), build_base(workload))

@@ -600,6 +600,35 @@ int fc_batchnorm_backward(const float* x, int64_t x_row_stride, const float* mea
                           float* grad_unconstrained_weight, float* grad_bias, float* workspace, int64_t B, int32_t D,
                           int32_t mode, void* stream);
 
+/*
+ * Diagonal Gaussian base densities (csrc/fc_diagnormal.cu; DiagonalNormal and ConditionalDiagonalNormal,
+ * flowcon/distributions/normal.py), any D >= 1.  The parameters are params [C, 2D] row-major (row stride >= 2D; ignored
+ * when one row serves every data row): means in columns [0, D), log standard deviations s in columns [D, 2D), so a
+ * context encoder's output is read in place.  Data row r uses parameter row r / group (C = ceil(R / group)):
+ * group 1 for a conditional log-density, n for n draws per context row, R for one shared row.
+ *   fc_diagnormal_log_prob   out[r] = −½ Σ_d z² − Σ_d s − ½ D ln 2π (+ logabsdet[r]),  z = (x − m) · e^{−s};
+ *                            logabsdet may be NULL
+ *   fc_diagnormal_sample     samples[r] = m + e^{s} · noise[r]
+ * The backward entries write grad_params [C, 2D] (dense): for the log-density, grad_x = −g z e^{−s} and the group sums
+ * of g z e^{−s} (means) and g (z² − 1) (log standard deviations), g = grad_out [R]; for sampling, the group sums of
+ * grad_samples (means) and grad_samples · e^{s} · noise (log standard deviations).  The sums are taken in a fixed
+ * order (deterministic); workspace: fc_diagnormal_workspace_floats(R, D, group) floats of device scratch (may be NULL
+ * when that is 0).  x, noise, samples and the gradients are [R, D] with their own row strides (>= D); any R >= 0.
+ */
+int fc_diagnormal_log_prob(const float* x, int64_t x_row_stride, const float* params, int64_t params_row_stride,
+                           const float* logabsdet, float* out, int64_t R, int32_t D, int64_t group, void* stream);
+int fc_diagnormal_log_prob_backward(const float* x, int64_t x_row_stride, const float* params,
+                                    int64_t params_row_stride, const float* grad_out, float* grad_x,
+                                    int64_t gx_row_stride, float* grad_params, float* workspace, int64_t R, int32_t D,
+                                    int64_t group, void* stream);
+int fc_diagnormal_sample(const float* noise, int64_t noise_row_stride, const float* params, int64_t params_row_stride,
+                         float* samples, int64_t samples_row_stride, int64_t R, int32_t D, int64_t group, void* stream);
+int fc_diagnormal_sample_backward(const float* noise, int64_t noise_row_stride, const float* params,
+                                  int64_t params_row_stride, const float* grad_samples, int64_t gs_row_stride,
+                                  float* grad_params, float* workspace, int64_t R, int32_t D, int64_t group,
+                                  void* stream);
+int64_t fc_diagnormal_workspace_floats(int64_t R, int32_t D, int64_t group);
+
 /* Library / build info (also used by the loader test). */
 const char* fc_version(void);
 int fc_built_for_sm(void); /* 100 */
