@@ -21,6 +21,7 @@ AFFINE_BLOCKED, AFFINE_INTERLEAVED = 0, 1
 BATCHNORM_TRAIN, BATCHNORM_EVAL_FORWARD, BATCHNORM_EVAL_INVERSE = 0, 1, 2
 SCALE_SIGMOID2, SCALE_SOFTPLUS_CLAMP3, SCALE_SOFTPLUS_EPS = 0, 1, 2
 LINEAR_A_T128, LINEAR_OUT_T128, LINEAR_RESIDUAL_GATES = 1, 2, 4
+POINTWISE_SIGMOID, POINTWISE_TANH, POINTWISE_LEAKY_RELU, POINTWISE_EXP, POINTWISE_CAUCHY_CDF = 0, 1, 2, 3, 4
 
 EXPORTS = ["fc_rqs_apply", "fc_rqs_backward", "fc_rqs_bins", "fc_linspline_apply", "fc_linspline_backward",
            "fc_quadspline_apply", "fc_quadspline_backward", "fc_cubicspline_apply", "fc_cubicspline_backward", "fc_affine_apply", "fc_affine_backward", "fc_sos_apply",
@@ -33,6 +34,7 @@ EXPORTS = ["fc_rqs_apply", "fc_rqs_backward", "fc_rqs_bins", "fc_linspline_apply
            "fc_batchnorm_workspace_floats", "fc_batchnorm_stats", "fc_batchnorm_apply", "fc_batchnorm_backward",
            "fc_diagnormal_log_prob", "fc_diagnormal_log_prob_backward", "fc_diagnormal_sample",
            "fc_diagnormal_sample_backward", "fc_diagnormal_workspace_floats",
+           "fc_pointwise_apply", "fc_pointwise_workspace_floats", "fc_pointwise_backward",
            "fc_made_inverse_smem_bytes", "fc_made_inverse_profile", "fc_made_inverse_rqs", "fc_made_inverse_affine",
            "fc_made_inverse_sos", "fc_made_inverse_linspline", "fc_made_inverse_quadspline", "fc_made_inverse_cubicspline",
            "fc_version", "fc_built_for_sm"]
@@ -54,6 +56,12 @@ class QuadSplineConfig(ctypes.Structure):
     _fields_ = [("num_bins", ctypes.c_int32), ("tails", ctypes.c_int32), ("inverse", ctypes.c_int32),
                 ("left", ctypes.c_float), ("right", ctypes.c_float), ("bottom", ctypes.c_float), ("top", ctypes.c_float),
                 ("min_bin_width", ctypes.c_float), ("min_bin_height", ctypes.c_float), ("wh_scale", ctypes.c_float)]
+
+
+class PointwiseConfig(ctypes.Structure):
+    """struct fc_pointwise_config"""
+    _fields_ = [("op", ctypes.c_int32), ("inverse", ctypes.c_int32), ("slope", ctypes.c_float), ("eps", ctypes.c_float),
+                ("temperature", ctypes.c_void_p)]
 
 
 class Cols(ctypes.Structure):
@@ -173,6 +181,10 @@ def lib():
         L.fc_diagnormal_sample.argtypes = [vp, i64, vp, i64, vp, i64, i64, i32, i64, vp]
         L.fc_diagnormal_sample_backward.argtypes = [vp, i64, vp, i64, vp, i64, vp, vp, i64, i32, i64, vp]
         L.fc_diagnormal_workspace_floats.argtypes = [i64, i32, i64]
+        L.fc_pointwise_apply.argtypes = [vp, i64, vp, i64, vp, i32, i64, i64, ctypes.POINTER(PointwiseConfig), vp, vp]
+        L.fc_pointwise_workspace_floats.argtypes = [i64, i64]
+        L.fc_pointwise_backward.argtypes = [vp, i64, vp, i64, vp, vp, i64, vp, vp, i64, i64,
+                                            ctypes.POINTER(PointwiseConfig), vp]
         L.fc_made_inverse_smem_bytes.argtypes = [i32, i32, i32, i32, i32]
         L.fc_made_inverse_profile.argtypes = [ctypes.POINTER(ctypes.c_uint64)]
         L.fc_made_inverse_rqs.argtypes = [ctypes.POINTER(MadeProgramStruct), vp, i64, vp, i64, vp, i32, i64,
@@ -195,6 +207,7 @@ def lib():
         L.fc_lulinear_workspace_floats.restype = ctypes.c_int64
         L.fc_batchnorm_workspace_floats.restype = ctypes.c_int64
         L.fc_diagnormal_workspace_floats.restype = ctypes.c_int64
+        L.fc_pointwise_workspace_floats.restype = ctypes.c_int64
         _lib = L
     return _lib
 

@@ -1038,3 +1038,100 @@ def _dn_sample_backward(ctx, gy):
 
 
 diagnormal_sample.register_autograd(_dn_sample_backward, setup_context=_dn_sample_setup)
+
+
+# ------------------------------------------------------------------------------------------------
+# element-wise squashing layers (Sigmoid / Logit, Tanh, LeakyReLU, Exp, CauchyCDF): x [B, N] -> (y [B, N], logabsdet [B])
+# ------------------------------------------------------------------------------------------------
+def _pw_cfg(op, inverse, slope, eps, temperature):
+    tp = None
+    if op == _cabi.POINTWISE_SIGMOID:
+        _cabi.require_cuda_f32(temperature, "temperature")
+        if temperature.numel() != 1:
+            raise ValueError("temperature must have one element")
+        tp = temperature.data_ptr()
+    return _cabi.PointwiseConfig(int(op), int(inverse), float(slope), float(eps), tp)
+
+
+@torch.library.custom_op("flowcon_b200::pointwise_layer", mutates_args=())
+def pointwise_layer(x: Tensor, temperature: Optional[Tensor], op: int, inverse: bool, slope: float,
+                    eps: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """(y, logabsdet, status): one pass over x [B, N] (any row stride >= N); status carries
+    FC_STATUS_INPUT_OUTSIDE_DOMAIN for the directions with a domain.  temperature: device [1] (Sigmoid only)."""
+    _cabi.require_cuda_f32(x, "inputs")
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    B, N = x.shape
+    if temperature is not None:
+        temperature = temperature.contiguous()
+    cfg = _pw_cfg(op, inverse, slope, eps, temperature)
+    y = torch.empty((B, N), dtype=x.dtype, device=x.device)
+    lad = torch.empty((B,), dtype=x.dtype, device=x.device)
+    status = torch.zeros((1,), dtype=torch.int32, device=x.device)
+    with torch.cuda.device(x.device), _cabi.launch("fc_pointwise_apply", x.device):
+        rc = L.fc_pointwise_apply(xp, xs, y.data_ptr(), N, lad.data_ptr(), 0, B, N, ctypes.byref(cfg),
+                                  status.data_ptr(), _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_pointwise_apply")
+    return y, lad, status
+
+
+@pointwise_layer.register_fake
+def _(x, temperature, op, inverse, slope, eps):
+    return torch.empty_like(x), x.new_empty((x.shape[0],)), x.new_empty((1,), dtype=torch.int32)
+
+
+@torch.library.custom_op("flowcon_b200::pointwise_layer_backward", mutates_args=())
+def pointwise_layer_backward(x: Tensor, temperature: Optional[Tensor], grad_y: Optional[Tensor],
+                             grad_lad: Optional[Tensor], op: int, inverse: bool, slope: float, eps: float,
+                             want_temperature: bool) -> Tuple[Tensor, Tensor]:
+    """(grad_x [B, N], grad_temperature [1]) at the layer's input x; grad_temperature is a fixed-order sum over every
+    element when want_temperature, else zero."""
+    L = _cabi.lib()
+    x, xp, xs = _cabi.rows(x)
+    B, N = x.shape
+    if temperature is not None:
+        temperature = temperature.contiguous()
+    cfg = _pw_cfg(op, inverse, slope, eps, temperature)
+    gyp, gys = None, N
+    if grad_y is not None:
+        grad_y, gyp, gys = _cabi.rows(_cabi.require_cuda_f32(grad_y, "grad outputs").reshape(B, N))
+    glp = None
+    if grad_lad is not None:
+        grad_lad = _cabi.require_cuda_f32(grad_lad, "grad logabsdet").contiguous()
+        glp = grad_lad.data_ptr()
+    gx = torch.empty((B, N), dtype=x.dtype, device=x.device)
+    gt = torch.zeros((1,), dtype=x.dtype, device=x.device)
+    gtp, ws = None, None
+    if want_temperature:
+        n = int(L.fc_pointwise_workspace_floats(B, N))
+        _cabi.check(min(n, 0), "fc_pointwise_workspace_floats")
+        ws = torch.empty((n,), dtype=torch.float32, device=x.device)
+        gtp = gt.data_ptr()
+    with torch.cuda.device(x.device), _cabi.launch("fc_pointwise_backward", x.device):
+        rc = L.fc_pointwise_backward(xp, xs, gyp, gys, glp, gx.data_ptr(), N, gtp,
+                                     None if ws is None else ws.data_ptr(), B, N, ctypes.byref(cfg),
+                                     _cabi.stream_ptr(x.device))
+    _cabi.check(rc, "fc_pointwise_backward")
+    return gx, gt
+
+
+@pointwise_layer_backward.register_fake
+def _(x, temperature, grad_y, grad_lad, op, inverse, slope, eps, want_temperature):
+    return torch.empty_like(x), x.new_empty((1,))
+
+
+def _pw_setup(ctx, inputs, output):
+    x, temperature, op, inverse, slope, eps = inputs
+    ctx.save_for_backward(x, temperature)
+    ctx.hyper = (op, inverse, slope, eps)
+    ctx.mark_non_differentiable(output[2])
+
+
+def _pw_backward(ctx, gy, gl, _gstatus):
+    x, temperature = ctx.saved_tensors
+    want_t = temperature is not None and ctx.needs_input_grad[1]
+    gx, gt = pointwise_layer_backward(x, temperature, gy, gl, *ctx.hyper, want_t)
+    return gx, (gt.reshape(temperature.shape) if want_t else None), None, None, None, None
+
+
+pointwise_layer.register_autograd(_pw_backward, setup_context=_pw_setup)

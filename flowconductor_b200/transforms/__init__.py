@@ -15,8 +15,9 @@ from .coupling import (AdditiveCouplingTransform, AffineCouplingTransform, Coupl
                        PiecewiseQuadraticCouplingTransform,
                        PiecewiseRationalQuadraticCouplingTransform)
 from .made import MADE, MaskedLinear  # noqa: F401
-from .nonlinearities import (PiecewiseCubicCDF, PiecewiseLinearCDF, PiecewiseQuadraticCDF,  # noqa: F401
-                            PiecewiseRationalQuadraticCDF)
+from .nonlinearities import (CauchyCDF, CauchyCDFInverse, CompositeCDFTransform, Exp, LeakyReLU,  # noqa: F401
+                             Logit, PiecewiseCubicCDF, PiecewiseLinearCDF, PiecewiseQuadraticCDF,
+                             PiecewiseRationalQuadraticCDF, Sigmoid, Tanh)
 from .lu import LULinear  # noqa: F401
 from .normalization import ActNorm, BatchNorm  # noqa: F401
 from .permutations import Permutation, RandomPermutation, ReversePermutation  # noqa: F401

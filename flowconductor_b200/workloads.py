@@ -59,6 +59,18 @@ def _realnvp_bn_stack(num_layers, hidden, num_blocks=2):
     return layers
 
 
+def _bounded_maf_stack(features, num_layers, num_bins, hidden, cdf_after=None, learn_logit_temperature=False):
+    """Data on the unit box: a Logit in front of cfg 3's MAF-RQS stack; cdf_after = i puts
+    CompositeCDFTransform(Sigmoid(learn_temperature=True), PiecewiseRationalQuadraticCDF([D], num_bins)) after layer i of
+    that stack (the neural-spline-flow way to run a tails=None spline on unbounded features)."""
+    layers = [{"kind": "logit", "learn_temperature": learn_logit_temperature}]
+    for i, layer in enumerate(_maf_prq_stack(features, num_layers, num_bins, hidden)):
+        layers.append(layer)
+        if i == cdf_after:
+            layers.append({"kind": "composite_cdf", "num_bins": 8, "learn_temperature": True})
+    return layers
+
+
 WORKLOADS = {
     # cfg 1: README.md:86-98 model (MAF(2, 4) + RandomPermutation), evaluated on 2-D toy batches
     "cfg1": {"features": 2, "context_features": None, "batch": 10000,
@@ -175,6 +187,13 @@ WORKLOADS = {
                       "layers": [{"kind": "cond_sos", "n_sigmoids": 10, "hidden_features": 64, "num_blocks": 2}
                                  for _ in range(3)],
                       "base": {"kind": "conditional_diagonal_normal", "encoder": "linear"}},
+    # bounded data (drawn in (0, 1)): Logit in front, a squashed spline CDF inside (nonlinearities.py).  The small twin
+    # learns its logit's temperature and has no layer that checks its domain in the sampling direction, so its sampler
+    # and a training-by-sampling step can be recorded into CUDA graphs.
+    "bounded_maf": {"features": 16, "context_features": None, "batch": 262144, "data": "unit_box",
+                    "layers": _bounded_maf_stack(16, 5, 16, 256, cdf_after=1)},
+    "bounded_maf_small": {"features": 6, "context_features": None, "batch": 128, "data": "unit_box",
+                          "layers": _bounded_maf_stack(6, 2, 16, 32, learn_logit_temperature=True)},
 }
 
 
@@ -242,6 +261,14 @@ def trained_like_(state, workload, seed=1, weight_gain=8.0):
         kind = layer["kind"]
         if kind == "permutation":
             continue
+        if kind in ("logit", "composite_cdf"):  # a learned temperature moves away from 1
+            if layer.get("learn_temperature"):
+                keys = ([layer_prefix(i) + "_transform.temperature"] if kind == "logit" else
+                        [layer_prefix(i) + "_transforms.0.temperature", layer_prefix(i) + "_transforms.2._transform.temperature"])
+                value = state[keys[0]] * torch.exp(0.3 * torch.randn(1, generator=g))
+                for key in keys:  # CompositeCDFTransform holds its squashing layer twice
+                    state[key] = value.clone()
+            continue
         if kind == "actnorm":  # a trained ActNorm has non-trivial per-feature scales and shifts
             for name, std in (("log_scale", 0.4), ("shift", 0.7)):
                 key = layer_prefix(i) + name
@@ -291,6 +318,15 @@ def trained_like_(state, workload, seed=1, weight_gain=8.0):
     return state
 
 
+def sample_data(workload, rows, seed=0):
+    """Seeded data for a workload: in (0, 1) for `"data": "unit_box"` workloads, standard normal otherwise."""
+    g = torch.Generator().manual_seed(seed)
+    x = torch.randn(rows, workload["features"], generator=g)
+    if workload.get("data") == "unit_box":
+        return torch.sigmoid(x)
+    return x
+
+
 def build_base(workload):
     """The workload's base density: `base` {"kind": "diagonal_normal"} or {"kind": "conditional_diagonal_normal",
     "encoder": "linear"}; StandardNormal without one."""
@@ -329,6 +365,15 @@ def build_flow(workload, seed=0):
             layers.append(transforms.ActNorm(features))
         elif kind == "batchnorm":
             layers.append(transforms.BatchNorm(features))
+        elif kind == "logit":
+            if layer.get("learn_temperature"):  # Logit with its Sigmoid's temperature learned
+                layers.append(transforms.InverseTransform(transforms.Sigmoid(learn_temperature=True)))
+            else:
+                layers.append(transforms.Logit())
+        elif kind == "composite_cdf":
+            layers.append(transforms.CompositeCDFTransform(
+                transforms.Sigmoid(learn_temperature=layer.get("learn_temperature", False)),
+                transforms.PiecewiseRationalQuadraticCDF([features], layer["num_bins"])))
         elif kind == "lu_linear":
             layers.append(transforms.LULinear(features, identity_init=layer.get("identity_init", True)))
         elif kind == "prq_coupling":

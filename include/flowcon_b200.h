@@ -629,6 +629,45 @@ int fc_diagnormal_sample_backward(const float* noise, int64_t noise_row_stride, 
                                   void* stream);
 int64_t fc_diagnormal_workspace_floats(int64_t R, int32_t D, int64_t group);
 
+/*
+ * Element-wise squashing layers (csrc/fc_pointwise.cu; Sigmoid / Logit, Tanh, LeakyReLU, Exp, CauchyCDF,
+ * flowcon/transforms/nonlinearities.py) on x [B, D], any B >= 0, D >= 1, row strides >= D:
+ *   op                         forward y, log-det term                      inverse x, log-det term
+ *   FC_POINTWISE_SIGMOID       σ(T x), log T − softplus(−T x) − softplus(T x)  logit(clamp(y, eps, 1 − eps)) / T, minus it
+ *   FC_POINTWISE_TANH          tanh x, log(1 − tanh² x)                      atanh y, −log(1 − y²)
+ *   FC_POINTWISE_LEAKY_RELU    leaky_relu(x, slope), log slope · [x < 0]      leaky_relu(y, 1 / slope), −log slope · [y < 0]
+ *   FC_POINTWISE_EXP           eˣ, x                                         log y, −log y
+ *   FC_POINTWISE_CAUCHY_CDF    atan(x) / π + ½, −log π − log(1 + x²)         tan(π (y − ½)), log π + log(1 + x²)
+ * logabsdet[b] = (accumulate ? logabsdet[b] : 0) + Σ_d (log-det term).  `temperature` is a device pointer to T (one
+ * float, read by the kernels: a captured graph sees later updates; Sigmoid only).  The directions in which the
+ * reference raises InputOutsideDomain (the inverses of Sigmoid, Tanh, Exp and CauchyCDF) OR
+ * FC_STATUS_INPUT_OUTSIDE_DOMAIN into *status (may be NULL) for inputs outside [0, 1], outside (−1, 1), <= 0 and
+ * outside [0, 1] respectively, and compute on.
+ * fc_pointwise_backward reads the layer's input x once and writes grad_x = grad_y · dy/dx + grad_logabsdet[b] ·
+ * d(log-det term)/dx (grad_y and grad_logabsdet may be NULL: zero).  With grad_temperature non-NULL (Sigmoid) it also
+ * writes ∂/∂T of the same objective, summed over every element through per-CTA partials in a fixed order and a finish
+ * kernel: two calls are bitwise equal.  workspace: fc_pointwise_workspace_floats(B, D) floats of device scratch.
+ */
+#define FC_POINTWISE_SIGMOID 0
+#define FC_POINTWISE_TANH 1
+#define FC_POINTWISE_LEAKY_RELU 2
+#define FC_POINTWISE_EXP 3
+#define FC_POINTWISE_CAUCHY_CDF 4
+typedef struct fc_pointwise_config {
+  int32_t op;                /* FC_POINTWISE_* */
+  int32_t inverse;           /* 0 forward, 1 inverse */
+  float slope;               /* LeakyReLU: the layer's negative slope (> 0) */
+  float eps;                 /* Sigmoid: the inverse's clamp */
+  const float* temperature;  /* Sigmoid: device [1] */
+} fc_pointwise_config;
+int fc_pointwise_apply(const float* x, int64_t x_row_stride, float* y, int64_t y_row_stride, float* logabsdet,
+                       int32_t accumulate_logabsdet, int64_t B, int64_t D, const fc_pointwise_config* cfg,
+                       int32_t* status, void* stream);
+int64_t fc_pointwise_workspace_floats(int64_t B, int64_t D);
+int fc_pointwise_backward(const float* x, int64_t x_row_stride, const float* grad_y, int64_t gy_row_stride,
+                          const float* grad_logabsdet, float* grad_x, int64_t gx_row_stride, float* grad_temperature,
+                          float* workspace, int64_t B, int64_t D, const fc_pointwise_config* cfg, void* stream);
+
 /* Library / build info (also used by the loader test). */
 const char* fc_version(void);
 int fc_built_for_sm(void); /* 100 */
